@@ -6,10 +6,10 @@ Metric (BASELINE.json): join input rows/s (and queries/s for the batch config).
   python bench.py [--gpus N --steps K --warmup W]     headline = config 2 (BASELINE.json configs[1]):
       single 2-way equi-join + range filter over 2 x 100M-row relations of 3 uint64 columns, query
       `0 1|0.1=1.1&0.2>500000|0.0 1.0 1.2` (SURVEY.md 8d).  The same line carries, under "configs",
-      short driver-visible runs of configs 3, 4 and 5 at their BASELINE sizes: the 4-way chain at
-      62.5M rows per relation per GPU (500M over 8 GPUs), the Zipf(1.2) 3-way join at 100M rows per
-      relation per GPU, and the 1000-query batch over 14 relations of 10^6..10^9 rows (one cold run +
-      one timed step: a step is ~10 s on one GPU).
+      runs of configs 3, 4 and 5 at their BASELINE sizes: the 4-way chain at 62.5M rows per relation
+      per GPU (500M over 8 GPUs), the Zipf(1.2) 3-way join at 100M rows per relation per GPU, and the
+      1000-query batch over 14 relations of 10^6..10^9 rows.  Every config (and every leg of config 2)
+      runs --warmup untimed steps, then --steps timed ones; a config-5 step is ~6 s on one GPU.
   python bench.py --config c3|c4|c5 ...                that config alone, at full size, as the line's workload
   python bench.py --impl reference ...                 the reference's own CPU binary (oracle/_ref/queries)
                                                        on the config-2 scaled twin
@@ -33,6 +33,9 @@ Every config is self-verifying (the line's "parity" block):
   e2e       headline only: every step first copies the referenced columns from pinned host memory
   roofline  per-kernel live CUDA-event times against the measured HBM peak (MEASURED_PEAKS.json)
   cpu_baseline  the reference binary on the config-2 scaled twin, on this box's host cores
+
+  --dump-outputs DIR  after the timed steps, writes what the last timed step of every config returned
+                      (the checksum lines the host layer prints) as DIR/<config>.npy; see dump_outputs
 """
 import argparse
 import ctypes as C
@@ -159,6 +162,24 @@ def time_reference(rows, steps, warmup):
         os.unlink(p)
     sec = float(np.mean(times))
     return {"rows_per_s": 2 * rows / sec, "sec_per_step": sec, "load_s": load_s, "stdout": out.strip()}
+
+
+def dump_outputs(outdir, outputs):
+    """outputs: config name -> stdout text of its last timed step.  Every value printed there (a uint64
+    checksum, a count, or NULL) becomes one row (line, high 32 bits, low 32 bits) of a float64 array, exact
+    (NULL = NaN in both halves), so two builds can be compared output for output with numpy:
+    np.array_equal(a, b, equal_nan=True).  The reference arm (--impl reference) writes reference_c2_twin."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, text in outputs.items():
+        rows = []
+        for ln, line in enumerate(text.splitlines()):
+            for tok in line.split():
+                if tok == "NULL":
+                    rows.append((ln, np.nan, np.nan))
+                else:
+                    v = int(tok)
+                    rows.append((ln, float(v >> 32), float(v & 0xFFFFFFFF)))
+        np.save(os.path.join(outdir, name + ".npy"), np.array(rows, dtype=np.float64).reshape(-1, 3))
 
 
 # ------------------------------------------------------------------ the engine as bench.py sees it
@@ -348,6 +369,7 @@ def run_generated(rig, name, w, twin, check, rel_offset, steps, warmup, twin_fir
     if sampler:
         sampler.start()
     ms, launches, out, wall_ms = rig.timed(text, steps, warmup, want=got)
+    rig.last_output = out
     clocks = sampler.stop() if sampler else None
     rows_in = w.join_input_rows()
     res = {
@@ -491,7 +513,7 @@ def config_c2(rig, rows, steps, warmup, args, local_rank):
     # the GPU arm on the very workload the reference arm times (vs_reference's same-config leg)
     if world > 1:
         rig.ck(rig.lib.qce_set_replicate_bytes(0))
-    twin_ms, _, _, _ = rig.timed(twin.text(100), max(steps, 5), 2)
+    twin_ms, _, _, _ = rig.timed(twin.text(100), steps, warmup)
     twin_leg = {"rows_per_relation": REF_SAMPLE_ROWS, "ms_per_step": twin_ms, "value": 2 * REF_SAMPLE_ROWS / (twin_ms / 1e3),
                 "unit": "rows/s", "note": "the reference arm's workload (config-2 scaled twin) through the same product path"}
 
@@ -553,6 +575,7 @@ def config_c2(rig, rows, steps, warmup, args, local_rank):
     rig.sync_all()
     sampler.start()
     ms_per_step, launches, out, wall_ms = rig.timed(q, steps, 0, want=want)
+    rig.last_output = out
     arena_c2 = getattr(rig, "last_arena", None)
     value = 2 * n / (ms_per_step / 1e3)
     # the same K steps again with CUDA events around every kernel launch (adds ~1.5 % to a step, so it is
@@ -567,7 +590,7 @@ def config_c2(rig, rows, steps, warmup, args, local_rank):
     rig.eng.profile(False)
 
     # ---- e2e: host buffers in, checksums out, every step
-    for _ in range(min(warmup, 2)):
+    for _ in range(warmup):
         upload_all(); rig.run(q)
     rig.sync_all()
     rig.eng.timer_reset()
@@ -661,7 +684,7 @@ def config_c2(rig, rows, steps, warmup, args, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every config (and of the reference arm)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="all", choices=["all", "c2", "c3", "c4", "c5"])
@@ -670,7 +693,11 @@ def main():
     ap.add_argument("--c5-scale", type=float, default=None, help="config 5: relation sizes = 10^6..10^9 rows x scale")
     ap.add_argument("--c5-queries", type=int, default=1000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write each config's output of its last timed step to DIR/<config>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     nproc = os.cpu_count() or 1
@@ -678,11 +705,13 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        steps, warm = max(1, min(args.steps, 20)), max(0, min(args.warmup, 3))
+        steps, warm = args.steps, args.warmup
         r = time_reference(REF_SAMPLE_ROWS, steps, warm)
         if r is None:
             print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/queries not built"}))
             return 0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"reference_c2_twin": r["stdout"]})
         line = {
             "impl": "reference", "metric": METRIC, "value": r["rows_per_s"], "unit": "rows/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": warm, "ms_per_step": 1e3 * r["sec_per_step"], "higher_is_better": True,
@@ -707,7 +736,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     rig = Rig(torch, dist, rank, world, local_rank)
-    short = max(2, min(args.steps, 5))
+    outputs = {}
 
     def drop():
         rig.sync_all()
@@ -716,14 +745,16 @@ def main():
 
     if args.config in ("all", "c2"):
         line = config_c2(rig, args.rows, args.steps, args.warmup, args, local_rank)
+        outputs["c2"] = rig.last_output
         others = {}
         if args.config == "all":
             drop()
-            for name, fn in (("c3", lambda: config_c3(rig, args.c3_rows, short, 2)),
-                             ("c4", lambda: config_c4(rig, args.rows, short, 2)),
-                             ("c5", lambda: config_c5(rig, args.c5_scale or 1.0, args.c5_queries, 1, 0))):
+            for name, fn in (("c3", lambda: config_c3(rig, args.c3_rows, args.steps, args.warmup)),
+                             ("c4", lambda: config_c4(rig, args.rows, args.steps, args.warmup)),
+                             ("c5", lambda: config_c5(rig, args.c5_scale or 1.0, args.c5_queries, args.steps, args.warmup))):
                 try:
                     others[name] = fn()
+                    outputs[name] = rig.last_output
                     drop()
                 except Exception as e:  # a side config never takes the headline down
                     others[name] = {"error": repr(e)[:400]}
@@ -733,6 +764,8 @@ def main():
                         rig.lib.qce_comm_abort()
                         line["configs"] = others
                         if rank == 0:
+                            if args.dump_outputs:
+                                dump_outputs(args.dump_outputs, outputs)
                             print(json.dumps(line), flush=True)
                         os._exit(0 if rank == 0 else 1)
                     drop()
@@ -745,6 +778,7 @@ def main():
             res = config_c4(rig, args.rows, args.steps, args.warmup, sampler)
         else:
             res = config_c5(rig, args.c5_scale or 1.0, args.c5_queries, args.steps, args.warmup, sampler=sampler)
+        outputs[args.config] = rig.last_output
         line = {"metric": METRIC if args.config != "c5" else "queries_per_s", "value": res["value"] if args.config != "c5" else res["queries_per_s"],
                 "unit": "rows/s" if args.config != "c5" else "queries/s", "n_gpus": world, "steps": res["steps"], "warmup": res["warmup"],
                 "ms_per_step": res["ms_per_step"], "higher_is_better": True,
@@ -753,6 +787,8 @@ def main():
                 "config": {"workload": res["workload"]}, "parity": res["parity"], "clocks": res.get("clocks"),
                 "gpu_launches": res["gpu_launches_per_step_main_stream"] * res["steps"], "detail": res}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -73,7 +73,7 @@ def test_golden_batch_replicas(world):
 def test_reference_main_unchanged_sharded():
     """The reference's own main/queries_main.c, linked against this library, sharded over 2 ranks."""
     if not os.path.exists(REFMAIN_BIN):
-        pytest.skip("build/queries_refmain needs /root/reference at build time")
+        pytest.skip("build/queries_refmain is built only where the reference's main/queries_main.c is (make REF=<its checkout>)")
     db = wl.gen_pair_db(400_000, 400_000, filt_domain=1000)
     q = "0 1|0.1=1.1&0.2>500|0.0 1.0 1.2\n0|0.1<1000&0.2>500|0.0\n"
     out, err, rc = run_queries_bin(REFMAIN_BIN, _paths(db), q, env=dict(SHARD_ALL, QCE_GPUS=2))

@@ -62,21 +62,22 @@ def test_loader_rejects_implausible_headers(tmp_path):
     """The relation file header is untrusted (src/utilities.c:105-121 trusts it): a rows x columns
     product that wraps around, or more cells than the file holds, fails before anything is uploaded."""
     import numpy as np
-    from tests.helpers import REFMAIN_BIN
-    if not os.path.exists(REFMAIN_BIN):
-        pytest.skip("needs build/queries_refmain (the reference's unchanged main linked against this library)")
+    from tests.helpers import QUERIES_BIN, REFMAIN_BIN
+    # our driver and, where it was built, the reference's unchanged main: both call read_relations
+    # before anything touches the device
+    binaries = [QUERIES_BIN] + ([REFMAIN_BIN] if os.path.exists(REFMAIN_BIN) else [])
     cases = {"wrap": np.array([1 << 61, 8, 1, 2, 3], dtype=np.uint64),       # 2^61 * 8 wraps to 0
              "trunc": np.array([1000, 3, 1, 2, 3], dtype=np.uint64),
              "huge_rows": np.array([1 << 33, 1, 5], dtype=np.uint64),
              "short": np.array([7], dtype=np.uint64)}
-    for name, words in cases.items():
-        path = tmp_path / name
-        words.tofile(path)
-        # the reference's main calls read_relations before anything touches the device
-        p = subprocess.run([REFMAIN_BIN], input=f"{path}\nDone\n".encode(), stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-        err = p.stderr.decode()
-        assert p.stdout == b"", name
-        assert ("implausible relation header" in err or "truncated" in err or "too short" in err), (name, err)
+    for binary in binaries:
+        for name, words in cases.items():
+            path = tmp_path / name
+            words.tofile(path)
+            p = subprocess.run([binary], input=f"{path}\nDone\n".encode(), stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+            err = p.stderr.decode()
+            assert p.stdout == b"", (binary, name)
+            assert ("implausible relation header" in err or "truncated" in err or "too short" in err), (binary, name, err)
 
 
 def test_library_exports_every_declared_symbol():

@@ -18,12 +18,15 @@ from tests.helpers import PKG, ROOT, load_db, load_json, run_queries_bin
 OUT = os.path.join(ROOT, "tests", "c", "build")
 SOURCES = [os.path.join(PKG, "main", "queries_driver.c"), os.path.join(ROOT, "tests", "c", "mock_engine.c")] + \
     sorted(os.path.join(PKG, "src", f) for f in os.listdir(os.path.join(PKG, "src")) if f.endswith(".c"))
+# a header change rebuilds the mocks too
+HEADERS = [os.path.join(ROOT, "include", "qce_b200.h")] + \
+    sorted(os.path.join(PKG, "src", f) for f in os.listdir(os.path.join(PKG, "src")) if f.endswith(".h"))
 
 
 def _build(name, flags):
     os.makedirs(OUT, exist_ok=True)
     exe = os.path.join(OUT, name)
-    newest = max(os.path.getmtime(s) for s in SOURCES)
+    newest = max(os.path.getmtime(s) for s in SOURCES + HEADERS)
     if not os.path.exists(exe) or os.path.getmtime(exe) < newest:
         subprocess.run(["gcc", "-g", "-Wall", "-I", os.path.join(ROOT, "include"), "-I", os.path.join(PKG, "src"),
                         "-o", exe] + flags + SOURCES + ["-lpthread"], check=True, stdout=subprocess.PIPE, stderr=subprocess.PIPE)

@@ -267,6 +267,13 @@ int qce_exchange_release(void *sendbuf);
 /* 256-bin histogram of the top 8 significant key bits of a run (for splitter
  * selection from an all-reduced global histogram).  hist = 256 uint64 on host. */
 int qce_key_histogram(const qce_tuples *t, uint32_t key_bits, uint64_t *hist);
+/* Wide runs (keys >= 2^32): the same over the key's offset from `base`, bin(key) =
+ * (key - base) >> max(width - 8, 0), width 1..64.  Every key must lie in
+ * [base, base + 2^width): the exchange takes base = the smallest key of all ranks and
+ * width = bitlen(largest - base), so keys clustered at a high offset (64-bit ids,
+ * timestamps) still spread over the bins.  Cached on the run like the packed histogram.  An
+ * empty run of either kind counts as an empty wide run (also for qce_push_tuples_wide). */
+int qce_key_histogram_wide(const qce_tuples *t, uint64_t base, uint32_t width, uint64_t *hist);
 
 /* ---- peer-memory exchange: partition + push over NVLink (SURVEY 8e) --------
  * The multi-GPU half of the reference's radix partitioning (build_histogram /
@@ -302,6 +309,12 @@ int qce_push_tuples(const qce_tuples *t, uint32_t key_bits, const uint64_t *spli
 int qce_push_tuples_cols(const qce_tuples *t, uint32_t key_bits, const uint64_t *splitters, uint32_t nparts,
                          const uint64_t *dst_word_offset, const uint32_t *dst_run_index, uint32_t ncols,
                          const qce_rowids *const *cols, const uint64_t *col_u32_offset);
+/* Scatter a wide run by the key range of key - base (qce_key_histogram_wide's bins; splitters
+ * as qce_exchange_plan returns them at that width): the keys for rank p are stored unchanged
+ * from 8-byte word dst_word_offset[p] of p's window on, their row ids in the same order from
+ * 4-byte element dst_id_offset[p] on.  Asynchronous on the engine stream. */
+int qce_push_tuples_wide(const qce_tuples *t, uint64_t base, uint32_t width, const uint64_t *splitters,
+                         uint32_t nparts, const uint64_t *dst_word_offset, const uint64_t *dst_id_offset);
 /* vals[i] -> 4-byte element dst_u32_offset[p] + position of rank p's window, (p, position) = slots[i] */
 int qce_push_u32_by_slot(const qce_rowids *vals, const qce_rowids *slots, uint32_t nparts,
                          const uint64_t *dst_u32_offset);
@@ -327,6 +340,12 @@ int qce_tuples_from_u32(const qce_rowids *keys, uint32_t key_bits, qce_tuples **
 /* Views into this rank's own window (no copy; valid until the window is reused). */
 int qce_tuples_from_window(uint64_t word_offset, uint64_t n, uint32_t key_bits, uint32_t id_bound,
                            uint64_t key_lo, uint64_t key_hi, qce_tuples **out);
+/* A wide run received by qce_push_tuples_wide: n keys from 8-byte word word_offset, their ids
+ * from 4-byte element id_u32_offset (both 16-byte aligned).  Every key lies in [key_lo, key_hi],
+ * so the keys agree above bit bitlen(key_lo ^ key_hi) and its sort passes cover only the bits
+ * below. */
+int qce_tuples_from_window_wide(uint64_t word_offset, uint64_t id_u32_offset, uint64_t n, uint32_t id_bound,
+                                uint64_t key_lo, uint64_t key_hi, qce_tuples **out);
 /* [id_min, id_bound) = range of the received ids (the owner's row window); bucketed != 0:
  * they arrived grouped by L2-sized row regions, the checksum needs no bucketing pass. */
 int qce_rowids_from_window(uint64_t u32_offset, uint64_t n, uint32_t id_min, uint32_t id_bound,
@@ -361,7 +380,10 @@ int qce_column_max_device(const void *dev, uint64_t n, uint64_t *max_value);
  * ranks put before this rank's segment (before = dst_run_index), the byte offset of the
  * side's run in the destination's window (run_off) and of each of its ncols[side] columns
  * (col_off[column][dst], columns numbered side-major), the window bytes the largest receiver
- * needs, and the tuples this rank sends off-rank per side. */
+ * needs, and the tuples this rank sends off-rank per side.  key_bits 1..64 (above 32: the width
+ * of a wide exchange; a wide side lays out its ids as one column, ncols = 1).  The splitter
+ * cutting before bin b is b << (key_bits - 8), except that a cut past the last bin at 64 bits
+ * (2^64) is returned as UINT64_MAX: it lies past every key. */
 int qce_exchange_plan(const uint64_t *hists, uint32_t world, uint32_t rank, uint32_t nsides,
                       const uint32_t *ncols, uint32_t key_bits, uint64_t *splitters, uint64_t *recv,
                       uint64_t *before, uint64_t *run_off, uint64_t *col_off, uint64_t *window_bytes,

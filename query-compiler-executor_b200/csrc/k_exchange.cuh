@@ -23,7 +23,9 @@
 //   * 4-byte row ids, digit = id / bin_width (<= 256 equal-width bins of the
 //     relation's row domain), destination = the rank that owns the bin's rows.
 //     The receiver gets its ids grouped by bin, i.e. already bucketed for
-//     L2-resident checksum gathers (this replaces partition_ids_by_top_bits).
+//     L2-resident checksum gathers (this replaces partition_ids_by_top_bits);
+//   * wide runs (SoA u64 keys + u32 ids, k_push_wide): destination = table[top 8
+//     bits of key - base], the ids follow the keys through the same staged tile.
 //
 // Algorithmic bytes: 8 B read + 8 B written per tuple (4 + 4 per id); the
 // written bytes cross NVLink for the (G-1)/G share that leaves the rank.
@@ -228,6 +230,200 @@ k_push(const KeyT *__restrict__ in, u32 n, PushDigit<KeyT> digit, PushPlan plan,
                 }
             }
         }
+    }
+}
+
+// Wide runs (keys >= 2^32: SoA u64 keys + u32 row ids).  Such keys usually sit at a high offset
+// (64-bit ids, timestamps), so the digit is the top byte of key - base over the exchange's width,
+// not of the key itself: the top bits of the key would put every tuple in one bin.
+struct PushDigitWide {
+    u64 base;
+    int shift; // width - 8 (0 below 8 bits)
+    const u32 *lut;
+    __device__ __forceinline__ u32 operator()(u64 k) const
+    {
+        const u32 b = (u32)((k - base) >> shift) & 255u;
+        return (__ldg(lut + (b >> 2)) >> ((b & 3u) * 8)) & 255u;
+    }
+};
+// id of the key stored at word w of destination d's window goes to 4-byte element w + id_delta[d]
+// (the id region is laid out like the key region; the delta wraps mod 2^64 when it is "negative")
+struct WideIdRegions {
+    unsigned long long id_delta[QCE_MAX_RANKS];
+};
+
+// k_push<u64, FEW, false> for a wide run: the key word leaves unchanged, and the row id is staged
+// through the same tile order (the REWRITE columns' mechanism) so that it too leaves as one
+// coalesced run per destination.  Destinations <= 16 (per-warp ballot ranking).
+__global__ void __launch_bounds__(QCE_PUSH_THREADS, 3)
+k_push_wide(const u64 *__restrict__ keys, const u32 *__restrict__ ids, u32 n, PushDigitWide digit, PushPlan plan,
+            const __grid_constant__ PeerWindows peers, int digit_bits, const __grid_constant__ WideIdRegions idr)
+{
+    constexpr int THREADS = QCE_PUSH_THREADS, ITEMS = PushTile<u64>::ITEMS, TILE = PushTile<u64>::TILE;
+    __shared__ u64 skeys[TILE];
+    __shared__ unsigned char sdig[TILE];
+    __shared__ u32 cnt[256], excl[256];
+    __shared__ unsigned long long goff[256];
+    __shared__ u32 scratch[33];
+    const int tid = threadIdx.x, lane = tid & 31;
+    const u32 begin = blockIdx.x * TILE;
+    if (begin >= n) return;
+    const u32 count = min((u32)TILE, n - begin);
+    if (tid < 256) cnt[tid] = 0;
+    __syncthreads();
+
+    // the keys wait in shared memory (input order) while they are ranked, and only their destinations
+    // (4 bits each) stay in registers: holding eight keys through the ranking spills at 3 CTAs per SM
+    u32 dest = 0;
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 i = tid + j * THREADS;
+        if (i < count) {
+            const u64 k = ld_stream_u64(keys + begin + i);
+            skeys[i] = k;
+            dest |= digit(k) << (4 * j);
+        }
+    }
+    u32 slot[ITEMS]; // digit << 16 | rank among the tile's elements with that digit
+    {
+        // cnt[d * 16 + warp], as in k_push<FEW>
+        const u32 lt = lanemask_lt();
+        const u32 warp = tid >> 5;
+#pragma unroll
+        for (int j = 0; j < ITEMS; j++) {
+            const u32 i = tid + j * THREADS;
+            const bool valid = i < count;
+            const u32 d = (dest >> (4 * j)) & 15u;
+            const u32 live = __ballot_sync(QCE_FULL_MASK, valid);
+            const u32 peersm = warp_peers_dyn(d, digit_bits) & live;
+            u32 b = 0;
+            const int leader = __ffs(peersm) - 1;
+            if (valid && lane == leader) {
+                b = cnt[d * 16 + warp];
+                cnt[d * 16 + warp] = b + (u32)__popc(peersm);
+            }
+            __syncwarp();
+            b = __shfl_sync(QCE_FULL_MASK, b, leader < 0 ? 0 : leader);
+            slot[j] = (d << 16) | (b + (u32)__popc(peersm & lt));
+        }
+    }
+    __syncthreads();
+    {
+        const u32 c = (tid < 256) ? cnt[tid] : 0u;
+        u32 tot;
+        const u32 ex = block_scan_excl<u32, THREADS>(c, scratch, &tot);
+        if (tid < 256) excl[tid] = ex;
+        __syncthreads();
+        if (tid < plan.ndigits) {
+            const u32 first = excl[tid * 16], end = (tid + 1 < 16) ? excl[(tid + 1) * 16] : tot;
+            const u32 cd = end - first;
+            unsigned long long r = 0;
+            if (cd) r = atomicAdd(&plan.cursor[tid], (unsigned long long)cd);
+            goff[tid] = r - first;
+        }
+    }
+    u64 key[ITEMS];
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 i = tid + j * THREADS;
+        key[j] = (i < count) ? skeys[i] : 0ull;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 i = tid + j * THREADS;
+        if (i < count) {
+            const u32 d = slot[j] >> 16, p = excl[d * 16 + (tid >> 5)] + (slot[j] & 0xffffu);
+            skeys[p] = key[j];
+            sdig[p] = (unsigned char)d;
+            slot[j] = p;
+        }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 p = tid + j * THREADS;
+        if (p < count) {
+            const u32 d = sdig[p];
+            ((u64 *)peers.base[d])[goff[d] + p] = skeys[p];
+        }
+    }
+    __syncthreads(); // the staging buffer takes the ids now
+    u32 *sids = reinterpret_cast<u32 *>(skeys);
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 i = tid + j * THREADS;
+        if (i < count) sids[slot[j]] = ld_stream_u32(ids + begin + i);
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 p = tid + j * THREADS;
+        if (p < count) {
+            const u32 d = sdig[p];
+            ((u32 *)peers.base[d])[goff[d] + p + idr.id_delta[d]] = sids[p];
+        }
+    }
+}
+
+// 256-bin histogram of (key - base) >> shift over a wide run (the counts every rank all-gathers
+// before k_push_wide)
+__global__ void __launch_bounds__(512)
+k_hist_wide(const u64 *__restrict__ keys, u64 n, u64 base, int shift, u32 *__restrict__ ghist)
+{
+    __shared__ u32 sh[256];
+    if (threadIdx.x < 256) sh[threadIdx.x] = 0;
+    __syncthreads();
+    const u64 stride = (u64)gridDim.x * 1024;
+    for (u64 e = ((u64)blockIdx.x * 512 + threadIdx.x) * 2; e < n; e += stride) {
+        if (e + 1 < n) {
+            u64 a, b;
+            ld_stream_u64x2(keys + e, a, b);
+            atomicAdd(&sh[(u32)((a - base) >> shift) & 255u], 1u);
+            atomicAdd(&sh[(u32)((b - base) >> shift) & 255u], 1u);
+        } else {
+            atomicAdd(&sh[(u32)((keys[e] - base) >> shift) & 255u], 1u);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 256 && sh[threadIdx.x]) atomicAdd(&ghist[threadIdx.x], sh[threadIdx.x]);
+}
+
+// out[0] = max(~w), out[1] = max(w) over n words (out zeroed first): the smallest and largest word
+// in the form the ranks' all-reduce (a max) combines
+__global__ void __launch_bounds__(256)
+k_minmax_u64(const u64 *__restrict__ w, u64 n, unsigned long long *__restrict__ out)
+{
+    u64 lo = ~0ull, hi = 0;
+    const u64 stride = (u64)gridDim.x * 512;
+    for (u64 e = ((u64)blockIdx.x * 256 + threadIdx.x) * 2; e < n; e += stride) {
+        if (e + 1 < n) {
+            u64 a, b;
+            ld_stream_u64x2(w + e, a, b);
+            lo = min(lo, min(a, b));
+            hi = max(hi, max(a, b));
+        } else {
+            lo = min(lo, w[e]);
+            hi = max(hi, w[e]);
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = min(lo, __shfl_xor_sync(QCE_FULL_MASK, lo, o));
+        hi = max(hi, __shfl_xor_sync(QCE_FULL_MASK, hi, o));
+    }
+    if ((threadIdx.x & 31) == 0) { atomicMax(out, ~lo); atomicMax(out + 1, hi); }
+}
+
+// A packed run widened for a wide exchange: keys[i] = in[i] >> 32, ids[i] = (u32)in[i]
+__global__ void __launch_bounds__(256)
+k_unpack_wide(const u64 *__restrict__ in, u64 n, u64 *__restrict__ keys, u32 *__restrict__ ids)
+{
+    const u64 stride = (u64)gridDim.x * 256;
+    for (u64 i = (u64)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) {
+        const u64 w = ld_stream_u64(in + i);
+        keys[i] = w >> 32;
+        ids[i] = (u32)w;
     }
 }
 

@@ -32,7 +32,7 @@
 #include "qce_comm.cuh"
 #include "qce_arena.hpp"
 
-#define QCE_ABI_VERSION 1
+#define QCE_ABI_VERSION 2
 
 // ------------------------------------------------------------------ handles
 // How the elements of a column / run are spread over the ranks of the node (SURVEY.md 8e).
@@ -45,6 +45,8 @@ struct Dist {
     u32 rel = 0, col = 0;    // ROWS: ids are rows of this rank's window of `rel`; KEYS: sorted by (rel, col)
     int key_bits = 0;        // KEYS: the exchange's key width (splitters sit on its 256-bin boundaries)
     std::vector<uint64_t> split;  // KEYS: world-1 ascending splitters, rank r holds keys in [split[r-1], split[r])
+    bool wide = false;       // KEYS of a wide exchange: the splitters and key_bits are those of key - base
+    u64 base = 0;            // (a splitter of ~0 lies past every key: the cut 2^64 at width 64)
 };
 struct qce_rowids {
     u32 *d;        // device row ids (this rank's share)
@@ -70,7 +72,10 @@ struct qce_tuples {
     bool skewed = false;    // the sort met a heavy key (a sub-bucket over the finish tile): joins take the two-phase route
     u32 *hist256 = nullptr; // device: 256-bin histogram of the top 8 of hist_key_bits key bits (taken by the build
     int hist_key_bits = 0;  // kernels, or by qce_key_histogram); valid while the run is unsorted and unmodified
+    u64 hist_base = 0;      // wide runs (qce_key_histogram_wide): the bins are those of key - hist_base
     std::vector<unsigned int> hist_host; // the same 256 counts on the host
+    bool range_sort = false; // wide run received from an exchange: its keys lie in [key_min, key_max], so
+                             // they agree above bit bitlen(key_min ^ key_max) and only the bits below are sorted
     u64 n_others = 0;         // tuples held by the other ranks
     Dist dist;
     bool sort_pending = false; // sharded: qce_sort_tuples is deferred to the join, which first moves
@@ -189,6 +194,13 @@ inline int bitlen(u64 v)
     return b;
 }
 inline u64 ceil_div(u64 a, u64 b) { return (a + b - 1) / b; }
+// Exchange splitters sit on the boundaries of the 256-bin histogram of the top 8 of key_bits bits
+// (shift = key_bits - 8): the cut before bin b is the key b << shift.  At 64 bits the cut past the
+// last bin would be 2^64, which wraps to 0; it is stored as ~0 instead, a value no other cut takes
+// (they are multiples of 2^56) and that is read back as bin 256 -- past every key.
+inline u64 cut_key(u32 bin, int shift) { return (bin >= 256 && shift >= 56) ? ~0ull : (u64)bin << shift; }
+inline u32 cut_bin(u64 split, int shift) { return split == ~0ull ? 256u : (u32)std::min<u64>(256, split >> shift); }
+inline bool on_bin_boundary(u64 split, int shift) { return split == ~0ull || (split & ((1ull << shift) - 1)) == 0; }
 inline u64 col_key(u32 rel, u32 col) { return ((u64)rel << 32) | col; }
 void row_share(u64 n, u32 rank, u32 world, u64 *begin, u64 *count, u64 *per_out = nullptr)
 {
@@ -2094,7 +2106,7 @@ int qce_sort_tuples(qce_tuples *t)
         // the sort would have noticed a run of few distinct keys (msd_sort); here the statistics have to
         if (t->key_max < ~0ull && t->n / (t->key_max + 1) >= 16) tl_sort_skewed = true;
     } else if (t->wide) {
-        RadixShifts rs = shifts_for(0, t->key_bits, 8);
+        RadixShifts rs = shifts_for(0, t->range_sort ? bitlen(t->key_min ^ t->key_max) : t->key_bits, 8);
         rc = radix_sort(&t->a, &t->ids, t->n, rs);
     } else {
         // the cached histogram counts key >> (hist_key_bits - 8); level A of the MSD sort counts
@@ -2464,6 +2476,27 @@ int qce_key_histogram(const qce_tuples *t, uint32_t key_bits, uint64_t *hist)
     mt->hist_host.assign(tmp.begin(), tmp.end());
     return 0;
 }
+int qce_key_histogram_wide(const qce_tuples *t, uint64_t base, uint32_t width, uint64_t *hist)
+{
+    NEED_INIT();
+    if (!t || !hist) return fail("null argument");
+    if (!t->wide && t->n) return fail("qce_key_histogram_wide takes wide runs (packed runs: qce_key_histogram)");
+    if (width == 0 || width > 64) return fail("key width must be 1..64");
+    qce_tuples *mt = const_cast<qce_tuples *>(t); // cached on the run like the packed histogram
+    if (!mt->hist256 && dalloc(&mt->hist256, QCE_RADIX_BINS) != 0) return -1;
+    u32 *gh = mt->hist256;
+    CK(cudaMemsetAsync(gh, 0, QCE_RADIX_BINS * sizeof(u32), cx().stream));
+    const int shift = width > 8 ? (int)width - 8 : 0;
+    if (t->n) LAUNCH("hist_wide", k_hist_wide, grid_for(2048, t->n, 4), 512, 0, (const u64 *)t->a, t->n, (u64)base, shift, gh);
+    std::vector<u32> tmp(QCE_RADIX_BINS);
+    CK(cudaMemcpyAsync(tmp.data(), gh, QCE_RADIX_BINS * sizeof(u32), cudaMemcpyDeviceToHost, cx().stream));
+    CK(cudaStreamSynchronize(cx().stream));
+    for (int i = 0; i < QCE_RADIX_BINS; i++) hist[i] = tmp[i];
+    mt->hist_key_bits = (int)width;
+    mt->hist_base = base;
+    mt->hist_host.assign(tmp.begin(), tmp.end());
+    return 0;
+}
 
 int qce_partition_tuples(const qce_tuples *t, uint32_t key_bits, const uint64_t *splitters, uint32_t nparts,
                          uint64_t *counts, void **sendbuf)
@@ -2673,6 +2706,27 @@ static int push_scratch(u32 ndigits, const uint64_t *seg_start, const u32 *run_b
     return 0;
 }
 
+// destination rank of each histogram bin: the number of splitters at or below the bin's first key
+static int push_lut(const uint64_t *splitters, uint32_t nparts, int shift, unsigned char *lut)
+{
+    for (u32 k = 0; k + 1 < nparts; k++)
+        if (!on_bin_boundary(splitters[k], shift))
+            return fail("splitter %llu is not on a boundary of the top-8-bit histogram bins", (unsigned long long)splitters[k]);
+    for (u32 b = 0; b < 256; b++) {
+        u32 part = 0;
+        for (u32 k = 0; k + 1 < nparts; k++) part += b >= cut_bin(splitters[k], shift);
+        lut[b] = (unsigned char)part;
+    }
+    return 0;
+}
+// the bytes of a destination's window a push may fill
+static u64 dst_window_bytes()
+{
+    const bool loopback = G.xworld > 1 && G.peers.base[0] && G.peers.base[1] && G.peers.base[1] > G.peers.base[0] &&
+                          (u64)(G.peers.base[1] - G.peers.base[0]) < G.xwin_bytes;
+    return loopback ? (u64)(G.peers.base[1] - G.peers.base[0]) : G.xwin_bytes; // loopback: each fake rank owns a slice
+}
+
 static int push_tuples_impl(const qce_tuples *t, uint32_t key_bits, const uint64_t *splitters, uint32_t nparts,
                             const uint64_t *dst_word_offset, const uint32_t *dst_run_index, qce_rowids **slots_out,
                             uint32_t ncols, const qce_rowids *const *cols, const uint64_t *col_u32_offset);
@@ -2705,24 +2759,13 @@ static int push_tuples_impl(const qce_tuples *t, uint32_t key_bits, const uint64
     if (nparts > 1 && !splitters) return fail("null argument");
     const int bin_shift = key_bits > 8 ? (int)key_bits - 8 : 0;
     unsigned char lut[256];
-    for (u32 b = 0; b < 256; b++) {
-        u32 part = 0;
-        for (u32 k = 0; k + 1 < nparts; k++) {
-            if ((splitters[k] & ((1ull << bin_shift) - 1)) != 0)
-                return fail("splitter %llu is not on a boundary of the top-8-bit histogram bins", (unsigned long long)splitters[k]);
-            if (((u64)b << bin_shift) >= splitters[k]) part++;
-        }
-        lut[b] = (unsigned char)part;
-    }
+    if (push_lut(splitters, nparts, bin_shift, lut) != 0) return -1;
     // a wrong plan must not scribble over a peer's memory: with the run's histogram at hand (the exchange
     // always has it) every destination segment is checked against the window before anything is stored
     if (t->hist_key_bits == (int)key_bits && t->hist_host.size() == QCE_RADIX_BINS) {
         u64 per_dst[QCE_MAX_RANKS] = {0};
         for (u32 b = 0; b < 256; b++) per_dst[lut[b]] += t->hist_host[b];
-        const u64 window_words = (G.xworld && G.peers.base[0] && G.xworld > 1 && G.peers.base[1] &&
-                                  (u64)(G.peers.base[1] - G.peers.base[0]) < G.xwin_bytes && G.peers.base[1] > G.peers.base[0])
-                                     ? (u64)(G.peers.base[1] - G.peers.base[0]) / 8   // loopback: each fake rank owns a slice
-                                     : G.xwin_bytes / 8;
+        const u64 window_words = dst_window_bytes() / 8;
         for (u32 p = 0; p < nparts; p++)
             if (per_dst[p] && dst_word_offset[p] + per_dst[p] > window_words)
                 return fail("push would overrun rank %u's window: words [%llu, +%llu) of %llu", p,
@@ -2753,6 +2796,50 @@ static int push_tuples_impl(const qce_tuples *t, uint32_t key_bits, const uint64
         LAUNCH("push_tuples", (k_push<u64, true, true>), grid, QCE_PUSH_THREADS, 0, (const u64 *)t->a, n, dg, plan, G.peers, dbits, so, pc);
     else
         LAUNCH("push_tuples", (k_push<u64, true, false>), grid, QCE_PUSH_THREADS, 0, (const u64 *)t->a, n, dg, plan, G.peers, dbits, so, pc);
+    dfree_after_push(d_seg); dfree_after_push(d_cur); dfree_after_push(d_run); dfree_after_push(dlut);
+    return 0;
+}
+
+int qce_push_tuples_wide(const qce_tuples *t, uint64_t base, uint32_t width, const uint64_t *splitters, uint32_t nparts,
+                         const uint64_t *dst_word_offset, const uint64_t *dst_id_offset)
+{
+    NEED_INIT();
+    if (!t || !dst_word_offset || !dst_id_offset) return fail("null argument");
+    if (!G.xwin) return fail("no exchange window (qce_xwin_create)");
+    if (!t->wide && t->n) return fail("qce_push_tuples_wide takes wide runs (packed runs: qce_push_tuples)");
+    if (nparts != G.xworld) return fail("nparts (%u) differs from the attached world size (%u)", nparts, G.xworld);
+    if (width == 0 || width > 64) return fail("key width must be 1..64");
+    if (t->n >= (1ull << 32) - 4096) return fail("push of %llu tuples exceeds the per-run limit", (unsigned long long)t->n);
+    if (nparts > 1 && !splitters) return fail("null argument");
+    const int shift = width > 8 ? (int)width - 8 : 0;
+    unsigned char lut[256];
+    if (push_lut(splitters, nparts, shift, lut) != 0) return -1;
+    if (t->hist_key_bits == (int)width && t->hist_base == base && t->hist_host.size() == QCE_RADIX_BINS) {
+        u64 per_dst[QCE_MAX_RANKS] = {0};
+        for (u32 b = 0; b < 256; b++) per_dst[lut[b]] += t->hist_host[b];
+        const u64 bytes = dst_window_bytes();
+        for (u32 p = 0; p < nparts; p++)
+            if (per_dst[p] && ((dst_word_offset[p] + per_dst[p]) * 8 > bytes || (dst_id_offset[p] + per_dst[p]) * 4 > bytes))
+                return fail("push would overrun rank %u's window: key words [%llu, +%llu), ids [%llu, +%llu) of %llu bytes", p,
+                            (unsigned long long)dst_word_offset[p], (unsigned long long)per_dst[p],
+                            (unsigned long long)dst_id_offset[p], (unsigned long long)per_dst[p], (unsigned long long)bytes);
+    }
+    if (t->n == 0) return 0;
+    unsigned long long *d_seg = nullptr, *d_cur = nullptr;
+    u32 *d_run = nullptr, *dlut = nullptr;
+    if (push_scratch(nparts, dst_word_offset, nullptr, &d_seg, &d_run, &d_cur) != 0 || dalloc(&dlut, 64)) return -1;
+    CK(cudaMemcpyAsync(dlut, lut, sizeof lut, cudaMemcpyHostToDevice, cx().stream));
+    PushDigitWide dg;
+    dg.base = base;
+    dg.shift = shift;
+    dg.lut = dlut;
+    WideIdRegions idr;
+    memset(&idr, 0, sizeof idr);
+    for (u32 p = 0; p < nparts; p++) idr.id_delta[p] = dst_id_offset[p] - dst_word_offset[p];
+    PushPlan plan{d_seg, d_run, d_cur, nparts, 1u};
+    const u32 n = (u32)t->n, grid = (u32)ceil_div(n, PushTile<u64>::TILE);
+    LAUNCH("push_wide", k_push_wide, grid, QCE_PUSH_THREADS, 0, (const u64 *)t->a, (const u32 *)t->ids, n, dg, plan, G.peers,
+           bitlen(nparts - 1), idr);
     dfree_after_push(d_seg); dfree_after_push(d_cur); dfree_after_push(d_run); dfree_after_push(dlut);
     return 0;
 }
@@ -2906,6 +2993,31 @@ int qce_tuples_from_window(uint64_t word_offset, uint64_t n, uint32_t key_bits, 
     if (word_offset & 1) return fail("runs in the window start on 16-byte boundaries");
     return tuples_from_device(G.peers.base[G.xrank] + word_offset * 8, n, key_bits, id_bound, key_lo, key_hi, true, out);
 }
+int qce_tuples_from_window_wide(uint64_t word_offset, uint64_t id_u32_offset, uint64_t n, uint32_t id_bound, uint64_t key_lo,
+                                uint64_t key_hi, qce_tuples **out)
+{
+    NEED_INIT();
+    if (!G.xwin) return fail("no exchange window (qce_xwin_create)");
+    if (!out) return fail("null argument");
+    if ((word_offset + n) * 8 > G.xwin_bytes || (id_u32_offset + n) * 4 > G.xwin_bytes)
+        return fail("run of %llu tuples at words %llu / ids %llu exceeds the exchange window", (unsigned long long)n,
+                    (unsigned long long)word_offset, (unsigned long long)id_u32_offset);
+    if ((word_offset & 1) || (id_u32_offset & 3)) return fail("runs in the window start on 16-byte boundaries");
+    if (n && key_hi < key_lo) return fail("empty key range [%llu, %llu]", (unsigned long long)key_lo, (unsigned long long)key_hi);
+    qce_tuples *t = new qce_tuples();
+    t->a = (u64 *)(G.peers.base[G.xrank] + word_offset * 8); // not from the arena: freeing the run leaves the window alone
+    t->ids = (u32 *)(G.peers.base[G.xrank] + id_u32_offset * 4);
+    t->n = n;
+    t->wide = true;
+    t->key_bits = bitlen(key_hi) ? bitlen(key_hi) : 1;
+    t->key_min = key_lo;
+    t->key_max = key_hi;
+    t->range_sort = true;
+    t->id_bound = id_bound;
+    t->sorted = false;
+    *out = t;
+    return 0;
+}
 int qce_rowids_from_window(uint64_t u32_offset, uint64_t n, uint32_t id_min, uint32_t id_bound, int bucketed,
                            qce_rowids **out)
 {
@@ -3000,7 +3112,7 @@ int exchange_plan_impl(const uint64_t *hists, uint32_t world, uint32_t rank, uin
     if (!hists || !ncols || !splitters || !recv || !before || !run_off || !col_off || !window_bytes || !sent_tuples)
         return fail("null argument");
     if (world < 1 || world > QCE_MAX_RANKS || rank >= world || nsides < 1 || nsides > 8) return fail("bad exchange shape");
-    if (key_bits == 0 || key_bits > 32) return fail("packed runs carry keys of 1..32 bits");
+    if (key_bits == 0 || key_bits > 64) return fail("key width must be 1..64");
     const int shift = key_bits > 8 ? (int)key_bits - 8 : 0;
     // global histogram -> splitters on bin boundaries that balance tuples per rank
     u64 cum[256], total = 0;
@@ -3020,12 +3132,12 @@ int exchange_plan_impl(const uint64_t *hists, uint32_t world, uint32_t rank, uin
         while (i < 256 && (unsigned __int128)cum[i] * world < (unsigned __int128)total * k) i++;
         u32 b = i + 1;
         if (fixed_splitters) { // a run already in place dictates the cut (must sit on a bin boundary)
-            if (fixed_splitters[k - 1] & ((1ull << shift) - 1)) return fail("fixed splitter off the histogram bins");
-            b = (u32)std::min<u64>(256, fixed_splitters[k - 1] >> shift);
+            if (!on_bin_boundary(fixed_splitters[k - 1], shift)) return fail("fixed splitter off the histogram bins");
+            b = cut_bin(fixed_splitters[k - 1], shift);
         }
         if (b < prev) b = prev;
         if (b > 256) b = 256;
-        splitters[k - 1] = (u64)b << shift;
+        splitters[k - 1] = cut_key(b, shift);
         prev = b;
         bnd[k] = b;
     }

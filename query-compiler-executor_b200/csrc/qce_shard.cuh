@@ -197,19 +197,26 @@ struct XRecv {
 };
 // sort_received: the received runs are sorted here, the first one on the context's aux stream as
 // soon as ITS tuples have landed everywhere -- while the second side's push still crosses NVLink.
+// wide_base != nullptr: every side is wide, binned by key - *wide_base over key_bits (1..64) bits; a
+// side's ids are laid out like one travelling column behind its keys.
 int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u64 key_max, const Dist *fixed,
-                  std::vector<XRecv> *out, Dist *dist_out, bool sort_received = false)
+                  std::vector<XRecv> *out, Dist *dist_out, bool sort_received = false, const u64 *wide_base = nullptr)
 {
     static int overlap = -1; // QCE_OVERLAP_PUSH=0: one barrier after all pushes, sorts afterwards
     if (overlap < 0) { const char *e = getenv("QCE_OVERLAP_PUSH"); overlap = e ? atoi(e) : 1; }
     const u32 W = G.world, me = G.rank, ns = (u32)sides.size();
+    const bool wide = wide_base != nullptr;
+    const u64 base = wide ? *wide_base : 0;
     std::vector<uint64_t> hists((size_t)ns * 256), all((size_t)W * ns * 256);
-    for (u32 k = 0; k < ns; k++)
-        if (qce_key_histogram(sides[k], (u32)key_bits, hists.data() + (size_t)k * 256) != 0) { qcecomm::abort_all(); return -1; }
+    for (u32 k = 0; k < ns; k++) {
+        const int rc = wide ? qce_key_histogram_wide(sides[k], base, (u32)key_bits, hists.data() + (size_t)k * 256)
+                            : qce_key_histogram(sides[k], (u32)key_bits, hists.data() + (size_t)k * 256);
+        if (rc != 0) { qcecomm::abort_all(); return -1; }
+    }
     CQ(qcecomm::allgather(hists.data(), hists.size() * sizeof(uint64_t), all.data()));
     std::vector<uint32_t> ncols(ns, 0);
     size_t total_cols = 0;
-    for (u32 k = 0; k < ns; k++) { ncols[k] = (u32)sides[k]->attached.size(); total_cols += ncols[k]; }
+    for (u32 k = 0; k < ns; k++) { ncols[k] = wide ? 1u : (u32)sides[k]->attached.size(); total_cols += ncols[k]; }
     std::vector<uint64_t> splitters(W), recv((size_t)ns * W), before((size_t)ns * W), run_off((size_t)ns * W),
         col_off((total_cols ? total_cols : 1) * W), sent(ns);
     uint64_t need = 0;
@@ -230,7 +237,11 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
         std::vector<uint64_t> dst_words(W);
         for (u32 d = 0; d < W; d++) dst_words[d] = run_off[(size_t)k * W + d] / 8 + before[(size_t)k * W + d];
         int rc;
-        if (ncols[k] == 0) {
+        if (wide) {
+            std::vector<uint64_t> dst_ids(W);
+            for (u32 d = 0; d < W; d++) dst_ids[d] = col_off[col_at * W + d] / 4 + before[(size_t)k * W + d];
+            rc = qce_push_tuples_wide(sides[k], base, (u32)key_bits, splitters.data(), W, dst_words.data(), dst_ids.data());
+        } else if (ncols[k] == 0) {
             rc = qce_push_tuples(sides[k], (u32)key_bits, splitters.data(), W, dst_words.data(), nullptr, nullptr);
         } else {
             // payload := index in the receiver's run; the attached columns follow in the same kernel, laid
@@ -249,13 +260,18 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
     }
     cx().defer_frees = false;
     if (!split && fence_barrier() != 0) return -1; // every peer's stores into this rank's window have completed
-    const u64 lo = me > 0 ? splitters[me - 1] : 0;
+    u64 lo = me > 0 ? splitters[me - 1] : 0;
     // the last rank's range ends at the largest key that exists, not at 2^key_bits - 1: the
     // local sort sizes its MSD buckets from this range
-    const u64 hi = me < W - 1 ? splitters[me] - 1 : key_max;
+    u64 hi = me < W - 1 ? splitters[me] - 1 : key_max;
+    if (wide) { // base + [cut, next cut), clipped to the largest key (base + a cut past it may overflow)
+        const u64 span = key_max - base, c0 = me > 0 ? splitters[me - 1] : 0, c1 = me < W - 1 ? splitters[me] : ~0ull;
+        lo = base + std::min(c0, span);
+        hi = (c1 == ~0ull || c1 > span) ? key_max : base + c1 - 1;
+    }
     out->assign(ns, XRecv());
     cudaStream_t main_stream = cx().stream;
-    for (u32 k = 0; k < ns; k++) {
+    for (u32 k = 0, id_col = 0; k < ns; id_col += ncols[k], k++) {
         if (split) {
             // side k has landed on every rank: this rank's push of it is done, and so is everybody else's
             cudaError_t e = cudaEventSynchronize(cx().ev_side[k]);
@@ -263,8 +279,11 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
             CQ(qcecomm::barrier());
         }
         const u64 n = recv[(size_t)k * W + me];
-        if (qce_tuples_from_window(run_off[(size_t)k * W + me] / 8, n, (u32)key_bits, sides[k]->id_bound, lo, std::max(lo, hi),
-                                   &(*out)[k].run) != 0) {
+        const int vrc = wide ? qce_tuples_from_window_wide(run_off[(size_t)k * W + me] / 8, col_off[(size_t)id_col * W + me] / 4, n,
+                                                           sides[k]->id_bound, lo, std::max(lo, hi), &(*out)[k].run)
+                             : qce_tuples_from_window(run_off[(size_t)k * W + me] / 8, n, (u32)key_bits, sides[k]->id_bound, lo,
+                                                      std::max(lo, hi), &(*out)[k].run);
+        if (vrc != 0) {
             qcecomm::abort_all();
             return -1;
         }
@@ -291,7 +310,7 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
     }
     if (split) release_deferred(); // the pushes that read this scratch have completed (ev_side[1])
     col_at = 0;
-    for (u32 k = 0; k < ns; k++) {
+    for (u32 k = 0; k < ns && !wide; k++) { // (a wide side's one column is its ids, part of the run's view)
         const u64 n = recv[(size_t)k * W + me];
         for (u32 c = 0; c < ncols[k]; c++) {
             qce_rowids *view = nullptr;
@@ -307,16 +326,68 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
     dist_out->kind = Dist::KEYS;
     dist_out->key_bits = key_bits;
     dist_out->split.assign(splitters.begin(), splitters.begin() + (W - 1));
+    dist_out->wide = wide;
+    dist_out->base = base;
     return 0;
 }
 
-bool splitters_fit(const Dist &d, int key_bits)
+bool splitters_fit(const Dist &d, int key_bits, bool wide = false, u64 base = 0)
 {
-    if (d.kind != Dist::KEYS || d.key_bits != key_bits || d.split.size() + 1 != G.world) return false;
+    if (d.kind != Dist::KEYS || d.wide != wide || d.base != base || d.key_bits != key_bits || d.split.size() + 1 != G.world)
+        return false;
     const int shift = key_bits > 8 ? key_bits - 8 : 0;
     for (u64 s : d.split)
-        if (s & ((1ull << shift) - 1)) return false;
+        if (!on_bin_boundary(s, shift)) return false;
     return true;
+}
+// a wide exchange's layout holds every key of [gmin, gmax]: its bins cover them
+bool wide_range_fits(const Dist &d, u64 gmin, u64 gmax)
+{
+    return d.kind == Dist::KEYS && d.wide && d.split.size() + 1 == G.world && d.base <= gmin &&
+           bitlen(gmax - d.base) <= d.key_bits;
+}
+
+// the smallest and largest key of a run on this rank, as {~min, max} (packed words: the key is the high half)
+int local_key_range(const qce_tuples *t, uint64_t *v)
+{
+    if (t->n == 0) return 0;
+    CK(cudaMemsetAsync(cx().d_scalars + 8, 0, 2 * sizeof(u64), cx().stream));
+    LAUNCH("key_range", k_minmax_u64, grid_for(512, t->n, 4), 256, 0, (const u64 *)t->a, t->n, cx().d_scalars + 8);
+    if (read_scalars(10) != 0) return -1;
+    const int drop = t->wide ? 0 : 32;
+    v[0] = std::max<uint64_t>(v[0], ~(~cx().h_scalars[8] >> drop));
+    v[1] = std::max<uint64_t>(v[1], cx().h_scalars[9] >> drop);
+    return 0;
+}
+// ... over both runs and all ranks: one all-reduce of two words
+int global_key_range(const qce_tuples *R, const qce_tuples *S, u64 *gmin, u64 *gmax)
+{
+    uint64_t v[2] = {0, 0};
+    if (local_key_range(R, v) != 0 || local_key_range(S, v) != 0) { qcecomm::abort_all(); return -1; }
+    CQ(qcecomm::allreduce_max(v, 2));
+    *gmin = ~v[0];
+    *gmax = v[1];
+    return 0;
+}
+
+// a packed run as a wide one (12 B per tuple), for a join whose other side has keys >= 2^32
+int widen(const qce_tuples *in, qce_tuples **out)
+{
+    qce_tuples *t = new qce_tuples();
+    t->n = in->n;
+    t->n_others = in->n_others;
+    t->wide = true;
+    t->key_bits = in->key_bits;
+    t->key_min = in->key_min;
+    t->key_max = in->key_max;
+    t->id_bound = in->id_bound;
+    t->sorted = false;
+    t->sort_pending = in->sort_pending;
+    t->dist.kind = Dist::ANY;
+    if (dalloc(&t->a, t->n) != 0 || dalloc(&t->ids, t->n) != 0) { qce_tuples_free(t); return -1; }
+    if (t->n) LAUNCH("widen", k_unpack_wide, grid_for(2048, t->n), 256, 0, (const u64 *)in->a, t->n, t->a, t->ids);
+    *out = t;
+    return 0;
 }
 
 int merge_join_any(const qce_tuples *R, const qce_tuples *S, bool want_r, bool want_s, qce_rowids **outR,
@@ -325,20 +396,27 @@ int merge_join_any(const qce_tuples *R, const qce_tuples *S, bool want_r, bool w
 // Sort-merge join of two distributed runs (join_relations, src/join.c:325-392).  A run whose
 // sort is pending is exchanged by key range and sorted by its new owner; a run that is already
 // in key order over the ranks (the output side of an earlier join on the same column) stays
-// where it is and lends its splitters.
+// where it is and lends its splitters.  When either side has keys >= 2^32 both sides are
+// exchanged wide (a packed side is widened first), binned by key - (smallest key) over the
+// width of the key range.  Only the pointer walk over an unsorted run gathers on rank 0.
 int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_rowids **outR, qce_rowids **outS, bool walk)
 {
     if (outR) *outR = nullptr;
     if (outS) *outS = nullptr;
-    const bool root_only = walk || R->wide || S->wide;
+    const bool root_only = walk, wide = R->wide || S->wide;
     int rc = -1;
     qce_tuples *lr = nullptr, *ls = nullptr;  // the local inputs of the merge
     bool own_r = false, own_s = false, travelled_r = false, travelled_s = false;
+    int trace_bits = std::max(R->key_bits, S->key_bits);
     Dist dist;
     dist.kind = Dist::ANY;
     if (root_only && (!R->attached.empty() || !S->attached.empty())) {
         qcecomm::abort_all();
         return fail("position-carrying runs cannot take the rank-0 fallback");
+    }
+    if (wide && (!R->attached.empty() || !S->attached.empty())) {
+        qcecomm::abort_all();
+        return fail("position-carrying runs need keys below 2^32 on both sides");
     }
     if (R->n + R->n_others == 0 || S->n + S->n_others == 0) {
         // an empty side: the pointer walk never starts (src/join.c:342), whatever the other side holds
@@ -357,23 +435,42 @@ int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_row
             rc = merge_join_any(lr, ls, want_r, want_s, outR, outS, walk);
         }
     } else {
-        const int key_bits = std::max(R->key_bits, S->key_bits);
-        const u64 key_max = std::max(R->key_max, S->key_max);
+        int key_bits = std::max(R->key_bits, S->key_bits);
+        u64 key_max = std::max(R->key_max, S->key_max), base = 0;
         bool push_r = R->sort_pending, push_s = S->sort_pending;
+        if (wide) {
+            u64 gmin, gmax;
+            if (global_key_range(R, S, &gmin, &gmax) != 0) return -1;
+            key_max = gmax;
+            // a side in place on a wide layout that covers every key lends its base and width
+            const Dist *in_place = !push_r && wide_range_fits(R->dist, gmin, gmax) ? &R->dist
+                                 : !push_s && wide_range_fits(S->dist, gmin, gmax) ? &S->dist : nullptr;
+            base = in_place ? in_place->base : gmin;
+            key_bits = in_place ? in_place->key_bits : std::max(1, bitlen(gmax - gmin));
+        }
+        trace_bits = key_bits;
         // a side that claims to be in place must really be laid out on this exchange's bins
-        if (!push_r && !splitters_fit(R->dist, key_bits)) push_r = true;
-        if (!push_s && !splitters_fit(S->dist, key_bits)) push_s = true;
+        if (!push_r && !splitters_fit(R->dist, key_bits, wide, base)) push_r = true;
+        if (!push_s && !splitters_fit(S->dist, key_bits, wide, base)) push_s = true;
         if (!push_r && !push_s && R->dist.split != S->dist.split) push_s = true;
         const Dist *fixed = !push_r ? &R->dist : (!push_s ? &S->dist : nullptr);
-        std::vector<const qce_tuples *> sides;
-        if (push_r) sides.push_back(R);
-        if (push_s) sides.push_back(S);
-        std::vector<XRecv> got;
-        if (sides.empty()) {
-            dist = R->dist;
-        } else if (exchange_runs(sides, key_bits, key_max, fixed, &got, &dist, true) != 0) {
+        // a packed side of a wide join is pushed (its layout cannot fit) and travels widened
+        qce_tuples *wr = nullptr, *ws = nullptr;
+        if (wide && ((!R->wide && widen(R, &wr) != 0) || (!S->wide && widen(S, &ws) != 0))) {
+            qce_tuples_free(wr);
+            qcecomm::abort_all();
             return -1;
         }
+        std::vector<const qce_tuples *> sides;
+        if (push_r) sides.push_back(wr ? wr : R);
+        if (push_s) sides.push_back(ws ? ws : S);
+        std::vector<XRecv> got;
+        int xrc = 0;
+        if (sides.empty()) dist = R->dist;
+        else xrc = exchange_runs(sides, key_bits, key_max, fixed, &got, &dist, true, wide ? &base : nullptr);
+        qce_tuples_free(wr); // the received copies live in the window
+        qce_tuples_free(ws);
+        if (xrc != 0) return -1;
         size_t at = 0;
         if (push_r) { travelled_r = got[at].travelled; lr = got[at++].run; } else lr = R;
         if (push_s) { travelled_s = got[at].travelled; ls = got[at++].run; } else ls = S;
@@ -382,6 +479,12 @@ int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_row
         LocalScope ls_; // the received runs were sorted inside the exchange
         rc = merge_join_any(lr, ls, want_r, want_s, outR, outS, false);
     }
+    static const bool trace = getenv("QCE_TRACE") != nullptr;
+    if (trace) // route "local": a side is empty everywhere, nothing moves
+        fprintf(stderr, "[qce] join rank %u/%u: route=%s keys=%s width=%d recv R=%llu/%llu S=%llu/%llu\n", G.rank, G.world,
+                !lr ? "local" : root_only ? "root" : "exchange", wide ? "wide" : "packed", trace_bits,
+                (unsigned long long)(lr ? lr->n : 0), (unsigned long long)(R->n + R->n_others), (unsigned long long)(ls ? ls->n : 0),
+                (unsigned long long)(S->n + S->n_others));
     if (own_r) qce_tuples_free(lr);
     if (own_s) qce_tuples_free(ls);
     if (rc != 0) { qcecomm::abort_all(); return -1; }

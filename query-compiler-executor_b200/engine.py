@@ -38,6 +38,7 @@ SYMBOLS = [
     "qce_comm_finish", "qce_upload_column_window", "qce_upload_column_window_device", "qce_row_share",
     "qce_set_replicate_bytes", "qce_column_would_be_whole", "qce_column_is_whole", "qce_rowids_count_local", "qce_xwin_unmap_peers", "qce_build_tuples_positions", "qce_merge_join_stats",
     "qce_elision_supported", "qce_tuples_attach", "qce_placement_cap",
+    "qce_key_histogram_wide", "qce_push_tuples_wide", "qce_tuples_from_window_wide",
 ]
 
 
@@ -108,6 +109,9 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
         "qce_rowids_count_local": (u64, [vp]), "qce_xwin_unmap_peers": (i32, []),
         "qce_build_tuples_positions": (i32, [u32, u32, vp, P(vp)]),
         "qce_merge_join_stats": (i32, [vp, vp, P(vp), P(vp), P(u32), P(u32)]), "qce_elision_supported": (i32, []), "qce_tuples_attach": (i32, [vp, u32, vp]), "qce_placement_cap": (i32, [vp, u32, P(u64)]),
+        "qce_key_histogram_wide": (i32, [vp, u64, u32, P(u64)]),
+        "qce_push_tuples_wide": (i32, [vp, u64, u32, vp, u32, vp, vp]),
+        "qce_tuples_from_window_wide": (i32, [u64, u64, u64, u32, u64, u64, P(vp)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -320,6 +324,11 @@ class Engine:
         self._ck(self.lib.qce_key_histogram(t, key_bits, out.ctypes.data_as(C.POINTER(C.c_uint64))))
         return out
 
+    def key_histogram_wide(self, t: int, base: int, width: int) -> np.ndarray:
+        out = np.zeros(256, dtype=np.uint64)
+        self._ck(self.lib.qce_key_histogram_wide(t, base, width, out.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return out
+
     def partition_tuples(self, t: int, key_bits: int, splitters, nparts: int):
         sp = _u64(splitters if len(splitters) else [0])
         counts = (C.c_uint64 * nparts)()
@@ -380,6 +389,12 @@ class Engine:
         self._ck(self.lib.qce_push_tuples_cols(t, key_bits, sp.ctypes.data, nparts, off.ctypes.data, ri.ctypes.data,
                                                len(cols), ca, co.ctypes.data))
 
+    def push_tuples_wide(self, t: int, base: int, width: int, splitters, nparts: int, dst_word_offset,
+                         dst_id_offset) -> None:
+        sp = _u64(splitters if len(splitters) else [0])
+        off, ido = _u64(dst_word_offset), _u64(dst_id_offset)
+        self._ck(self.lib.qce_push_tuples_wide(t, base, width, sp.ctypes.data, nparts, off.ctypes.data, ido.ctypes.data))
+
     def push_u32_by_slot(self, vals: int, slots: int, nparts: int, dst_u32_offset) -> None:
         off = _u64(dst_u32_offset)
         self._ck(self.lib.qce_push_u32_by_slot(vals, slots, nparts, off.ctypes.data))
@@ -418,6 +433,12 @@ class Engine:
                            key_lo: int = 0, key_hi: int = 0) -> int:
         h = C.c_void_p()
         self._ck(self.lib.qce_tuples_from_window(word_offset, n, key_bits, id_bound, key_lo, key_hi, C.byref(h)))
+        return h.value
+
+    def tuples_from_window_wide(self, word_offset: int, id_u32_offset: int, n: int, id_bound: int = 0,
+                                key_lo: int = 0, key_hi: int = 0) -> int:
+        h = C.c_void_p()
+        self._ck(self.lib.qce_tuples_from_window_wide(word_offset, id_u32_offset, n, id_bound, key_lo, key_hi, C.byref(h)))
         return h.value
 
     def rowids_from_window(self, u32_offset: int, n: int, id_bound: int = 0, bucketed: bool = False, id_min: int = 0) -> int:

@@ -480,6 +480,7 @@ int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs, int digit_b
     if (n >= (1ull << 30)) return fail("sort of %llu tuples exceeds the 2^30 per-run limit", (unsigned long long)n);
     if (n <= BS_TILE) {
         // small run: the whole sort in one CTA (k_block_sort), in place
+        if (digit_bits != 8) return fail("internal: the block sort ranks 8-bit digits, not %d-bit ones", digit_bits);
         const size_t smem = BS_TILE * sizeof(u64) + (vals ? BS_TILE * sizeof(u32) : 0) +
                             ((BS_THREADS / 32) * 256 + 256 + 33) * sizeof(u32);
         static bool attr_k = false, attr_kv = false;
@@ -825,7 +826,8 @@ int sort_packed(u64 **a, u64 n, int key_bits, u64 key_min, u64 key_max, const u3
     if (key_min > key_max) key_min = 0;
     if (msd_sort(a, n, key_min, key_max, &done, hist_top8, hist_key_bits) != 0) return -1;
     if (done) return 0;
-    const int db = digit_bits_for(key_bits, true);
+    // k_block_sort ranks 8-bit digits: 9-bit shifts would skip every ninth key bit
+    const int db = n <= BS_TILE ? 8 : digit_bits_for(key_bits, true);
     RadixShifts rs = shifts_for(32, key_bits, db);
     return radix_sort(a, nullptr, n, rs, db);
 }

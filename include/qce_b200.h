@@ -141,6 +141,10 @@ int qce_column_is_whole(uint32_t rel, uint32_t col); /* 1 whole / 0 row-sharded 
 /* Adopt a device buffer without copying (caller keeps ownership, must outlive use). */
 int qce_adopt_column_device(uint32_t rel, uint32_t col, const void *dev, uint64_t n);
 int qce_column_info(uint32_t rel, uint32_t col, uint64_t *n, uint64_t *max_value);
+/* The histogram of key >> (*key_bits - 8) over a whole column, *key_bits = bit length of its maximum,
+ * counted with the statistics the upload takes; bins[256].  *key_bits = 0 (bins untouched) when the
+ * column has none: row windows, fewer than 2^20 rows, or a maximum outside [2^8, 2^32). */
+int qce_column_histogram(uint32_t rel, uint32_t col, uint32_t *bins, int *key_bits);
 int qce_drop_relations(void);
 
 /* ---- filter operator -----------------------------------------------------
@@ -178,6 +182,13 @@ int qce_build_tuples_rowids(uint32_t rel, uint32_t col, const qce_rowids *ids, q
  * unspecified, as in the reference (its quicksort is rand()-driven): runs below
  * 2^20 tuples are sorted stably, larger ones may take the MSD partition path. */
 int qce_sort_tuples(qce_tuples *t);
+/* qce_build_tuples_base followed by qce_sort_tuples, in one call: the same run, sorted, with the same
+ * unspecified order among equal keys.  A large whole column whose run takes the MSD route is never
+ * stored unsorted: the first partition level reads the column and forms the tuples on the fly, which
+ * saves one write and one read of the whole run.  Every other run (several ranks, keys of 2^32 or
+ * more, a column stored in key order, a small or dense one) is built, then sorted.  Like
+ * qce_sort_tuples, it takes a sorted run from the batch's cache and leaves one there. */
+int qce_build_sorted_tuples_base(uint32_t rel, uint32_t col, qce_tuples **out);
 /* 1 if keys are non-decreasing (the reference never checks; the host layer
  * uses it to refuse JOIN_SORT_* merges over unsorted input, SURVEY 8a-10). */
 int qce_tuples_is_sorted(const qce_tuples *t, int *sorted);

@@ -754,12 +754,31 @@ k_checksum(const u32 *__restrict__ ids, u64 n, ChecksumCols cols, u64 *__restric
 // Sum of a base column over all its rows (projection of an unfiltered binding
 // never happens in the reference -- every projected binding has a mid result --
 // but the sharded driver uses it for load-time fingerprints).
+// HIST: the same pass also counts every key below 2^32 in the bin (L, top) of its bit length L and its
+// top 8 bits up to and including the leading one (the key itself when L < 8): 33 x 256 counters in
+// lhist.  The column's bit length b is only known once the pass is over; from these counters the
+// level-A histogram of the MSD sort, key >> (b - 8), folds exactly for any 9 <= b <= 32
+// (k_column_hist_fold).  A block folds the rows L <= bitlen(block max) - 8 into bin (0, 0) itself:
+// every such b puts those keys in digit 0.
+#define QCE_LEN_BINS (33 * 256)
+__device__ __forceinline__ void len_count(u32 *sh, u64 k)
+{
+    const int L = 64 - __clzll((long long)k);
+    if (L <= 32) atomicAdd(&sh[L * 256 + (L >= 8 ? (u32)(k >> (L - 8)) : (u32)k)], 1u);
+}
+template <bool HIST>
 __global__ void __launch_bounds__(256)
-k_column_stats(const u64 *__restrict__ col, u64 n, u64 *__restrict__ max_out, u32 *__restrict__ unordered)
+k_column_stats(const u64 *__restrict__ col, u64 n, u64 *__restrict__ max_out, u32 *__restrict__ unordered,
+               u32 *__restrict__ lhist)
 {
     // max(column) sizes the sort passes; *unordered stays 0 when the column is stored in ascending order (a primary
     // key usually is): a run built from it is sorted as it stands and its sort is skipped (qce_sort_tuples)
     __shared__ u64 smax[8];
+    __shared__ u32 sh[HIST ? QCE_LEN_BINS : 1];
+    if (HIST) {
+        for (int i = threadIdx.x; i < QCE_LEN_BINS; i += 256) sh[i] = 0;
+        __syncthreads();
+    }
     u64 m = 0;
     bool bad = false;
     const u64 stride = (u64)gridDim.x * 512;
@@ -770,8 +789,11 @@ k_column_stats(const u64 *__restrict__ col, u64 n, u64 *__restrict__ max_out, u3
             m = max(m, max(a, b));
             bad |= a > b;
             if (e + 2 < n) bad |= b > col[e + 2];
+            if (HIST) { len_count(sh, a); len_count(sh, b); }
         } else {
-            m = max(m, col[e]);
+            const u64 a = col[e];
+            m = max(m, a);
+            if (HIST) len_count(sh, a);
         }
     }
     if (__any_sync(QCE_FULL_MASK, bad) && (threadIdx.x & 31) == 0) atomicOr(unordered, 1u);
@@ -779,9 +801,33 @@ k_column_stats(const u64 *__restrict__ col, u64 n, u64 *__restrict__ max_out, u3
     for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(QCE_FULL_MASK, m, o));
     if ((threadIdx.x & 31) == 0) smax[threadIdx.x >> 5] = m;
     __syncthreads();
-    if (threadIdx.x == 0) {
 #pragma unroll
-        for (int w = 1; w < 8; w++) m = max(m, smax[w]);
-        atomicMax(max_out, m);
+    for (int w = 0; w < 8; w++) m = max(m, smax[w]);
+    if (threadIdx.x == 0) atomicMax(max_out, m);
+    if (HIST) {
+        const int low = (64 - __clzll((long long)m)) - 8; // rows up to this one are digit 0 for the column
+        u32 zero = 0;
+        for (int L = 0; L <= 32; L++) {
+            const u32 c = sh[L * 256 + threadIdx.x];
+            if (!c) continue;
+            if (L <= low) zero += c;
+            else atomicAdd(&lhist[L * 256 + threadIdx.x], c);
+        }
+        zero = __reduce_add_sync(QCE_FULL_MASK, zero);
+        if ((threadIdx.x & 31) == 0 && zero) atomicAdd(&lhist[0], zero);
     }
+}
+// One CTA: the level-A histogram (digit key >> (b - 8), b = bit length of the column maximum) from
+// k_column_stats' 33 x 256 counters.
+__global__ void __launch_bounds__(256) k_column_hist_fold(const u32 *__restrict__ lhist, int b, u32 *__restrict__ out)
+{
+    __shared__ u32 sh[256];
+    sh[threadIdx.x] = 0;
+    __syncthreads();
+    for (int L = 0; L <= b; L++) { // rows above b are empty
+        const u32 c = lhist[L * 256 + threadIdx.x];
+        if (c) atomicAdd(&sh[threadIdx.x >> (L >= 8 ? b - L : b - 8)], c);
+    }
+    __syncthreads();
+    out[threadIdx.x] = sh[threadIdx.x];
 }

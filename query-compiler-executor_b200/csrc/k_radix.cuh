@@ -811,6 +811,14 @@ __device__ __forceinline__ void fence_proxy_async()
 constexpr int QCE_MSDB_THREADS = 512, QCE_MSDB_ITEMS = 8;
 constexpr int QCE_MSDB_SLOTS = QCE_MSD_TILE + 2;                 // a misaligned tile start costs up to 2 extra words
 constexpr size_t QCE_MSDB_SMEM = 2 * QCE_MSDB_SLOTS * sizeof(u64); // dynamic shared memory of the kernel
+// FROM_COL: `in` is a whole base column (keys below 2^32) and the tiles are those of one bucket
+// covering it, so tile positions are row ids: the landed word w at position p is the tuple
+// w << 32 | p.  The tuples are formed in registers and never stored unsorted (MSD level A straight
+// from the column, qce_build_sorted_tuples_base).  The column's odd last word is loaded plainly
+// rather than by a bulk copy reaching past its end.
+template <bool FROM_COL> struct MsdbWord { using T = u64; };
+template <> struct MsdbWord<true> { using T = u32; }; // a column word below 2^32: half the registers of a tuple
+template <bool FROM_COL>
 __global__ void __launch_bounds__(QCE_MSDB_THREADS, 3)
 k_msd_partition_bulk(const u64 *__restrict__ in, u64 *__restrict__ out, const MsdTileDesc *__restrict__ desc, u32 ntiles,
                      u64 base, int shift, u32 bins, u32 *__restrict__ cursor)
@@ -831,10 +839,15 @@ k_msd_partition_bulk(const u64 *__restrict__ in, u64 *__restrict__ out, const Ms
         MsdTileDesc d = desc[t];
         sdesc[b] = d;
         if (d.count == 0) return;
-        const u32 first = d.begin & ~1u, last = (d.begin + d.count + 1u) & ~1u; // 16-byte aligned superset
+        const u32 first = d.begin & ~1u, end = d.begin + d.count;
+        u32 last = (end + 1u) & ~1u; // 16-byte aligned superset
+        if (FROM_COL && (end & 1u)) {
+            last = end - 1u;
+            MSDB_BUF(b)[last - first] = in[last];
+        }
         const u32 bytes = (last - first) * (u32)sizeof(u64);
         mbar_expect_tx(&bar[b], bytes);
-        bulk_g2s(MSDB_BUF(b), in + first, bytes, &bar[b]);
+        if (bytes) bulk_g2s(MSDB_BUF(b), in + first, bytes, &bar[b]);
     };
     if (tid == 0) {
         mbar_init(&bar[0], 1);
@@ -855,7 +868,7 @@ k_msd_partition_bulk(const u64 *__restrict__ in, u64 *__restrict__ out, const Ms
         const int b = it & 1;
         const MsdTileDesc d = sdesc[b];
         const u32 count = d.count;
-        u64 key[ITEMS];
+        typename MsdbWord<FROM_COL>::T key[ITEMS];
         u32 slot[ITEMS];
         if (count) {
             mbar_wait(&bar[b], (it >> 1) & 1);
@@ -867,8 +880,9 @@ k_msd_partition_bulk(const u64 *__restrict__ in, u64 *__restrict__ out, const Ms
                 const bool live = i < count;
                 u32 dg = 0;
                 if (live) {
-                    key[j] = src[i];
-                    dg = (u32)((key[j] - base) >> shift) & mask;
+                    key[j] = (typename MsdbWord<FROM_COL>::T)src[i];
+                    const u64 k = FROM_COL ? (u64)key[j] << 32 : (u64)key[j]; // shift >= 32: the row id adds no digit bit
+                    dg = (u32)((k - base) >> shift) & mask;
                 }
                 if (j == 0) agg = bins > 4 && msd_warp_skewed(dg, live);
                 const u32 r = msd_rank(cnt, dg, live, agg);
@@ -891,7 +905,8 @@ k_msd_partition_bulk(const u64 *__restrict__ in, u64 *__restrict__ out, const Ms
 #pragma unroll
         for (int j = 0; j < ITEMS; j++) {
             const u32 i = tid + j * THREADS;
-            if (i < count) stage[excl[slot[j] >> 16] + (slot[j] & 0xffffu)] = key[j];
+            if (i < count)
+                stage[excl[slot[j] >> 16] + (slot[j] & 0xffffu)] = FROM_COL ? ((u64)key[j] << 32) | (d.begin + i) : (u64)key[j];
         }
         __syncthreads();
 #pragma unroll

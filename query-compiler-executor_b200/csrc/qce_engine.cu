@@ -32,7 +32,7 @@
 #include "qce_comm.cuh"
 #include "qce_arena.hpp"
 
-#define QCE_ABI_VERSION 2
+#define QCE_ABI_VERSION 3
 
 // ------------------------------------------------------------------ handles
 // How the elements of a column / run are spread over the ranks of the node (SURVEY.md 8e).
@@ -106,6 +106,10 @@ struct Column {
     void *alloc = nullptr;             // the cudaMalloc behind d (reused by a re-upload of the same shape)
     u64 alloc_bytes = 0;
     std::vector<void *> opened;        // the peers' mappings (cudaIpcCloseMemHandle on drop)
+    // whole columns of 2^20 rows or more with 9 <= hist_bits = bitlen(maxv) <= 32: the 256-bin histogram of
+    // key >> (hist_bits - 8), MSD level A of a run built from the column (taken with the load-time statistics)
+    u32 *hist = nullptr;               // device, cudaMalloc'ed; kept for a re-upload, freed on drop
+    int hist_bits = 0;                 // 0: hist holds nothing
 };
 ColRef ref_of(const Column *c)
 {
@@ -570,14 +574,21 @@ RadixShifts shifts_for(int base_shift, int bits, int digit_bits = QCE_RADIX_BITS
 }
 
 // ---- MSD partition + shared-memory finish (k_radix.cuh) --------------------------
-// For large packed runs.  *done = false means "not applicable or skewed": the
-// caller sorts with the LSD passes instead (the run is left untouched).
 constexpr u32 MSD_LOCAL_CAP = 256 * 16; // tuples the largest k_msd_local_sort shape can hold
 thread_local bool tl_sort_skewed = false; // set by msd_sort: some sub-bucket holds more than the finish tile (a heavy key)
-int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 *hist_top8 = nullptr,
-             int hist_key_bits = 0)
+// The sort runs in three stages: msd_plan decides from the run's length and key range alone whether
+// the MSD route applies; msd_level_a scatters the run by its top 8 key bits, from the packed tuples
+// or straight from a base column (qce_build_sorted_tuples_base); msd_after_level_a does the rest.
+struct MsdPlan {
+    u64 n, base;       // the kernels work on key - key_min: base = key_min << 32
+    int key_bits, P, R, shiftA, shiftB;
+    u32 nbA, nbB, nsub, ntiles0;
+    int shape, variant, bulk; // QCE_MSD_SHAPE / QCE_MSD_VARIANT / QCE_MSD_BULK
+};
+// 1: the MSD route applies; 0: the LSD passes sort the run; -1: error.  Flags a run of few
+// distinct keys in tl_sort_skewed on the way.
+int msd_plan(u64 n, u64 key_min, u64 key_max, MsdPlan *p)
 {
-    *done = false;
     static int enabled = -1;
     if (enabled < 0) {
         const char *e = getenv("QCE_MSD");
@@ -597,31 +608,17 @@ int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 
     int P = 9;
     while (P < 16 && P < key_bits && n / (((key_max >> (key_bits - P)) + 1)) > 2700) P++;
     if (n / (((key_max >> (key_bits - P)) + 1)) > 2700) return 0; // too dense for 16 partition bits: LSD
-    const int P1 = 8, P2 = P - 8, R = key_bits - P;
-    const int shiftA = 32 + key_bits - P1, shiftB = 32 + key_bits - P;
-    const u32 nbA = 256, nbB = 1u << P2, nsub = nbA * nbB;
-    const u32 ntiles0 = (u32)ceil_div(n, QCE_MSD_TILE);
-
-    u64 *alt = nullptr;
-    u32 *lvl0 = nullptr, *histA = nullptr, *offA = nullptr, *curA = nullptr, *tstart1 = nullptr, *histB = nullptr,
-        *suboff = nullptr, *curB = nullptr;
-    Scratch sc; // level A scatters into alt, level B back into *keys: every buffer here is a temporary
-    if (sc.get(&alt, n) || sc.get(&lvl0, 4) || sc.get(&histA, nbA) || sc.get(&offA, nbA) || sc.get(&curA, nbA) ||
-        sc.get(&tstart1, nbA + 1) || sc.get(&histB, nsub) || sc.get(&suboff, nsub) || sc.get(&curB, nsub))
-        return -1;
-    // level 0: one bucket = the whole run.  lvl0 = {tile_start[0], tile_start[1], bucket_off, bucket_size}
-    const u32 h_lvl0[4] = {0u, ntiles0, 0u, (u32)n};
-    CK(cudaMemcpyAsync(lvl0, h_lvl0, sizeof h_lvl0, cudaMemcpyHostToDevice, cx().stream));
-    CK(cudaMemsetAsync(histA, 0, nbA * sizeof(u32), cx().stream));
-    CK(cudaMemsetAsync(histB, 0, nsub * sizeof(u32), cx().stream));
-    CK(cudaMemsetAsync(cx().d_scalars + 10, 0, sizeof(u64), cx().stream));
-    if (hist_top8 && key_min == 0 && hist_key_bits == key_bits) // level A was counted while the run was built
-        CK(cudaMemcpyAsync(histA, hist_top8, nbA * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
-    else
-        LAUNCH("msd_hist", k_msd_hist, ntiles0, QCE_MSD_THREADS, 0, *keys, lvl0, lvl0 + 2, lvl0 + 3, 1u, base, shiftA, nbA,
-               histA);
-    LAUNCH("radix_bases", k_radix_bases, 1, (int)nbA, 0, histA, offA);
-    CK(cudaMemcpyAsync(curA, offA, nbA * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
+    p->n = n;
+    p->base = base;
+    p->key_bits = key_bits;
+    p->P = P;
+    p->R = key_bits - P;
+    p->shiftA = 32 + key_bits - 8;
+    p->shiftB = 32 + key_bits - P;
+    p->nbA = 256;
+    p->nbB = 1u << (P - 8);
+    p->nsub = p->nbA * p->nbB;
+    p->ntiles0 = (u32)ceil_div(n, QCE_MSD_TILE);
     static int shape = -1; // QCE_MSD_SHAPE: 0 = 256 threads x 16 tuples, 1 = 512 x 8
     if (shape < 0) {
         const char *e = getenv("QCE_MSD_SHAPE");
@@ -636,32 +633,100 @@ int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 
     if (bulk < 0) {
         const char *e = getenv("QCE_MSD_BULK");
         bulk = e ? atoi(e) : 1;
-        if (bulk) CK(cudaFuncSetAttribute(k_msd_partition_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QCE_MSDB_SMEM));
+        if (bulk) {
+            CK(cudaFuncSetAttribute(k_msd_partition_bulk<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QCE_MSDB_SMEM));
+            CK(cudaFuncSetAttribute(k_msd_partition_bulk<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QCE_MSDB_SMEM));
+        }
     }
+    p->shape = shape;
+    p->variant = variant;
+    p->bulk = bulk;
+    return 1;
+}
+
+// Buffers of one MSD sort.  Level A scatters into alt, level B back into the run.
+struct MsdLevels {
+    Scratch sc;
+    u64 *alt = nullptr; // freed with the levels unless a caller takes it
+    u32 *lvl0 = nullptr, *histA = nullptr, *offA = nullptr, *curA = nullptr, *tstart1 = nullptr, *histB = nullptr,
+        *suboff = nullptr, *curB = nullptr;
     MsdTileDesc *tdesc = nullptr;
+    ~MsdLevels() { if (alt) dfree(alt); }
+};
+
+// Level A: scatter the run by its top 8 key bits into m->alt.  `in` is the packed run, or with
+// from_col the base column itself (the bulk partition kernel only).  hist_top8: the level-A
+// histogram when it is already known (taken while the run was built, or with the column statistics).
+int msd_level_a(const MsdPlan &p, MsdLevels *m, const u64 *in, bool from_col, const u32 *hist_top8)
+{
+    const u64 n = p.n, base = p.base;
+    const int shiftA = p.shiftA, shape = p.shape, variant = p.variant;
+    const u32 nbA = p.nbA, nsub = p.nsub, ntiles0 = p.ntiles0;
+    if (from_col && !p.bulk) return fail("internal: level A from a column needs the bulk partition kernel");
+    Scratch &sc = m->sc;
+    if (dalloc(&m->alt, n) || sc.get(&m->lvl0, 4) || sc.get(&m->histA, nbA) || sc.get(&m->offA, nbA) ||
+        sc.get(&m->curA, nbA) || sc.get(&m->tstart1, nbA + 1) || sc.get(&m->histB, nsub) || sc.get(&m->suboff, nsub) ||
+        sc.get(&m->curB, nsub))
+        return -1;
+    u64 *alt = m->alt;
+    u32 *lvl0 = m->lvl0, *histA = m->histA, *offA = m->offA, *curA = m->curA;
+    // level 0: one bucket = the whole run.  lvl0 = {tile_start[0], tile_start[1], bucket_off, bucket_size}
+    const u32 h_lvl0[4] = {0u, ntiles0, 0u, (u32)n};
+    CK(cudaMemcpyAsync(lvl0, h_lvl0, sizeof h_lvl0, cudaMemcpyHostToDevice, cx().stream));
+    CK(cudaMemsetAsync(histA, 0, nbA * sizeof(u32), cx().stream));
+    CK(cudaMemsetAsync(m->histB, 0, nsub * sizeof(u32), cx().stream));
+    CK(cudaMemsetAsync(cx().d_scalars + 10, 0, sizeof(u64), cx().stream));
+    if (hist_top8)
+        CK(cudaMemcpyAsync(histA, hist_top8, nbA * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
+    else
+        LAUNCH("msd_hist", k_msd_hist, ntiles0, QCE_MSD_THREADS, 0, in, lvl0, lvl0 + 2, lvl0 + 3, 1u, base, shiftA, nbA,
+               histA);
+    LAUNCH("radix_bases", k_radix_bases, 1, (int)nbA, 0, histA, offA);
+    CK(cudaMemcpyAsync(curA, offA, nbA * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
     const u32 ntiles_cap = ntiles0 + nbA;
     const int bulk_grid = G.sms * 3;
-    if (bulk) {
-        if (sc.get(&tdesc, ntiles_cap) != 0) return -1;
-        LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles0, 256), 256, 0, lvl0, lvl0 + 2, lvl0 + 3, 1u, ntiles0, tdesc);
-        LAUNCH("msd_partition", k_msd_partition_bulk, (int)std::min<u32>(ntiles0, (u32)bulk_grid), QCE_MSDB_THREADS, QCE_MSDB_SMEM, *keys, alt,
-               tdesc, ntiles0, base, shiftA, nbA, curA);
+    if (p.bulk) {
+        if (sc.get(&m->tdesc, ntiles_cap) != 0) return -1;
+        LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles0, 256), 256, 0, lvl0, lvl0 + 2, lvl0 + 3, 1u, ntiles0, m->tdesc);
+        if (from_col)
+            LAUNCH("msd_partition", k_msd_partition_bulk<true>, (int)std::min<u32>(ntiles0, (u32)bulk_grid), QCE_MSDB_THREADS,
+                   QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0, base, shiftA, nbA, curA);
+        else
+            LAUNCH("msd_partition", k_msd_partition_bulk<false>, (int)std::min<u32>(ntiles0, (u32)bulk_grid), QCE_MSDB_THREADS,
+                   QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0, base, shiftA, nbA, curA);
     } else
     if (shape >= 1 && variant == 1)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, false>), ntiles0, 512, 0, *keys, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
+        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, false>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
                base, shiftA, nbA, curA, (const u32 *)nullptr);
     else if (shape >= 1 && variant == 2)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 3, true>), ntiles0, 512, 0, *keys, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
+        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 3, true>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
                base, shiftA, nbA, curA, (const u32 *)nullptr);
     else if (shape >= 1 && variant == 3)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, true>), ntiles0, 512, 0, *keys, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
+        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, true>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
                base, shiftA, nbA, curA, (const u32 *)nullptr);
     else if (shape >= 1)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8>), ntiles0, 512, 0, *keys, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
+        LAUNCH("msd_partition", (k_msd_partition<512, 8>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
                base, shiftA, nbA, curA, (const u32 *)nullptr);
     else
-        LAUNCH("msd_partition", (k_msd_partition<256, 16>), ntiles0, 256, 0, *keys, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
+        LAUNCH("msd_partition", (k_msd_partition<256, 16>), ntiles0, 256, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
                base, shiftA, nbA, curA, (const u32 *)nullptr);
+    return 0;
+}
+
+// Everything after level A: level B back into *keys and the finish.  *done = false means a
+// sub-bucket is too heavy for the finish kernels: the caller sorts with the LSD passes instead;
+// *keys is then left as it was, and m->alt holds level A's scatter.
+int msd_after_level_a(const MsdPlan &p, MsdLevels *m, u64 **keys, bool *done)
+{
+    *done = false;
+    const u64 base = p.base;
+    const int R = p.R, shiftB = p.shiftB, shape = p.shape, variant = p.variant, bulk = p.bulk;
+    const u32 nbA = p.nbA, nbB = p.nbB, nsub = p.nsub, ntiles0 = p.ntiles0;
+    const int bulk_grid = G.sms * 3;
+    Scratch &sc = m->sc;
+    u64 *alt = m->alt;
+    u32 *histA = m->histA, *offA = m->offA, *tstart1 = m->tstart1, *histB = m->histB, *suboff = m->suboff, *curB = m->curB;
+    MsdTileDesc *tdesc = m->tdesc;
     // level 1: the 256 buckets of level 0, each cut into tiles of its own
     const u32 ntiles1 = ntiles0 + nbA; // upper bound; surplus CTAs exit
     LAUNCH("msd_tiles", k_msd_tile_starts, 1, 256, 0, histA, nbA, tstart1);
@@ -694,7 +759,7 @@ int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 
         CK(cudaMemcpyAsync(curB, suboff, nsub * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
         if (bulk) {
             LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles1, 256), 256, 0, tstart1, offA, histA, nbA, ntiles1, tdesc);
-            LAUNCH("msd_partition", k_msd_partition_bulk, (int)std::min<u32>(ntiles1, (u32)bulk_grid), QCE_MSDB_THREADS, QCE_MSDB_SMEM, alt,
+            LAUNCH("msd_partition", k_msd_partition_bulk<false>, (int)std::min<u32>(ntiles1, (u32)bulk_grid), QCE_MSDB_THREADS, QCE_MSDB_SMEM, alt,
                    *keys, tdesc, ntiles1, base, shiftB, nbB, curB);
         } else
         if (shape >= 1 && variant == 1)
@@ -817,6 +882,30 @@ int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 
     return 0;
 }
 
+// For large packed runs.  *done = false means "not applicable or skewed": the
+// caller sorts with the LSD passes instead (the run is left untouched).
+int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 *hist_top8 = nullptr,
+             int hist_key_bits = 0)
+{
+    *done = false;
+    MsdPlan p;
+    const int applies = msd_plan(n, key_min, key_max, &p);
+    if (applies <= 0) return applies;
+    MsdLevels m;
+    const bool counted = hist_top8 && key_min == 0 && hist_key_bits == p.key_bits; // level A was counted while the run was built
+    if (msd_level_a(p, &m, *keys, false, counted ? hist_top8 : nullptr) != 0) return -1;
+    return msd_after_level_a(p, &m, keys, done);
+}
+
+// The LSD passes over a packed run's `key_bits` key bits.
+int lsd_sort_packed(u64 **a, u64 n, int key_bits)
+{
+    // k_block_sort ranks 8-bit digits: 9-bit shifts would skip every ninth key bit
+    const int db = n <= BS_TILE ? 8 : digit_bits_for(key_bits, true);
+    RadixShifts rs = shifts_for(32, key_bits, db);
+    return radix_sort(a, nullptr, n, rs, db);
+}
+
 // Sort a packed run on its `key_bits` key bits.
 int sort_packed(u64 **a, u64 n, int key_bits, u64 key_min, u64 key_max, const u32 *hist_top8 = nullptr,
                 int hist_key_bits = 0)
@@ -826,10 +915,7 @@ int sort_packed(u64 **a, u64 n, int key_bits, u64 key_min, u64 key_max, const u3
     if (key_min > key_max) key_min = 0;
     if (msd_sort(a, n, key_min, key_max, &done, hist_top8, hist_key_bits) != 0) return -1;
     if (done) return 0;
-    // k_block_sort ranks 8-bit digits: 9-bit shifts would skip every ninth key bit
-    const int db = n <= BS_TILE ? 8 : digit_bits_for(key_bits, true);
-    RadixShifts rs = shifts_for(32, key_bits, db);
-    return radix_sort(a, nullptr, n, rs, db);
+    return lsd_sort_packed(a, n, key_bits);
 }
 
 TupleView view_of(const qce_tuples *t)
@@ -1462,6 +1548,9 @@ static void release_column(Column &c)
     if (c.owned && c.alloc) cudaFree(c.alloc);
     c.alloc = nullptr;
     c.owned = false;
+    if (c.hist) cudaFree(c.hist);
+    c.hist = nullptr;
+    c.hist_bits = 0;
 }
 // the buffer of (rel, col): the previous upload's when the shape is unchanged (a refreshed
 // batch of the same relation), else a fresh cudaMalloc.  *reused tells the caller whether the
@@ -1488,14 +1577,34 @@ static int column_buffer(u32 rel, u32 col, u64 bytes, Column *c, bool *reused)
     c->owned = true;
     return 0;
 }
-static int column_max(const u64 *d, u64 n, u64 *maxv, bool *in_order = nullptr)
+// hist_of: a whole column, whose level-A histogram (Column::hist) is taken in the same pass
+static int column_max(const u64 *d, u64 n, u64 *maxv, bool *in_order = nullptr, Column *hist_of = nullptr)
 {
+    const bool hist = hist_of && n >= (1ull << 20);
+    if (hist_of) hist_of->hist_bits = 0;
+    Scratch sc;
+    u32 *lhist = nullptr;
+    if (hist) {
+        if (sc.get(&lhist, QCE_LEN_BINS) != 0) return -1;
+        CK(cudaMemsetAsync(lhist, 0, QCE_LEN_BINS * sizeof(u32), cx().stream));
+    }
     CK(cudaMemsetAsync(cx().d_scalars + 8, 0, 2 * sizeof(u64), cx().stream));
-    if (n > 0) LAUNCH("column_stats", k_column_stats, grid_for(512, n, 4), 256, 0, d, n, cx().d_scalars + 8, (u32 *)(cx().d_scalars + 9));
+    if (hist)
+        LAUNCH("column_stats", k_column_stats<true>, grid_for(512, n, 4), 256, 0, d, n, cx().d_scalars + 8,
+               (u32 *)(cx().d_scalars + 9), lhist);
+    else if (n > 0)
+        LAUNCH("column_stats", k_column_stats<false>, grid_for(512, n, 4), 256, 0, d, n, cx().d_scalars + 8,
+               (u32 *)(cx().d_scalars + 9), (u32 *)nullptr);
     CK(cudaMemcpyAsync(cx().h_scalars + 8, cx().d_scalars + 8, 2 * sizeof(u64), cudaMemcpyDeviceToHost, cx().stream));
     CK(cudaStreamSynchronize(cx().stream));
     *maxv = cx().h_scalars[8];
     if (in_order) *in_order = (cx().h_scalars[9] & 0xffffffffu) == 0;
+    const int b = bitlen(*maxv);
+    if (hist && b >= 9 && b <= 32) {
+        if (!hist_of->hist) CK(cudaMalloc(&hist_of->hist, QCE_RADIX_BINS * sizeof(u32)));
+        LAUNCH("column_stats", k_column_hist_fold, 1, 256, 0, lhist, b, hist_of->hist);
+        hist_of->hist_bits = b;
+    }
     return 0;
 }
 static void install_column(u32 rel, u32 col, const Column &c)
@@ -1658,7 +1767,8 @@ static int upload_impl(u32 rel, u32 col, const void *src, int src_kind, u64 src_
     c.windowed = !whole;
     c.win_begin = begin;
     c.win_count = count;
-    if (column_max((const u64 *)c.alloc, count, &c.maxv, &c.in_order) != 0) return -1;
+    if (column_max((const u64 *)c.alloc, count, &c.maxv, &c.in_order, whole ? &c : nullptr) != 0) return -1;
+    if (!whole) c.hist_bits = 0; // a re-upload of the same shape keeps the buffer, not its counts
     if (!whole) c.in_order = false; // a row window: the runs built from it are exchanged by key range anyway
     if (!whole && share_window(&c, per, reused) != 0) return -1;
     install_column(rel, col, c);
@@ -1773,7 +1883,7 @@ int qce_adopt_column_device(uint32_t rel, uint32_t col, const void *dev, uint64_
     (void)reused;
     c.d = (const u64 *)dev;
     c.n = n;
-    if (column_max(c.d, n, &c.maxv, &c.in_order) != 0) return -1;
+    if (column_max(c.d, n, &c.maxv, &c.in_order, &c) != 0) { release_column(c); return -1; }
     install_column(rel, col, c);
     return 0;
 }
@@ -1815,6 +1925,19 @@ int qce_column_info(uint32_t rel, uint32_t col, uint64_t *n, uint64_t *max_value
     if (get_column(rel, col, &c) != 0) return -1;
     if (n) *n = c->n;
     if (max_value) *max_value = c->maxv;
+    return 0;
+}
+int qce_column_histogram(uint32_t rel, uint32_t col, uint32_t *bins, int *key_bits)
+{
+    NEED_INIT();
+    if (!bins || !key_bits) return fail("null argument");
+    const Column *c;
+    if (get_column(rel, col, &c) != 0) return -1;
+    *key_bits = c->hist_bits;
+    if (c->hist_bits) {
+        CK(cudaMemcpyAsync(bins, c->hist, QCE_RADIX_BINS * sizeof(u32), cudaMemcpyDeviceToHost, cx().stream));
+        CK(cudaStreamSynchronize(cx().stream));
+    }
     return 0;
 }
 int qce_drop_relations(void)
@@ -1970,36 +2093,50 @@ static int build_tuples(const Column *cl, const qce_rowids *ids, qce_tuples **ou
     *out = t;
     return 0;
 }
-int qce_build_tuples_base(uint32_t rel, uint32_t col, qce_tuples **out)
+static int build_base(const Column *cl, uint32_t rel, uint32_t col, qce_tuples **out)
 {
-    NEED_INIT();
-    const Column *cl;
-    if (sharded()) return sh_build_base(rel, col, out);
-    if (get_column(rel, col, &cl) != 0) return -1;
-    if (G.cache_on) {
-        std::unique_lock<std::mutex> lk(G.mu);
-        auto it = G.run_cache.find(col_key(rel, col));
-        if (it != G.run_cache.end()) {
-            const Global::CachedRun c = it->second;
-            G.cache_hits++;
-            lk.unlock();
-            qce_tuples *t = new qce_tuples();
-            t->a = c.a; t->ids = nullptr; t->n = c.n; t->wide = false; t->key_bits = c.key_bits;
-            t->key_min = c.key_min; t->key_max = c.key_max; t->id_bound = c.id_bound;
-            t->sorted = true; t->borrowed = true; t->src_rel = rel; t->src_col = col; t->whole_base = true;
-            t->skewed = c.skewed;
-            CK(cudaStreamWaitEvent(cx().stream, c.ready, 0)); // sorted on another context's stream
-            *out = t;
-            return 0;
-        }
-        G.cache_misses++;
-    }
     if (build_tuples(cl, nullptr, out) != 0) return -1;
     (*out)->src_rel = rel;
     (*out)->src_col = col;
     (*out)->whole_base = true;
     (*out)->in_order = cl->in_order && !cl->windowed;
     return 0;
+}
+// 1: the batch's sorted-run cache holds (rel, col); *out borrows the sorted run.  0: a miss.  -1: error.
+static int cached_run(uint32_t rel, uint32_t col, qce_tuples **out)
+{
+    if (!G.cache_on) return 0;
+    std::unique_lock<std::mutex> lk(G.mu);
+    auto it = G.run_cache.find(col_key(rel, col));
+    if (it == G.run_cache.end()) {
+        G.cache_misses++;
+        return 0;
+    }
+    const Global::CachedRun c = it->second;
+    G.cache_hits++;
+    lk.unlock();
+    qce_tuples *t = new qce_tuples();
+    t->a = c.a; t->ids = nullptr; t->n = c.n; t->wide = false; t->key_bits = c.key_bits;
+    t->key_min = c.key_min; t->key_max = c.key_max; t->id_bound = c.id_bound;
+    t->sorted = true; t->borrowed = true; t->src_rel = rel; t->src_col = col; t->whole_base = true;
+    t->skewed = c.skewed;
+    if (cudaStreamWaitEvent(cx().stream, c.ready, 0) != cudaSuccess) { // sorted on another context's stream
+        (void)cudaGetLastError();
+        delete t;
+        return fail("cudaStreamWaitEvent on a cached sorted run failed");
+    }
+    *out = t;
+    return 1;
+}
+int qce_build_tuples_base(uint32_t rel, uint32_t col, qce_tuples **out)
+{
+    NEED_INIT();
+    const Column *cl;
+    if (sharded()) return sh_build_base(rel, col, out);
+    if (get_column(rel, col, &cl) != 0) return -1;
+    const int hit = cached_run(rel, col, out);
+    if (hit != 0) return hit < 0 ? -1 : 0;
+    return build_base(cl, rel, col, out);
 }
 int qce_build_tuples_base_range(uint32_t rel, uint32_t col, uint64_t row_begin, uint64_t row_count, qce_tuples **out)
 {
@@ -2089,6 +2226,26 @@ int qce_merge_join_stats(const qce_tuples *R, const qce_tuples *S, qce_rowids **
     return rc;
 }
 
+// A run that has just been sorted: its flags, and a whole base run goes to the batch's cache.
+static void sorted_run_done(qce_tuples *t)
+{
+    t->sorted = true;
+    t->skewed = tl_sort_skewed;
+    if (G.cache_on && t->whole_base && !t->wide && !t->borrowed && t->n >= 1024) {
+        // hand the run to the batch's cache; this handle (and later ones) borrow it
+        std::lock_guard<std::mutex> lk(G.mu);
+        const u64 bytes = t->n * sizeof(u64);
+        if (!G.run_cache.count(col_key(t->src_rel, t->src_col)) && G.cache_bytes + bytes <= G.cache_budget) {
+            Global::CachedRun c{t->a, t->n, t->key_bits, t->key_min, t->key_max, t->id_bound, nullptr, &cx().arena, t->skewed};
+            if (cudaEventCreateWithFlags(&c.ready, cudaEventDisableTiming) == cudaSuccess) {
+                cudaEventRecord(c.ready, cx().stream);
+                G.run_cache[col_key(t->src_rel, t->src_col)] = c;
+                G.cache_bytes += bytes;
+                t->borrowed = true;
+            } else (void)cudaGetLastError();
+        }
+    }
+}
 int qce_sort_tuples(qce_tuples *t)
 {
     NEED_INIT();
@@ -2116,22 +2273,74 @@ int qce_sort_tuples(qce_tuples *t)
         rc = sort_packed(&t->a, t->n, t->key_bits, t->key_min, t->key_max, t->hist256,
                          bitlen(t->key_max) == t->hist_key_bits ? t->hist_key_bits : -1);
     }
-    if (rc == 0) { t->sorted = true; t->skewed = tl_sort_skewed; }
-    if (rc == 0 && G.cache_on && t->whole_base && !t->wide && !t->borrowed && t->n >= 1024) {
-        // hand the run to the batch's cache; this handle (and later ones) borrow it
-        std::lock_guard<std::mutex> lk(G.mu);
-        const u64 bytes = t->n * sizeof(u64);
-        if (!G.run_cache.count(col_key(t->src_rel, t->src_col)) && G.cache_bytes + bytes <= G.cache_budget) {
-            Global::CachedRun c{t->a, t->n, t->key_bits, t->key_min, t->key_max, t->id_bound, nullptr, &cx().arena, t->skewed};
-            if (cudaEventCreateWithFlags(&c.ready, cudaEventDisableTiming) == cudaSuccess) {
-                cudaEventRecord(c.ready, cx().stream);
-                G.run_cache[col_key(t->src_rel, t->src_col)] = c;
-                G.cache_bytes += bytes;
-                t->borrowed = true;
-            } else (void)cudaGetLastError();
+    if (rc == 0) sorted_run_done(t);
+    return rc;
+}
+
+/* allocate_relation + iterative_sort of a whole base column in one: what qce_build_tuples_base followed
+ * by qce_sort_tuples returns.  A column with its level-A histogram (Column::hist) whose run takes the MSD
+ * route is never stored unsorted: MSD level A reads the column and forms the tuples in registers
+ * (k_msd_partition_bulk<true>), which saves the build's write and level A's read of the whole run.
+ * Every other run is built, then sorted.  QCE_FUSED_BUILD_SORT=0: always build, then sort. */
+int qce_build_sorted_tuples_base(uint32_t rel, uint32_t col, qce_tuples **out)
+{
+    NEED_INIT();
+    if (!out) return fail("null argument");
+    static int fused_on = -1;
+    if (fused_on < 0) { const char *e = getenv("QCE_FUSED_BUILD_SORT"); fused_on = e ? atoi(e) : 1; }
+    qce_tuples *t = nullptr;
+    if (!fused_on || sharded()) {
+        if (qce_build_tuples_base(rel, col, &t) != 0) return -1;
+        if (qce_sort_tuples(t) != 0) { qce_tuples_free(t); return -1; }
+        *out = t;
+        return 0;
+    }
+    const Column *cl;
+    if (get_column(rel, col, &cl) != 0) return -1;
+    const int hit = cached_run(rel, col, out);
+    if (hit != 0) return hit < 0 ? -1 : 0;
+    // the route is decided before any kernel runs, from the column's statistics alone
+    MsdPlan p;
+    int applies = 0;
+    tl_sort_skewed = false;
+    if (!cl->windowed && !cl->in_order && cl->hist_bits && cl->hist_bits == bitlen(cl->maxv)) {
+        applies = msd_plan(cl->n, 0, cl->maxv, &p);
+        if (applies < 0) return -1;
+    }
+    if (!applies || !p.bulk) {
+        if (build_base(cl, rel, col, &t) != 0) return -1;
+        if (qce_sort_tuples(t) != 0) { qce_tuples_free(t); return -1; }
+        *out = t;
+        return 0;
+    }
+    t = new qce_tuples();
+    t->n = cl->n;
+    t->key_bits = bitlen(cl->maxv);
+    t->key_min = 0;
+    t->key_max = cl->maxv;
+    t->wide = false;
+    t->ids = nullptr;
+    t->id_bound = (u32)cl->n;
+    t->src_rel = rel;
+    t->src_col = col;
+    t->whole_base = true;
+    if (dalloc(&t->a, t->n) != 0) { delete t; return -1; }
+    int rc;
+    {
+        MsdLevels m;
+        bool done = false;
+        rc = msd_level_a(p, &m, cl->d, true, cl->hist);
+        if (rc == 0) rc = msd_after_level_a(p, &m, &t->a, &done);
+        if (rc == 0 && !done) {
+            // a heavy key: the LSD passes sort level A's scatter, which holds every tuple of the run
+            std::swap(t->a, m.alt);
+            rc = lsd_sort_packed(&t->a, t->n, t->key_bits);
         }
     }
-    return rc;
+    if (rc != 0) { qce_tuples_free(t); return -1; }
+    sorted_run_done(t);
+    *out = t;
+    return 0;
 }
 
 /* A batch = one execute_queries call: sorted base runs are kept between its queries and

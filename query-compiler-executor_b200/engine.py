@@ -39,6 +39,7 @@ SYMBOLS = [
     "qce_set_replicate_bytes", "qce_column_would_be_whole", "qce_column_is_whole", "qce_rowids_count_local", "qce_xwin_unmap_peers", "qce_build_tuples_positions", "qce_merge_join_stats",
     "qce_elision_supported", "qce_tuples_attach", "qce_placement_cap",
     "qce_key_histogram_wide", "qce_push_tuples_wide", "qce_tuples_from_window_wide",
+    "qce_build_sorted_tuples_base", "qce_column_histogram",
 ]
 
 
@@ -67,6 +68,8 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
         "qce_filter_refine": (i32, [vp, u32, u32, C.c_char, u64, P(u64)]),
         "qce_build_tuples_base": (i32, [u32, u32, P(vp)]), "qce_build_tuples_rowids": (i32, [u32, u32, vp, P(vp)]),
         "qce_sort_tuples": (i32, [vp]), "qce_tuples_is_sorted": (i32, [vp, P(i32)]),
+        "qce_build_sorted_tuples_base": (i32, [u32, u32, P(vp)]),
+        "qce_column_histogram": (i32, [u32, u32, vp, P(i32)]),
         "qce_merge_join": (i32, [vp, vp, P(vp), P(vp), P(vp), P(vp)]),
         "qce_merge_join_walk": (i32, [vp, vp, P(vp), P(vp)]),
         "qce_distinct_pairs": (i32, [vp, vp, P(vp), P(vp)]),
@@ -207,6 +210,13 @@ class Engine:
         self._ck(self.lib.qce_column_info(rel, col, C.byref(n), C.byref(mx)))
         return n.value, mx.value
 
+    def column_histogram(self, rel: int, col: int) -> Tuple[Optional[np.ndarray], int]:
+        """(bins of key >> (key_bits - 8), key_bits) taken at upload, or (None, 0) when the column has none."""
+        bins = np.zeros(256, dtype=np.uint32)
+        kb = C.c_int()
+        self._ck(self.lib.qce_column_histogram(rel, col, bins.ctypes.data, C.byref(kb)))
+        return (bins if kb.value else None), kb.value
+
     def drop_relations(self) -> None:
         self._ck(self.lib.qce_drop_relations())
 
@@ -276,6 +286,11 @@ class Engine:
 
     def sort_tuples(self, h: int) -> None:
         self._ck(self.lib.qce_sort_tuples(h))
+
+    def build_sorted_tuples(self, rel: int, col: int) -> int:
+        h = C.c_void_p()
+        self._ck(self.lib.qce_build_sorted_tuples_base(rel, col, C.byref(h)))
+        return h.value
 
     def is_sorted(self, h: int) -> bool:
         s = C.c_int()

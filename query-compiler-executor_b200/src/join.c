@@ -180,10 +180,29 @@ static int plan_join(predicate *pred, uint32_t *relations, DArray *entities, joi
     return 0;
 }
 
-static int build_side(const join_side *s, qce_tuples **out)
+/* A base run that is sorted right after its build: built and sorted in one engine call, which can start the
+ * sort from the column.  The reference to that entry is weak because the plain-C stand-in engine of the host
+ * layer's CPU tests (tests/c/mock_engine.c) does not define it; libqce_b200 always does.  Without it the run is
+ * built, then sorted -- which is what the entry returns. */
+#pragma weak qce_build_sorted_tuples_base
+static int build_sorted_base(uint32_t rel, uint32_t col, qce_tuples **out)
 {
-    return s->source ? qce_build_tuples_rowids(s->rel, s->col, s->source->payloads, out)
-                     : qce_build_tuples_base(s->rel, s->col, out);
+    if (qce_build_sorted_tuples_base) return qce_build_sorted_tuples_base(rel, col, out);
+    if (qce_build_tuples_base(rel, col, out) != 0) return -1;
+    if (qce_sort_tuples(*out) == 0) return 0;
+    qce_tuples_free(*out);
+    *out = NULL;
+    return -1;
+}
+
+/* sorted: the side is sorted right after its build */
+static int build_side(const join_side *s, int sorted, qce_tuples **out)
+{
+    if (s->source) {
+        if (qce_build_tuples_rowids(s->rel, s->col, s->source->payloads, out) != 0) return -1;
+        return sorted ? qce_sort_tuples(*out) : 0;
+    }
+    return sorted ? build_sorted_base(s->rel, s->col, out) : qce_build_tuples_base(s->rel, s->col, out);
 }
 
 static int require_sorted(const qce_tuples *t, const char *which)
@@ -216,23 +235,21 @@ static int run_join(const join_plan *plan, join_result *res)
         return rc;
     }
 
-    check(build_side(&plan->lhs, &tl) == 0 && build_side(&plan->rhs, &tr) == 0, "Couldn't allocate relations: %s",
-          qce_last_error());
+    const int sort_lhs = plan->kind == CLASSIC_JOIN || plan->kind == JOIN_SORT_LHS;
+    const int sort_rhs = plan->kind == CLASSIC_JOIN || plan->kind == JOIN_SORT_RHS;
+    check(build_side(&plan->lhs, sort_lhs, &tl) == 0 && build_side(&plan->rhs, sort_rhs, &tr) == 0,
+          "Couldn't allocate relations: %s", qce_last_error());
     /* with an empty side the pointer walk of src/join.c:342 never starts: the
      * result is empty whatever the order of the other side */
     const int trivially_empty = qce_tuples_count(tl) == 0 || qce_tuples_count(tr) == 0;
     int outer_in_order = 1;
-    if (plan->kind == CLASSIC_JOIN || plan->kind == JOIN_SORT_LHS) {
-        check(qce_sort_tuples(tl) == 0, "sort failed: %s", qce_last_error());
-    } else if (!trivially_empty) {
+    if (!sort_lhs && !trivially_empty) {
         /* JOIN_SORT_RHS trusts the lhs to be in key order.  When it is not (the
          * asymmetric tests of src/join.c:253-267), the reference's walk is still a
          * function of the data -- qce_merge_join_walk computes it. */
         check(qce_tuples_is_sorted(tl, &outer_in_order) == 0, "%s", qce_last_error());
     }
-    if (plan->kind == CLASSIC_JOIN || plan->kind == JOIN_SORT_RHS) {
-        check(qce_sort_tuples(tr) == 0, "sort failed: %s", qce_last_error());
-    } else if (!trivially_empty) {
+    if (!sort_rhs && !trivially_empty) {
         check(require_sorted(tr, "right") == 0, "Join failed!");
     }
     if (outer_in_order) {
@@ -427,12 +444,13 @@ static int elided_join(const join_plan *plan, DArray *entities)
         }
         if (qce_tuples_attach(t[s], nc, cols) != 0) { rc = QCE_JOIN_UNSAFE; goto done; }
     }
-    if (qce_build_tuples_base(sides[o]->rel, sides[o]->col, &t[o]) != 0) {
-        log_err("Couldn't allocate relations: %s", qce_last_error());
+    /* the base side is always sorted */
+    if (build_sorted_base(sides[o]->rel, sides[o]->col, &t[o]) != 0) {
+        log_err("Couldn't build and sort a relation: %s", qce_last_error());
         goto done;
     }
     if (plan->kind == CLASSIC_JOIN) {
-        if (qce_sort_tuples(t[0]) != 0 || qce_sort_tuples(t[1]) != 0) { log_err("sort failed: %s", qce_last_error()); goto done; }
+        if (qce_sort_tuples(t[s]) != 0) { log_err("sort failed: %s", qce_last_error()); goto done; }
     } else {
         /* the entity side is trusted to be in key order (src/join.c:197-204): only vouched for when it is */
         int sorted = 0;
@@ -440,7 +458,6 @@ static int elided_join(const join_plan *plan, DArray *entities)
             if (qce_tuples_is_sorted(t[s], &sorted) != 0) { log_err("%s", qce_last_error()); goto done; }
             if (!sorted) { rc = QCE_JOIN_UNSAFE; goto done; }
         }
-        if (qce_sort_tuples(t[o]) != 0) { log_err("sort failed: %s", qce_last_error()); goto done; }
     }
     uint32_t lo = 0, hi = 0;
     if (qce_merge_join_stats(t[0], t[1], &out[0], &out[1], &lo, &hi) != 0) { log_err("merge join failed: %s", qce_last_error()); goto done; }

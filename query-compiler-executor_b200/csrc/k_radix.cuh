@@ -28,8 +28,7 @@
 #include "qce_common.cuh"
 
 #define QCE_RADIX_BITS 8
-#define QCE_RADIX_BINS 256  // 8-bit digits: the default
-#define QCE_MAX_BINS 512    // 9-bit digits, when they save a pass
+#define QCE_RADIX_BINS 256
 #define QCE_MAX_PASSES 8
 
 template <typename KeyT> __device__ __forceinline__ KeyT ld_stream_key(const KeyT *p);
@@ -135,11 +134,11 @@ k_unpack_lo(const u64 *__restrict__ in, u64 n, u32 *__restrict__ out)
 
 // ---- digit histograms of every pass in one read (build_histogram,
 // src/utilities.c:20-31, hoisted out of the per-bucket loop) ------------------------
-// `bins` = 256 or 512 (8- or 9-bit digits), the same for every pass of a sort.
+// `bins` = QCE_RADIX_BINS, the same for every pass of a sort.
 __global__ void __launch_bounds__(512)
 k_radix_hist(const u64 *__restrict__ keys, u64 n, RadixShifts rs, u32 bins, u32 *__restrict__ ghist)
 {
-    __shared__ u32 sh[QCE_MAX_PASSES * QCE_MAX_BINS];
+    __shared__ u32 sh[QCE_MAX_PASSES * QCE_RADIX_BINS];
     const u32 mask = bins - 1;
     for (u32 i = threadIdx.x; i < rs.npass * bins; i += 512) sh[i] = 0;
     __syncthreads();
@@ -184,13 +183,13 @@ k_hist_u32(const u32 *__restrict__ keys, u64 n, u32 base, int shift, u32 *__rest
 }
 
 // build_psum (src/utilities.c:34-48): exclusive prefix over the bins of each
-// pass.  One CTA of `bins` (256 or 512) threads per pass.
+// pass.  One CTA of `bins` (256) threads per pass.
 __global__ void __launch_bounds__(512) k_radix_bases(const u32 *__restrict__ ghist, u32 *__restrict__ gbase)
 {
     __shared__ u32 scratch[33];
     const u32 bins = blockDim.x;
     u32 v = ghist[blockIdx.x * bins + threadIdx.x];
-    // block_scan_excl is written for a compile-time thread count; 16 warps cover both sizes
+    // block_scan_excl is written for a compile-time thread count; this scan takes `bins` threads
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     u32 incl = warp_scan_incl<u32>(v);
     if (lane == 31) scratch[warp] = incl;
@@ -209,7 +208,6 @@ __global__ void __launch_bounds__(512) k_radix_bases(const u32 *__restrict__ ghi
 struct DigitShift {
     int shift;
     __device__ __forceinline__ u32 operator()(u64 k, u32 mask) const { return (u32)(k >> shift) & mask; }
-    __device__ __forceinline__ u32 operator()(u32 k, u32 mask) const { return (k >> shift) & mask; }
 };
 // Packed words always sort key bits, i.e. word bits >= 32: the digit only needs
 // the high register (no 64-bit funnel shifts).  hi_shift = shift - 32.
@@ -266,28 +264,31 @@ template <int BITS> __device__ __forceinline__ u32 warp_peers(u32 d)
 #define QCE_ST_INCL 0x80000000u
 #define QCE_ST_MASK 0x3fffffffu
 
-template <int THREADS, int ITEMS, int BITS, typename KeyT = u64> struct OnesweepSmem {
-    static constexpr int BINS = 1 << BITS;
-    u32 warp_hist[(THREADS / 32) * BINS]; // per-warp digit counts -> bases
-    u32 tile_excl[BINS];                  // digit start inside the sorted tile
-    u32 goff[BINS];                       // global start of digit minus tile_excl
+// Tile shape: 256 threads x 16 tuples, 4 CTAs per SM (other shapes were swept on B200,
+// DESIGN.md §4.2).
+constexpr int QCE_OS_THREADS = 256, QCE_OS_ITEMS = 16, QCE_OS_TILE = QCE_OS_THREADS * QCE_OS_ITEMS;
+constexpr int QCE_OS_MIN_CTAS = 4;
+
+struct OnesweepSmem {
+    u32 warp_hist[(QCE_OS_THREADS / 32) * QCE_RADIX_BINS]; // per-warp digit counts -> bases
+    u32 tile_excl[QCE_RADIX_BINS];                         // digit start inside the sorted tile
+    u32 goff[QCE_RADIX_BINS];                              // global start of digit minus tile_excl
     u32 scratch[33];
     u32 tile_id;
-    KeyT keys[THREADS * ITEMS];
+    u64 keys[QCE_OS_TILE];
 };
 
 // One tile of the pass.  FULL = every slot of the tile holds a real tuple (no
 // bounds checks, no padding logic): all tiles but the last.
-template <int THREADS, int ITEMS, int BITS, bool HAS_VALS, bool FULL, int MATCH_EVERY, typename KeyT,
-          typename DigitOp>
+template <bool HAS_VALS, bool FULL, typename DigitOp>
 __device__ __forceinline__ void
-onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const KeyT *__restrict__ keys_in,
-              KeyT *__restrict__ keys_out, const u32 *__restrict__ vals_in, u32 *__restrict__ vals_out, u32 n,
-              const DigitOp &digit, const u32 *__restrict__ gbase, u32 *__restrict__ status, u32 tile)
+onesweep_tile(OnesweepSmem &sm, u32 *svals, const u64 *__restrict__ keys_in, u64 *__restrict__ keys_out,
+              const u32 *__restrict__ vals_in, u32 *__restrict__ vals_out, u32 n, const DigitOp &digit,
+              const u32 *__restrict__ gbase, u32 *__restrict__ status, u32 tile)
 {
-    constexpr int TILE = THREADS * ITEMS;
+    constexpr int THREADS = QCE_OS_THREADS, ITEMS = QCE_OS_ITEMS, TILE = QCE_OS_TILE;
     constexpr int WARPS = THREADS / 32;
-    constexpr int BINS = 1 << BITS;
+    constexpr int BINS = QCE_RADIX_BINS;
     constexpr u32 DMASK = BINS - 1;
     constexpr int BPT = (BINS + THREADS - 1) / THREADS; // bins per thread, consecutive
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -296,17 +297,17 @@ onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const Ke
     const u32 npad = TILE - nvalid; // padding slots of the last tile (digit BINS-1)
 
     // ---- load: warp-striped so that (warp, item, lane) order == input order
-    KeyT key[ITEMS];
+    u64 key[ITEMS];
     u32 val[HAS_VALS ? ITEMS : 1];
     const u32 wbase = tbase + warp * (32 * ITEMS) + lane;
 #pragma unroll
     for (int j = 0; j < ITEMS; j++) {
         const u32 idx = wbase + j * 32;
         if (FULL || idx < n) {
-            key[j] = ld_stream_key<KeyT>(keys_in + idx);
+            key[j] = ld_stream_u64(keys_in + idx);
             if (HAS_VALS) val[j] = ld_stream_u32(vals_in + idx);
         } else {
-            key[j] = (KeyT)~(KeyT)0;
+            key[j] = ~0ull;
             if (HAS_VALS) val[j] = 0u;
         }
     }
@@ -320,7 +321,8 @@ onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const Ke
     u32 rd[ITEMS]; // digit << 16 | rank inside (warp, digit)
     u32 *wh = sm.warp_hist + warp * BINS;
     const u32 lt = lanemask_lt();
-    constexpr int CH = (ITEMS % 4 == 0) ? 4 : ((ITEMS % 3 == 0) ? 3 : 1);
+    constexpr int CH = 4;
+    static_assert(ITEMS % CH == 0, "items come in chunks of CH");
 #pragma unroll
     for (int j0 = 0; j0 < ITEMS; j0 += CH) {
         u32 d[CH], peers[CH], old[CH];
@@ -328,11 +330,10 @@ onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const Ke
         for (int c = 0; c < CH; c++) {
             // padding of the last tile must sort behind every real tuple of the tile
             d[c] = (!FULL && (wbase + (j0 + c) * 32) >= n) ? DMASK : digit(key[j0 + c], DMASK);
-            // every MATCH_EVERY-th item goes to match.any: the ADU pipe is idle
-            // otherwise, so it takes a share of the ranking off the ALU ballots
-            peers[c] = (MATCH_EVERY > 0 && ((j0 + c) % (MATCH_EVERY > 0 ? MATCH_EVERY : 1)) == MATCH_EVERY - 1)
-                           ? __match_any_sync(QCE_FULL_MASK, d[c])
-                           : warp_peers<BITS>(d[c]);
+            // every 4th item goes to match.any: the ADU pipe is idle otherwise,
+            // so it takes a share of the ranking off the ALU ballots
+            peers[c] = ((j0 + c) % 4 == 3) ? __match_any_sync(QCE_FULL_MASK, d[c])
+                                           : warp_peers<QCE_RADIX_BITS>(d[c]);
         }
 #pragma unroll
         for (int c = 0; c < CH; c++) {
@@ -433,7 +434,7 @@ onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const Ke
     for (int j = 0; j < ITEMS; j++) {
         const u32 p = tid + j * THREADS;
         if (FULL || p < nvalid) {
-            const KeyT k = sm.keys[p];
+            const u64 k = sm.keys[p];
             const u32 g = sm.goff[digit(k, DMASK)] + p;
             keys_out[g] = k;
             if (HAS_VALS) vals_out[g] = svals[p];
@@ -441,21 +442,19 @@ onesweep_tile(OnesweepSmem<THREADS, ITEMS, BITS, KeyT> &sm, u32 *svals, const Ke
     }
 }
 
-template <int THREADS, int ITEMS, int MIN_CTAS, int BITS, int MATCH_EVERY, bool HAS_VALS, typename KeyT,
-          typename DigitOp>
-__global__ void __launch_bounds__(THREADS, MIN_CTAS)
-k_onesweep(const KeyT *__restrict__ keys_in, KeyT *__restrict__ keys_out,
+template <bool HAS_VALS, typename DigitOp>
+__global__ void __launch_bounds__(QCE_OS_THREADS, QCE_OS_MIN_CTAS)
+k_onesweep(const u64 *__restrict__ keys_in, u64 *__restrict__ keys_out,
            const u32 *__restrict__ vals_in, u32 *__restrict__ vals_out, u32 n, DigitOp digit,
            const u32 *__restrict__ gbase, u32 *__restrict__ status, u32 *__restrict__ tile_counter)
 {
-    static_assert(THREADS * ITEMS <= 65536 && ITEMS * 32 < 65536, "tile shape");
-    constexpr int TILE = THREADS * ITEMS;
+    constexpr int THREADS = QCE_OS_THREADS, TILE = QCE_OS_TILE;
+    static_assert(TILE <= 65536 && QCE_OS_ITEMS * 32 < 65536, "tile shape");
     constexpr int WARPS = THREADS / 32;
-    constexpr int BINS = 1 << BITS;
+    constexpr int BINS = QCE_RADIX_BINS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef OnesweepSmem<THREADS, ITEMS, BITS, KeyT> Smem;
-    Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
-    u32 *svals = reinterpret_cast<u32 *>(smem_raw + sizeof(Smem));
+    OnesweepSmem &sm = *reinterpret_cast<OnesweepSmem *>(smem_raw);
+    u32 *svals = reinterpret_cast<u32 *>(smem_raw + sizeof(OnesweepSmem));
 
     // Tiles are claimed in launch order so that every tile a CTA may wait on in
     // the look-back is owned by a CTA that is already resident.
@@ -464,11 +463,9 @@ k_onesweep(const KeyT *__restrict__ keys_in, KeyT *__restrict__ keys_out,
     __syncthreads();
     const u32 tile = sm.tile_id;
     if ((tile + 1) * (u32)TILE <= n)
-        onesweep_tile<THREADS, ITEMS, BITS, HAS_VALS, true, MATCH_EVERY, KeyT>(sm, svals, keys_in, keys_out, vals_in,
-                                                                              vals_out, n, digit, gbase, status, tile);
+        onesweep_tile<HAS_VALS, true>(sm, svals, keys_in, keys_out, vals_in, vals_out, n, digit, gbase, status, tile);
     else
-        onesweep_tile<THREADS, ITEMS, BITS, HAS_VALS, false, MATCH_EVERY, KeyT>(sm, svals, keys_in, keys_out, vals_in,
-                                                                               vals_out, n, digit, gbase, status, tile);
+        onesweep_tile<HAS_VALS, false>(sm, svals, keys_in, keys_out, vals_in, vals_out, n, digit, gbase, status, tile);
 }
 
 // ---- small runs: whole sort in one CTA's shared memory --------------------------
@@ -563,8 +560,8 @@ k_block_sort(u64 *__restrict__ keys, u32 *__restrict__ vals, u32 n, RadixShifts 
 // buckets below 4096 tuples to a small sort (iterative_sort, src/join.c:5-94).
 // The same shape is the cheapest one here, because an MSD partition does not
 // have to be stable: no per-bit ballots, no look-back chain.
-//   pass A   scatter by the top P1 key bits          (k_msd_partition, level 0)
-//   pass B   per bucket, scatter by the next P2 bits (k_msd_partition, level 1)
+//   pass A   scatter by the top P1 key bits          (k_msd_partition_bulk, level 0)
+//   pass B   per bucket, scatter by the next P2 bits (k_msd_partition_bulk, level 1)
 //   finish   every sub-bucket (<= 4096 tuples) is sorted on the remaining key
 //            bits inside one CTA's shared memory     (k_msd_local_sort)
 // Inside a tile a key's slot among equal digits comes from a shared-memory
@@ -658,10 +655,9 @@ __device__ __forceinline__ bool msd_warp_skewed(u32 dg, bool live)
 
 // One unstable partition pass.  cursor[bucket * bins + digit] starts at the
 // global output offset of that (bucket, digit) range and is advanced by the tiles.
-// MIN_CTAS = 4 caps the kernel at 32 registers (100 % occupancy with 512 threads); VEC loads
-// two adjacent tuples with one 128-bit load where the tile starts on a 16-byte boundary.
-template <int THREADS, int ITEMS, typename KeyT = u64, int MIN_CTAS = (THREADS == 512 ? 3 : 1), bool VEC = false>
-__global__ void __launch_bounds__(THREADS, MIN_CTAS)
+// Used by the exchange partition (u64 tuples) and the checksum's row-id partition (u32).
+template <int THREADS, int ITEMS, typename KeyT = u64>
+__global__ void __launch_bounds__(THREADS, 3)
 k_msd_partition(const KeyT *__restrict__ in, KeyT *__restrict__ out, const u32 *__restrict__ tile_start,
                 const u32 *__restrict__ bucket_off, const u32 *__restrict__ bucket_size, u32 nbuckets, KeyT base,
                 int shift, u32 bins, u32 *__restrict__ cursor, const u32 *__restrict__ lut)
@@ -685,33 +681,15 @@ k_msd_partition(const KeyT *__restrict__ in, KeyT *__restrict__ out, const u32 *
 
     KeyT key[ITEMS];
     u32 slot[ITEMS]; // digit << 16 | slot among the tile's keys with that digit
-    // element index of item j: strided by THREADS, or (VEC) adjacent pairs strided by 2 * THREADS
-    const bool vec = VEC && sizeof(KeyT) == 8 && ((begin & 1u) == 0);
-#define MSD_ITEM_INDEX(j) (vec ? (u32)(2 * tid + ((j) & 1) + ((j) >> 1) * 2 * THREADS) : (u32)(tid + (j) * THREADS))
-    if (vec) {
 #pragma unroll
-        for (int j = 0; j < ITEMS; j += 2) {
-            const u32 i = MSD_ITEM_INDEX(j);
-            if (i + 1 < count) {
-                u64 a, b;
-                ld_stream_u64x2(reinterpret_cast<const u64 *>(in) + begin + i, a, b);
-                key[j] = (KeyT)a;
-                key[j + 1] = (KeyT)b;
-            } else if (i < count) {
-                key[j] = ld_stream_key<KeyT>(in + begin + i);
-            }
-        }
-    } else {
-#pragma unroll
-        for (int j = 0; j < ITEMS; j++) {
-            const u32 i = tid + j * THREADS;
-            if (i < count) key[j] = ld_stream_key<KeyT>(in + begin + i);
-        }
+    for (int j = 0; j < ITEMS; j++) {
+        const u32 i = tid + j * THREADS;
+        if (i < count) key[j] = ld_stream_key<KeyT>(in + begin + i);
     }
     bool agg = false;
 #pragma unroll
     for (int j = 0; j < ITEMS; j++) {
-        const u32 i = MSD_ITEM_INDEX(j);
+        const u32 i = tid + j * THREADS;
         const bool live = i < count;
         u32 d = 0;
         if (live) {
@@ -737,10 +715,9 @@ k_msd_partition(const KeyT *__restrict__ in, KeyT *__restrict__ out, const u32 *
     __syncthreads();
 #pragma unroll
     for (int j = 0; j < ITEMS; j++) {
-        const u32 i = MSD_ITEM_INDEX(j);
+        const u32 i = tid + j * THREADS;
         if (i < count) skeys[excl[slot[j] >> 16] + (slot[j] & 0xffffu)] = key[j];
     }
-#undef MSD_ITEM_INDEX
     __syncthreads();
 #pragma unroll
     for (int j = 0; j < ITEMS; j++) {
@@ -1064,14 +1041,15 @@ k_msd_local_sort(u64 *__restrict__ keys, const u32 *__restrict__ seg_off, const 
 // remaining key bits (2^R shared-memory counters).  Equal digits are now equal
 // keys, so no stability is needed: a key's slot inside its digit comes from
 // atomicAdd-with-return on the digit's counter -- no ballots, one pass.
-// MAXB = counters cleared and scanned per sub-bucket (>= 2^rbits): with 11 remaining bits half of the
-// 4096 is dead work that costs as much as ranking the ~2300 tuples themselves.
-template <int THREADS, int ITEMS, int MIN_CTAS, int MAXB = 4096>
+// Launched when the largest sub-bucket holds 3073-4096 tuples; the bulk-copy kernel below
+// takes runs whose sub-buckets all fit its 3072-tuple tile.
+template <int THREADS, int ITEMS, int MIN_CTAS>
 __global__ void __launch_bounds__(THREADS, MIN_CTAS)
 k_msd_count_sort(u64 *__restrict__ keys, const u32 *__restrict__ seg_off, const u32 *__restrict__ seg_size,
                  u64 key_base, int rbits)
 {
     constexpr int TILE = THREADS * ITEMS;
+    constexpr int MAXB = 4096;          // counters cleared and scanned per sub-bucket (>= 2^rbits)
     constexpr int BPT = MAXB / THREADS; // counters per thread in the scan (consecutive)
     static_assert(BPT % 4 == 0, "the counter scan works on uint4 groups");
     extern __shared__ __align__(16) unsigned char smem_raw[]; // TILE*8 + MAXB*4 + 33*4 bytes
@@ -1146,6 +1124,8 @@ k_msd_count_sort(u64 *__restrict__ keys, const u32 *__restrict__ seg_off, const 
 // bulk-copy engine (cp.async.bulk + mbarrier, as in k_msd_partition_bulk) while sub-bucket k is counted,
 // scanned and scattered -- the plain kernel above spends a third of every sub-bucket waiting for its own
 // loads (ncu: long + short scoreboard, issue 27 %).  The landing buffer is the staging buffer.
+// MAXB = counters cleared and scanned per sub-bucket (>= 2^rbits): with 11 remaining bits half of
+// 4096 would be dead work that costs as much as ranking the ~2300 tuples themselves.
 template <int THREADS, int ITEMS, int MAXB>
 __global__ void __launch_bounds__(THREADS, 3)
 k_msd_count_sort_bulk(u64 *__restrict__ keys, const u32 *__restrict__ seg_off, const u32 *__restrict__ seg_size, u32 nsub,

@@ -418,73 +418,34 @@ int compact_from_mask(int layout, int mode, const u32 *mask, const u32 *tile_cou
 }
 
 // ---- radix sort driver -------------------------------------------------------
-// Tile shapes of the one-sweep pass.  The default was picked by sweeping them on
-// B200 (tools/sort_bench.py, profiles/); QCE_ONESWEEP_CFG=<index> overrides it.
-struct OnesweepCfg { int threads, items, min_ctas, match_every; };
-static const OnesweepCfg kOnesweepCfgs[] = {{256, 16, 4, 4}, {256, 16, 3, 4}, {256, 24, 2, 4}, {384, 12, 3, 4},
-                                            {512, 8, 3, 4},  {256, 16, 4, 0}};
-constexpr int kNumOnesweepCfgs = (int)(sizeof(kOnesweepCfgs) / sizeof(kOnesweepCfgs[0]));
-static int g_onesweep_cfg = -1;
-static int onesweep_cfg()
+// One digit pass of the LSD sort (k_onesweep).
+template <bool HAS_VALS, typename DigitOp>
+int launch_onesweep(const u64 *kin, u64 *kout, const u32 *vin, u32 *vout, u32 n, DigitOp dop, const u32 *gbase,
+                    u32 *status, u32 *counter)
 {
-    if (g_onesweep_cfg < 0) {
-        const char *e = getenv("QCE_ONESWEEP_CFG");
-        int c = e ? atoi(e) : 0;
-        g_onesweep_cfg = (c >= 0 && c < kNumOnesweepCfgs) ? c : 0;
-    }
-    return g_onesweep_cfg;
-}
-static int onesweep_tile_size() { const OnesweepCfg &c = kOnesweepCfgs[onesweep_cfg()]; return c.threads * c.items; }
-
-template <int THREADS, int ITEMS, int MIN_CTAS, int BITS, int MATCH_EVERY, bool HAS_VALS, typename KeyT,
-          typename DigitOp>
-int launch_onesweep_cfg(const KeyT *kin, KeyT *kout, const u32 *vin, u32 *vout, u32 n, DigitOp dop,
-                        const u32 *gbase, u32 *status, u32 *counter)
-{
-    auto kern = k_onesweep<THREADS, ITEMS, MIN_CTAS, BITS, MATCH_EVERY, HAS_VALS, KeyT, DigitOp>;
-    constexpr int TILE = THREADS * ITEMS;
-    const size_t smem = sizeof(OnesweepSmem<THREADS, ITEMS, BITS, KeyT>) + (HAS_VALS ? TILE * sizeof(u32) : 0);
+    auto kern = k_onesweep<HAS_VALS, DigitOp>;
+    const size_t smem = sizeof(OnesweepSmem) + (HAS_VALS ? QCE_OS_TILE * sizeof(u32) : 0);
     static bool attr_set = false; // per instantiation
     if (!attr_set) {
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_set = true;
     }
-    const u32 ntiles = (u32)ceil_div(n, TILE);
-    LAUNCH(sizeof(KeyT) == 4 ? "onesweep_u32" : (HAS_VALS ? "onesweep_kv" : "onesweep_k"), kern, ntiles, THREADS, smem,
-           kin, kout, vin, vout, n, dop, gbase, status, counter);
+    const u32 ntiles = (u32)ceil_div(n, QCE_OS_TILE);
+    LAUNCH(HAS_VALS ? "onesweep_kv" : "onesweep_k", kern, ntiles, QCE_OS_THREADS, smem, kin, kout, vin, vout, n, dop, gbase,
+           status, counter);
     return 0;
-}
-
-// BITS = 8 (256 bins) or 9 (512 bins, when it saves a pass)
-template <bool HAS_VALS, int BITS, typename KeyT, typename DigitOp>
-int launch_onesweep(const KeyT *kin, KeyT *kout, const u32 *vin, u32 *vout, u32 n, DigitOp dop,
-                    const u32 *gbase, u32 *status, u32 *counter)
-{
-#define QCE_OS_CASE(I, T, IT, MC, ME) \
-    case I: return launch_onesweep_cfg<T, IT, MC, BITS, ME, HAS_VALS, KeyT>(kin, kout, vin, vout, n, dop, gbase, status, counter);
-    switch (onesweep_cfg()) {
-        QCE_OS_CASE(0, 256, 16, 4, 4)
-        QCE_OS_CASE(1, 256, 16, 3, 4)
-        QCE_OS_CASE(2, 256, 24, 2, 4)
-        QCE_OS_CASE(3, 384, 12, 3, 4)
-        QCE_OS_CASE(4, 512, 8, 3, 4)
-        QCE_OS_CASE(5, 256, 16, 4, 0)
-    }
-#undef QCE_OS_CASE
-    return fail("bad one-sweep configuration");
 }
 
 constexpr int BS_THREADS = 512, BS_ITEMS = 8, BS_TILE = BS_THREADS * BS_ITEMS; // block sort: runs <= 4096 tuples
 
 // Sort words (and optional 32-bit values) by the digits listed in rs, least
 // significant first.  *keys / *vals are replaced by the sorted buffers.
-int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs, int digit_bits = QCE_RADIX_BITS)
+int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs)
 {
     if (n <= 1 || rs.npass == 0) return 0;
     if (n >= (1ull << 30)) return fail("sort of %llu tuples exceeds the 2^30 per-run limit", (unsigned long long)n);
     if (n <= BS_TILE) {
         // small run: the whole sort in one CTA (k_block_sort), in place
-        if (digit_bits != 8) return fail("internal: the block sort ranks 8-bit digits, not %d-bit ones", digit_bits);
         const size_t smem = BS_TILE * sizeof(u64) + (vals ? BS_TILE * sizeof(u32) : 0) +
                             ((BS_THREADS / 32) * 256 + 256 + 33) * sizeof(u32);
         static bool attr_k = false, attr_kv = false;
@@ -503,8 +464,8 @@ int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs, int digit_b
         }
         return 0;
     }
-    const u32 bins = 1u << digit_bits;
-    const u32 ntiles = (u32)ceil_div(n, onesweep_tile_size());
+    const u32 bins = QCE_RADIX_BINS;
+    const u32 ntiles = (u32)ceil_div(n, QCE_OS_TILE);
     u64 *alt_k = nullptr;
     u32 *alt_v = nullptr, *ghist = nullptr, *gbase = nullptr, *status = nullptr, *counters = nullptr;
     Scratch sc; // the ping-pong buffers change hands with *keys / *vals and are released by hand
@@ -528,13 +489,10 @@ int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs, int digit_b
         const u32 m = (u32)n;
         int rc;
         if (vals)
-            rc = launch_onesweep<true, 8, u64>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
-        else if (digit_bits == 9)
-            rc = rs.shift[p] >= 32 ? launch_onesweep<false, 9, u64>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
-                                   : launch_onesweep<false, 9, u64>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+            rc = launch_onesweep<true>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
         else
-            rc = rs.shift[p] >= 32 ? launch_onesweep<false, 8, u64>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
-                                   : launch_onesweep<false, 8, u64>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+            rc = rs.shift[p] >= 32 ? launch_onesweep<false>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
+                                   : launch_onesweep<false>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
         if (rc != 0) return -1;
         std::swap(kin, kout);
         std::swap(vin, vout);
@@ -547,28 +505,13 @@ int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs, int digit_b
     return 0;
 }
 
-// Digit plan for `bits` significant key bits starting at word bit `base_shift`:
-// 9-bit digits when that saves a whole pass over 8-bit digits (9, 17-18, 25-27,
-// 33-36 ... bits; keys-only runs), otherwise 8-bit.  The digit width is the same
-// for every pass of one sort; the last digit may cover bits above the key, which
-// are zero.
-int digit_bits_for(int bits, bool keys_only)
-{
-    static int force = -1; // QCE_DIGIT_BITS=8|9 overrides
-    if (force < 0) {
-        const char *e = getenv("QCE_DIGIT_BITS");
-        force = e ? atoi(e) : 0;
-    }
-    if (!keys_only) return 8;
-    if (force == 8 || force == 9) return force;
-    (void)bits;
-    return 8; // 9-bit digits measured slower on B200: +35 % per pass outweighs the saved pass (profiles/)
-}
-RadixShifts shifts_for(int base_shift, int bits, int digit_bits = QCE_RADIX_BITS)
+// Digit plan for `bits` significant key bits starting at word bit `base_shift`: 8-bit
+// digits; the last digit may cover bits above the key, which are zero.
+RadixShifts shifts_for(int base_shift, int bits)
 {
     RadixShifts rs;
     rs.npass = 0;
-    for (int b = 0; b < bits && rs.npass < QCE_MAX_PASSES; b += digit_bits) rs.shift[rs.npass++] = base_shift + b;
+    for (int b = 0; b < bits && rs.npass < QCE_MAX_PASSES; b += QCE_RADIX_BITS) rs.shift[rs.npass++] = base_shift + b;
     for (int i = rs.npass; i < QCE_MAX_PASSES; i++) rs.shift[i] = 0;
     return rs;
 }
@@ -583,8 +526,28 @@ struct MsdPlan {
     u64 n, base;       // the kernels work on key - key_min: base = key_min << 32
     int key_bits, P, R, shiftA, shiftB;
     u32 nbA, nbB, nsub, ntiles0;
-    int shape, variant, bulk; // QCE_MSD_SHAPE / QCE_MSD_VARIANT / QCE_MSD_BULK
 };
+
+// Dynamic shared memory of the MSD kernels that need more than the default 48 KB.
+constexpr size_t CS_SMEM = 512 * 8 * sizeof(u64) + 4096 * sizeof(u32) + 33 * sizeof(u32); // k_msd_count_sort<512, 8, 3>
+constexpr size_t CSB_TILE = (256 * 12 + 2) * sizeof(u64) * 2; // k_msd_count_sort_bulk<256, 12, MAXB>: + MAXB counters
+constexpr size_t BIG_SMEM = QCE_MSD_TILE * sizeof(u64) + 3 * 4096 * sizeof(u32); // k_big_partition<4096>
+int msd_set_smem_attrs()
+{
+    static bool set = false;
+    if (set) return 0;
+    const cudaFuncAttribute a = cudaFuncAttributeMaxDynamicSharedMemorySize;
+    CK(cudaFuncSetAttribute(k_msd_partition_bulk<false>, a, (int)QCE_MSDB_SMEM));
+    CK(cudaFuncSetAttribute(k_msd_partition_bulk<true>, a, (int)QCE_MSDB_SMEM));
+    CK(cudaFuncSetAttribute(k_msd_count_sort<512, 8, 3>, a, (int)CS_SMEM));
+    CK(cudaFuncSetAttribute(k_msd_count_sort_bulk<256, 12, 1024>, a, (int)(CSB_TILE + 1024 * sizeof(u32))));
+    CK(cudaFuncSetAttribute(k_msd_count_sort_bulk<256, 12, 2048>, a, (int)(CSB_TILE + 2048 * sizeof(u32))));
+    CK(cudaFuncSetAttribute(k_msd_count_sort_bulk<256, 12, 4096>, a, (int)(CSB_TILE + 4096 * sizeof(u32))));
+    CK(cudaFuncSetAttribute(k_big_partition<4096>, a, (int)BIG_SMEM));
+    set = true;
+    return 0;
+}
+
 // 1: the MSD route applies; 0: the LSD passes sort the run; -1: error.  Flags a run of few
 // distinct keys in tl_sort_skewed on the way.
 int msd_plan(u64 n, u64 key_min, u64 key_max, MsdPlan *p)
@@ -619,28 +582,7 @@ int msd_plan(u64 n, u64 key_min, u64 key_max, MsdPlan *p)
     p->nbB = 1u << (P - 8);
     p->nsub = p->nbA * p->nbB;
     p->ntiles0 = (u32)ceil_div(n, QCE_MSD_TILE);
-    static int shape = -1; // QCE_MSD_SHAPE: 0 = 256 threads x 16 tuples, 1 = 512 x 8
-    if (shape < 0) {
-        const char *e = getenv("QCE_MSD_SHAPE");
-        shape = e ? atoi(e) : 2;
-    }
-    static int variant = -1; // QCE_MSD_VARIANT: 0 = 40 regs, 1 = 32 regs (4 CTAs/SM), 2 = 40 regs + 128-bit loads, 3 = both
-    if (variant < 0) {
-        const char *e = getenv("QCE_MSD_VARIANT");
-        variant = e ? atoi(e) : 0;
-    }
-    static int bulk = -1; // QCE_MSD_BULK=0: the plain-load partition kernel (for comparison)
-    if (bulk < 0) {
-        const char *e = getenv("QCE_MSD_BULK");
-        bulk = e ? atoi(e) : 1;
-        if (bulk) {
-            CK(cudaFuncSetAttribute(k_msd_partition_bulk<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QCE_MSDB_SMEM));
-            CK(cudaFuncSetAttribute(k_msd_partition_bulk<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QCE_MSDB_SMEM));
-        }
-    }
-    p->shape = shape;
-    p->variant = variant;
-    p->bulk = bulk;
+    if (msd_set_smem_attrs() != 0) return -1;
     return 1;
 }
 
@@ -655,14 +597,13 @@ struct MsdLevels {
 };
 
 // Level A: scatter the run by its top 8 key bits into m->alt.  `in` is the packed run, or with
-// from_col the base column itself (the bulk partition kernel only).  hist_top8: the level-A
+// from_col the base column itself (k_msd_partition_bulk<true>).  hist_top8: the level-A
 // histogram when it is already known (taken while the run was built, or with the column statistics).
 int msd_level_a(const MsdPlan &p, MsdLevels *m, const u64 *in, bool from_col, const u32 *hist_top8)
 {
     const u64 n = p.n, base = p.base;
-    const int shiftA = p.shiftA, shape = p.shape, variant = p.variant;
+    const int shiftA = p.shiftA;
     const u32 nbA = p.nbA, nsub = p.nsub, ntiles0 = p.ntiles0;
-    if (from_col && !p.bulk) return fail("internal: level A from a column needs the bulk partition kernel");
     Scratch &sc = m->sc;
     if (dalloc(&m->alt, n) || sc.get(&m->lvl0, 4) || sc.get(&m->histA, nbA) || sc.get(&m->offA, nbA) ||
         sc.get(&m->curA, nbA) || sc.get(&m->tstart1, nbA + 1) || sc.get(&m->histB, nsub) || sc.get(&m->suboff, nsub) ||
@@ -684,32 +625,15 @@ int msd_level_a(const MsdPlan &p, MsdLevels *m, const u64 *in, bool from_col, co
     LAUNCH("radix_bases", k_radix_bases, 1, (int)nbA, 0, histA, offA);
     CK(cudaMemcpyAsync(curA, offA, nbA * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
     const u32 ntiles_cap = ntiles0 + nbA;
-    const int bulk_grid = G.sms * 3;
-    if (p.bulk) {
-        if (sc.get(&m->tdesc, ntiles_cap) != 0) return -1;
-        LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles0, 256), 256, 0, lvl0, lvl0 + 2, lvl0 + 3, 1u, ntiles0, m->tdesc);
-        if (from_col)
-            LAUNCH("msd_partition", k_msd_partition_bulk<true>, (int)std::min<u32>(ntiles0, (u32)bulk_grid), QCE_MSDB_THREADS,
-                   QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0, base, shiftA, nbA, curA);
-        else
-            LAUNCH("msd_partition", k_msd_partition_bulk<false>, (int)std::min<u32>(ntiles0, (u32)bulk_grid), QCE_MSDB_THREADS,
-                   QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0, base, shiftA, nbA, curA);
-    } else
-    if (shape >= 1 && variant == 1)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, false>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
-               base, shiftA, nbA, curA, (const u32 *)nullptr);
-    else if (shape >= 1 && variant == 2)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 3, true>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
-               base, shiftA, nbA, curA, (const u32 *)nullptr);
-    else if (shape >= 1 && variant == 3)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, true>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
-               base, shiftA, nbA, curA, (const u32 *)nullptr);
-    else if (shape >= 1)
-        LAUNCH("msd_partition", (k_msd_partition<512, 8>), ntiles0, 512, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
-               base, shiftA, nbA, curA, (const u32 *)nullptr);
+    const int grid = (int)std::min<u32>(ntiles0, (u32)G.sms * 3);
+    if (sc.get(&m->tdesc, ntiles_cap) != 0) return -1;
+    LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles0, 256), 256, 0, lvl0, lvl0 + 2, lvl0 + 3, 1u, ntiles0, m->tdesc);
+    if (from_col)
+        LAUNCH("msd_partition", k_msd_partition_bulk<true>, grid, QCE_MSDB_THREADS, QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0,
+               base, shiftA, nbA, curA);
     else
-        LAUNCH("msd_partition", (k_msd_partition<256, 16>), ntiles0, 256, 0, in, alt, lvl0, lvl0 + 2, lvl0 + 3, 1u,
-               base, shiftA, nbA, curA, (const u32 *)nullptr);
+        LAUNCH("msd_partition", k_msd_partition_bulk<false>, grid, QCE_MSDB_THREADS, QCE_MSDB_SMEM, in, alt, m->tdesc, ntiles0,
+               base, shiftA, nbA, curA);
     return 0;
 }
 
@@ -720,9 +644,8 @@ int msd_after_level_a(const MsdPlan &p, MsdLevels *m, u64 **keys, bool *done)
 {
     *done = false;
     const u64 base = p.base;
-    const int R = p.R, shiftB = p.shiftB, shape = p.shape, variant = p.variant, bulk = p.bulk;
+    const int R = p.R, shiftB = p.shiftB;
     const u32 nbA = p.nbA, nbB = p.nbB, nsub = p.nsub, ntiles0 = p.ntiles0;
-    const int bulk_grid = G.sms * 3;
     Scratch &sc = m->sc;
     u64 *alt = m->alt;
     u32 *histA = m->histA, *offA = m->offA, *tstart1 = m->tstart1, *histB = m->histB, *suboff = m->suboff, *curB = m->curB;
@@ -740,8 +663,6 @@ int msd_after_level_a(const MsdPlan &p, MsdLevels *m, u64 **keys, bool *done)
     if (big_path < 0) {
         const char *e = getenv("QCE_MSD_BIG");
         big_path = e ? atoi(e) : 1;
-        CK(cudaFuncSetAttribute(k_big_partition<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)(QCE_MSD_TILE * sizeof(u64) + 3 * 4096 * sizeof(u32))));
     }
     u32 *big_off = nullptr, *big_size = nullptr, *big_tiles = nullptr;
     if (sc.get(&big_off, BIG_MAX) || sc.get(&big_size, BIG_MAX) || sc.get(&big_tiles, BIG_MAX)) return -1;
@@ -757,93 +678,24 @@ int msd_after_level_a(const MsdPlan &p, MsdLevels *m, u64 **keys, bool *done)
     const bool big_route = max_sub > MSD_LOCAL_CAP && big_path && R > 0 && R <= 12 && nbig <= BIG_MAX;
     if (max_sub <= MSD_LOCAL_CAP || R == 0 || big_route) {
         CK(cudaMemcpyAsync(curB, suboff, nsub * sizeof(u32), cudaMemcpyDeviceToDevice, cx().stream));
-        if (bulk) {
-            LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles1, 256), 256, 0, tstart1, offA, histA, nbA, ntiles1, tdesc);
-            LAUNCH("msd_partition", k_msd_partition_bulk<false>, (int)std::min<u32>(ntiles1, (u32)bulk_grid), QCE_MSDB_THREADS, QCE_MSDB_SMEM, alt,
-                   *keys, tdesc, ntiles1, base, shiftB, nbB, curB);
-        } else
-        if (shape >= 1 && variant == 1)
-            LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, false>), ntiles1, 512, 0, alt, *keys, tstart1, offA, histA, nbA,
-                   base, shiftB, nbB, curB, (const u32 *)nullptr);
-        else if (shape >= 1 && variant == 2)
-            LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 3, true>), ntiles1, 512, 0, alt, *keys, tstart1, offA, histA, nbA,
-                   base, shiftB, nbB, curB, (const u32 *)nullptr);
-        else if (shape >= 1 && variant == 3)
-            LAUNCH("msd_partition", (k_msd_partition<512, 8, u64, 4, true>), ntiles1, 512, 0, alt, *keys, tstart1, offA, histA, nbA,
-                   base, shiftB, nbB, curB, (const u32 *)nullptr);
-        else if (shape >= 1)
-            LAUNCH("msd_partition", (k_msd_partition<512, 8>), ntiles1, 512, 0, alt, *keys, tstart1, offA, histA, nbA,
-                   base, shiftB, nbB, curB, (const u32 *)nullptr);
-        else
-            LAUNCH("msd_partition", (k_msd_partition<256, 16>), ntiles1, 256, 0, alt, *keys, tstart1, offA, histA, nbA,
-                   base, shiftB, nbB, curB, (const u32 *)nullptr);
+        LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles1, 256), 256, 0, tstart1, offA, histA, nbA, ntiles1, tdesc);
+        LAUNCH("msd_partition", k_msd_partition_bulk<false>, (int)std::min<u32>(ntiles1, (u32)G.sms * 3), QCE_MSDB_THREADS,
+               QCE_MSDB_SMEM, alt, *keys, tdesc, ntiles1, base, shiftB, nbB, curB);
         if (R > 0 && R <= 12) {
-            const size_t sm8 = 256 * 8 * sizeof(u64) + 4096 * sizeof(u32) + 33 * sizeof(u32);
-            const size_t sm16 = 256 * 16 * sizeof(u64) + 4096 * sizeof(u32) + 33 * sizeof(u32);
-            const size_t sm12 = 256 * 12 * sizeof(u64) + 4096 * sizeof(u32) + 33 * sizeof(u32);
-            static int mid_shape = -1; // QCE_COUNT_SORT_MID=0 disables the 3072-tuple shape
-            if (mid_shape < 0) { const char *e = getenv("QCE_COUNT_SORT_MID"); mid_shape = e ? atoi(e) : 1; }
-            static bool attr_set = false;
-            if (!attr_set) {
-                CK(cudaFuncSetAttribute(k_msd_count_sort<256, 8, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm8));
-                CK(cudaFuncSetAttribute(k_msd_count_sort<256, 16, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16));
-                CK(cudaFuncSetAttribute(k_msd_count_sort<256, 12, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm12));
-                CK(cudaFuncSetAttribute(k_msd_count_sort<512, 8, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16));
-                CK(cudaFuncSetAttribute(k_msd_count_sort<512, 8, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16));
-                CK(cudaFuncSetAttribute(k_msd_count_sort<512, 8, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16));
-                attr_set = true;
-            }
-            static int small_counters = -1; // QCE_COUNT_SORT_SMALL=0: always clear and scan 4096 counters
-            if (small_counters < 0) {
-                const char *e = getenv("QCE_COUNT_SORT_SMALL");
-                small_counters = e ? atoi(e) : 1;
-                CK(cudaFuncSetAttribute((k_msd_count_sort<256, 12, 4, 2048>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm12));
-                CK(cudaFuncSetAttribute((k_msd_count_sort<256, 12, 4, 1024>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm12));
-                CK(cudaFuncSetAttribute((k_msd_count_sort<256, 8, 4, 2048>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm8));
-                CK(cudaFuncSetAttribute((k_msd_count_sort<256, 8, 4, 1024>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm8));
-            }
-            // persistent, bulk-copy pipelined variant (QCE_COUNT_SORT_BULK=0: the plain kernels below)
-            static int cs_bulk = -1;
-            constexpr size_t csb_tile = (256 * 12 + 2) * sizeof(u64) * 2;
-            if (cs_bulk < 0) {
-                const char *e = getenv("QCE_COUNT_SORT_BULK");
-                cs_bulk = e ? atoi(e) : 1;
-                CK(cudaFuncSetAttribute((k_msd_count_sort_bulk<256, 12, 1024>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(csb_tile + 1024 * 4)));
-                CK(cudaFuncSetAttribute((k_msd_count_sort_bulk<256, 12, 2048>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(csb_tile + 2048 * 4)));
-                CK(cudaFuncSetAttribute((k_msd_count_sort_bulk<256, 12, 4096>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(csb_tile + 4096 * 4)));
-            }
-            if (cs_bulk && (max_sub <= 256 * 12 || big_route)) {
+            if (max_sub <= 256 * 12 || big_route) {
+                // persistent, bulk-copy pipelined; the oversized sub-buckets of the big route are skipped here
                 const int cgrid = (int)std::min<u32>(nsub, (u32)G.sms * 3);
                 if (R <= 10)
-                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 1024>), cgrid, 256, csb_tile + 1024 * 4, *keys, suboff, histB, nsub, base, R);
+                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 1024>), cgrid, 256, CSB_TILE + 1024 * sizeof(u32),
+                           *keys, suboff, histB, nsub, base, R);
                 else if (R == 11)
-                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 2048>), cgrid, 256, csb_tile + 2048 * 4, *keys, suboff, histB, nsub, base, R);
+                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 2048>), cgrid, 256, CSB_TILE + 2048 * sizeof(u32),
+                           *keys, suboff, histB, nsub, base, R);
                 else
-                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 4096>), cgrid, 256, csb_tile + 4096 * 4, *keys, suboff, histB, nsub, base, R);
-            } else {
-            const size_t cut11 = 2048 * sizeof(u32), cut10 = 3072 * sizeof(u32); // counters not needed below 12 / 11 bits
-            if (max_sub <= 256 * 8 && small_counters && R <= 10)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 8, 4, 1024>), nsub, 256, sm8 - cut10, *keys, suboff, histB, base, R);
-            else if (max_sub <= 256 * 8 && small_counters && R == 11)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 8, 4, 2048>), nsub, 256, sm8 - cut11, *keys, suboff, histB, base, R);
-            else if (max_sub <= 256 * 8)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 8, 4>), nsub, 256, sm8, *keys, suboff, histB, base, R);
-            else if (big_route)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 12, 4>), nsub, 256, sm12, *keys, suboff, histB, base, R);
-            else if (mid_shape && max_sub <= 256 * 12 && small_counters && R <= 10)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 12, 4, 1024>), nsub, 256, sm12 - cut10, *keys, suboff, histB, base, R);
-            else if (mid_shape && max_sub <= 256 * 12 && small_counters && R == 11)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 12, 4, 2048>), nsub, 256, sm12 - cut11, *keys, suboff, histB, base, R);
-            else if (mid_shape && max_sub <= 256 * 12) // sparse key ranges leave sub-buckets of 2-3 K tuples
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 12, 4>), nsub, 256, sm12, *keys, suboff, histB, base, R);
-            else if (shape == 1)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<512, 8, 2>), nsub, 512, sm16, *keys, suboff, histB, base, R);
-            else if (shape == 2)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<512, 8, 3>), nsub, 512, sm16, *keys, suboff, histB, base, R);
-            else if (shape == 3)
-                LAUNCH("msd_count_sort", (k_msd_count_sort<512, 8, 4>), nsub, 512, sm16, *keys, suboff, histB, base, R);
-            else
-                LAUNCH("msd_count_sort", (k_msd_count_sort<256, 16, 3>), nsub, 256, sm16, *keys, suboff, histB, base, R);
+                    LAUNCH("msd_count_sort", (k_msd_count_sort_bulk<256, 12, 4096>), cgrid, 256, CSB_TILE + 4096 * sizeof(u32),
+                           *keys, suboff, histB, nsub, base, R);
+            } else { // 3072 < max_sub <= 4096
+                LAUNCH("msd_count_sort", (k_msd_count_sort<512, 8, 3>), nsub, 512, CS_SMEM, *keys, suboff, histB, base, R);
             }
             if (big_route && nbig > 0) {
                 // the oversized sub-buckets: one more counting pass on all their remaining bits, through alt
@@ -857,8 +709,8 @@ int msd_after_level_a(const MsdPlan &p, MsdLevels *m, u64 **keys, bool *done)
                 LAUNCH("msd_tiles", k_msd_tile_desc, (int)ceil_div(ntiles_big, 256), 256, 0, tstartB, big_off, big_size, nbig, ntiles_big, bdesc);
                 LAUNCH("msd_big_hist", k_big_hist<4096>, (int)ntiles_big, 512, 0, *keys, bdesc, base, R, bhist);
                 LAUNCH("msd_big_scan", k_big_scan, (int)nbig, 1024, 0, bhist, nbR);
-                LAUNCH("msd_big_partition", k_big_partition<4096>, (int)ntiles_big, 512,
-                       QCE_MSD_TILE * sizeof(u64) + 3 * 4096 * sizeof(u32), *keys, alt, bdesc, big_off, base, R, bhist);
+                LAUNCH("msd_big_partition", k_big_partition<4096>, (int)ntiles_big, 512, BIG_SMEM, *keys, alt, bdesc, big_off,
+                       base, R, bhist);
                 LAUNCH("msd_big_copy", k_big_copyback, (int)ntiles_big, 512, 0, alt, *keys, bdesc);
             }
         } else if (R > 0) {
@@ -900,10 +752,8 @@ int msd_sort(u64 **keys, u64 n, u64 key_min, u64 key_max, bool *done, const u32 
 // The LSD passes over a packed run's `key_bits` key bits.
 int lsd_sort_packed(u64 **a, u64 n, int key_bits)
 {
-    // k_block_sort ranks 8-bit digits: 9-bit shifts would skip every ninth key bit
-    const int db = n <= BS_TILE ? 8 : digit_bits_for(key_bits, true);
-    RadixShifts rs = shifts_for(32, key_bits, db);
-    return radix_sort(a, nullptr, n, rs, db);
+    RadixShifts rs = shifts_for(32, key_bits);
+    return radix_sort(a, nullptr, n, rs);
 }
 
 // Sort a packed run on its `key_bits` key bits.
@@ -2265,7 +2115,7 @@ int qce_sort_tuples(qce_tuples *t)
         // the sort would have noticed a run of few distinct keys (msd_sort); here the statistics have to
         if (t->key_max < ~0ull && t->n / (t->key_max + 1) >= 16) tl_sort_skewed = true;
     } else if (t->wide) {
-        RadixShifts rs = shifts_for(0, t->range_sort ? bitlen(t->key_min ^ t->key_max) : t->key_bits, 8);
+        RadixShifts rs = shifts_for(0, t->range_sort ? bitlen(t->key_min ^ t->key_max) : t->key_bits);
         rc = radix_sort(&t->a, &t->ids, t->n, rs);
     } else {
         // the cached histogram counts key >> (hist_key_bits - 8); level A of the MSD sort counts
@@ -2307,7 +2157,7 @@ int qce_build_sorted_tuples_base(uint32_t rel, uint32_t col, qce_tuples **out)
         applies = msd_plan(cl->n, 0, cl->maxv, &p);
         if (applies < 0) return -1;
     }
-    if (!applies || !p.bulk) {
+    if (!applies) {
         if (build_base(cl, rel, col, &t) != 0) return -1;
         if (qce_sort_tuples(t) != 0) { qce_tuples_free(t); return -1; }
         *out = t;

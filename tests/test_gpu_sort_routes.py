@@ -32,22 +32,18 @@ P_MIN, P_MAX, P_AVG = 9, 16, 2700   # partition bits: the smallest P whose avera
 MSD_LOCAL_CAP = 4096                # largest finish tile (k_msd_local_sort<256, 16>, k_msd_count_sort<512, 8>)
 BIG_CAP, BIG_MAX = 3072, 8192       # k_big_list: sub-buckets over 3072 tuples, at most 8192 of them
 COUNT_MAX_R = 12                    # the count sort holds 2^R <= 4096 counters
-ONESWEEP_TILES = (256 * 16, 256 * 24, 384 * 12)  # threads x items of kOnesweepCfgs (QCE_ONESWEEP_CFG=0..5)
+BULK_COUNT_CAP = 3072               # k_msd_count_sort_bulk<256, 12>: sub-buckets of up to 3072 tuples
+ONESWEEP_TILE = 256 * 16            # k_onesweep: threads x items
 
-SORT_SWITCHES = ("QCE_MSD", "QCE_MSD_BULK", "QCE_MSD_SHAPE", "QCE_MSD_VARIANT", "QCE_MSD_BIG", "QCE_COUNT_SORT_BULK",
-                 "QCE_COUNT_SORT_SMALL", "QCE_COUNT_SORT_MID", "QCE_DIGIT_BITS", "QCE_ONESWEEP_CFG", "QCE_FUSED_BUILD_HIST",
-                 "QCE_SORT_PROBE")
+SORT_SWITCHES = ("QCE_MSD", "QCE_MSD_BIG", "QCE_FUSED_BUILD_HIST", "QCE_SORT_PROBE")
 
 # kernel families whose launch counts identify a route (a tag names a family, not a template instance)
 WATCH = ("block_sort", "radix_hist", "onesweep_k", "onesweep_kv", "msd_hist", "msd_partition", "msd_count_sort",
          "msd_local_sort", "msd_big_partition")
 
-COUNT_SHAPES = ["256x8x4_1024", "256x8x4_2048", "256x8x4_4096", "256x12x4_1024", "256x12x4_2048", "256x12x4_4096",
-                "512x8x2_4096", "512x8x3_4096", "512x8x4_4096", "256x16x3_4096"]
-ROUTES = (["block", "lsd8", "lsd9", "msd_bulk_1024", "msd_bulk_2048", "msd_bulk_4096"]
-          + ["msd_count_" + s for s in COUNT_SHAPES]
-          + ["msd_big", "msd_local", "msd_r0", "msd_lsd_fallback", "wide_block", "wide_onesweep", "in_order"])
-STABLE = {"block", "lsd8", "lsd9", "msd_lsd_fallback", "wide_block", "wide_onesweep", "in_order"}
+ROUTES = ["block", "lsd", "msd_bulk_1024", "msd_bulk_2048", "msd_bulk_4096", "msd_count_512x8x3", "msd_big", "msd_local",
+          "msd_r0", "msd_lsd_fallback", "wide_block", "wide_onesweep", "in_order"]
+STABLE = {"block", "lsd", "msd_lsd_fallback", "wide_block", "wide_onesweep", "in_order"}
 
 
 def _bitlen(x: int) -> int:
@@ -66,12 +62,8 @@ def _sw(env, name, default):
 
 
 def switches(env):
-    digit = _sw(env, "QCE_DIGIT_BITS", 0)
-    return {"msd": _sw(env, "QCE_MSD", 1), "shape": _sw(env, "QCE_MSD_SHAPE", 2),
-            "big": _sw(env, "QCE_MSD_BIG", 1), "cs_bulk": _sw(env, "QCE_COUNT_SORT_BULK", 1),
-            "small": _sw(env, "QCE_COUNT_SORT_SMALL", 1), "mid": _sw(env, "QCE_COUNT_SORT_MID", 1),
-            "digit_bits": digit if digit in (8, 9) else 8, "fused_hist": _sw(env, "QCE_FUSED_BUILD_HIST", 1),
-            "probe": _sw(env, "QCE_SORT_PROBE", 1)}
+    return {"msd": _sw(env, "QCE_MSD", 1), "big": _sw(env, "QCE_MSD_BIG", 1),
+            "fused_hist": _sw(env, "QCE_FUSED_BUILD_HIST", 1), "probe": _sw(env, "QCE_SORT_PROBE", 1)}
 
 
 def partition_bits(n: int, span: int):
@@ -81,26 +73,6 @@ def partition_bits(n: int, span: int):
     while P < P_MAX and P < kb and n // ((span >> (kb - P)) + 1) > P_AVG:
         P += 1
     return None if n // ((span >> (kb - P)) + 1) > P_AVG else P
-
-
-def _count_shape(sw, R, max_sub, big_route):
-    """The plain count-sort instance msd_sort launches (QCE_COUNT_SORT_BULK=0 or 3072 < max_sub <= 4096)."""
-    small, mid = sw["small"], sw["mid"]
-    if max_sub <= 2048 and small and R <= 10:
-        return "256x8x4_1024"
-    if max_sub <= 2048 and small and R == 11:
-        return "256x8x4_2048"
-    if max_sub <= 2048:
-        return "256x8x4_4096"
-    if big_route:
-        return "256x12x4_4096"
-    if mid and max_sub <= 3072 and small and R <= 10:
-        return "256x12x4_1024"
-    if mid and max_sub <= 3072 and small and R == 11:
-        return "256x12x4_2048"
-    if mid and max_sub <= 3072:
-        return "256x12x4_4096"
-    return {1: "512x8x2_4096", 2: "512x8x3_4096", 3: "512x8x4_4096"}.get(sw["shape"], "256x16x3_4096")
 
 
 def _msd(keys, n, kmin, kmax, hist_bits, sw, info):
@@ -132,13 +104,13 @@ def _msd(keys, n, kmin, kmax, hist_bits, sw, info):
         tags["msd_local_sort"] = 1
         return "msd_local", tags
     tags["msd_count_sort"] = 1
-    if sw["cs_bulk"] and (max_sub <= 3072 or big_route):
+    if max_sub <= BULK_COUNT_CAP or big_route:
         maxb = 1024 if R <= 10 else (2048 if R == 11 else 4096)
         info["count_sort"] = "bulk_%d" % maxb
         route = "msd_bulk_%d" % maxb
-    else:
-        info["count_sort"] = _count_shape(sw, R, max_sub, big_route)
-        route = "msd_count_" + info["count_sort"]
+    else:  # BULK_COUNT_CAP < max_sub <= MSD_LOCAL_CAP
+        info["count_sort"] = "512x8x3"
+        route = "msd_count_512x8x3"
     if big_route:
         tags["msd_big_partition"] = 1
         route = "msd_big"
@@ -175,9 +147,8 @@ def plan(run, keys, env):
         return route, tags, info
     if n <= BS_TILE:
         return "block", {"block_sort": 1}, info
-    db = sw["digit_bits"]
-    tags.update(radix_hist=1, onesweep_k=-(-key_bits // db))
-    return ("msd_lsd_fallback" if tags.get("msd_hist") else "lsd%d" % db), tags, info
+    tags.update(radix_hist=1, onesweep_k=-(-key_bits // 8))
+    return ("msd_lsd_fallback" if tags.get("msd_hist") else "lsd"), tags, info
 
 
 # ---- cases ---------------------------------------------------------------------------------------------------
@@ -195,7 +166,7 @@ CASES = {
     "lsd_2^20-1_b20": dict(kind="host", n=(1 << 20) - 1, bits=20),
     "lsd_2^20+1_b8": dict(kind="host", n=(1 << 20) + 1, bits=8),            # key bits below 9: no MSD attempt
     "lsd_dense_b9": dict(kind="host", n=1_500_001, bits=9),                  # P cannot reach 2700 per sub-bucket
-    **{"lsd_%d_b27" % (3 * t + d): dict(kind="host", n=3 * t + d, bits=27) for t in ONESWEEP_TILES for d in (-1, 1)},
+    **{"lsd_%d_b27" % (3 * ONESWEEP_TILE + d): dict(kind="host", n=3 * ONESWEEP_TILE + d, bits=27) for d in (-1, 1)},
     # MSD at R = 0 .. 20 remaining bits
     "r0_2^20_b9": dict(kind="host", n=1 << 20, bits=9),
     "r0_odd_b10": dict(kind="host", n=N_ODD, bits=10),
@@ -235,67 +206,34 @@ CASES = {
     "wide_os_hi_100003": dict(kind="host", n=100003, wide="hi"),
 }
 
-_LSD_TILES = ["lsd_%d_b27" % (3 * t + d) for t in ONESWEEP_TILES for d in (-1, 1)]
+_LSD_TILES = ["lsd_%d_b27" % (3 * ONESWEEP_TILE + d) for d in (-1, 1)]
 _WIDE = ["wide_block_max_4096", "wide_block_hi_3001", "wide_os_max_4097", "wide_os_hi_12289", "wide_os_top_18433",
          "wide_os_hi_100003"]
 _WIDE_ROUTES = {c: ("wide_block" if CASES[c]["n"] <= BS_TILE else "wide_onesweep") for c in _WIDE}
-_BULK_PLANTS = {"plant%d_r%d" % (s, r): ("msd_bulk_%d" % m if s <= 3072 else
-                                         ("msd_count_512x8x3_4096" if s <= 4096 else "msd_big"))
+_BULK_PLANTS = {"plant%d_r%d" % (s, r): ("msd_bulk_%d" % m if s <= BULK_COUNT_CAP else
+                                         ("msd_count_512x8x3" if s <= MSD_LOCAL_CAP else "msd_big"))
                 for r, m in ((10, 1024), (11, 2048), (12, 4096)) for s in (2048, 2049, 3072, 3073, 4096, 4097)}
-_PARTITION_CASES = {"r12_odd_b22": "msd_bulk_4096", "r0_odd_b10": "msd_r0", "r13_odd_b23": "msd_local",
-                    "plant4097_r12": "msd_big", "dev_lo_hi_b22": "msd_bulk_4096", "built_b22": "msd_bulk_4096"}
-_PLAIN_COUNT = {"plant2048_r10": "256x8x4_1024", "plant2049_r10": "256x12x4_1024", "plant2048_r11": "256x8x4_2048",
-                "plant3072_r11": "256x12x4_2048", "plant2048_r12": "256x8x4_4096", "plant3072_r12": "256x12x4_4096"}
-
-
-def _count_bulk_off(shape):
-    big = {"plant3073_r12": None, "plant4096_r12": None, "plant4097_r12": "msd_big", "dev_lo_plant4097": "msd_big"}
-    cases = {c: "msd_count_" + s for c, s in _PLAIN_COUNT.items()} if shape == 2 else {}
-    for c, r in big.items():
-        cases[c] = r or "msd_count_" + {0: "256x16x3_4096", 1: "512x8x2_4096", 2: "512x8x3_4096",
-                                        3: "512x8x4_4096"}[shape]
-    return cases
 
 
 # switch set -> (environment, {case: route it must take})
 SWITCH_SETS = {
     "defaults": ({}, {
-        "block_1000_b12": "block", "block_4096_b27": "block", "lsd_4097_b27": "lsd8", "lsd_2^20-1_b20": "lsd8",
-        "lsd_2^20+1_b8": "lsd8", "lsd_dense_b9": "lsd8", **{c: "lsd8" for c in _LSD_TILES},
+        "block_1000_b12": "block", "block_4096_b27": "block", "lsd_4097_b27": "lsd", "lsd_2^20-1_b20": "lsd",
+        "lsd_2^20+1_b8": "lsd", "lsd_dense_b9": "lsd", **{c: "lsd" for c in _LSD_TILES},
         "r0_2^20_b9": "msd_r0", "r0_odd_b10": "msd_r0", "r1_odd_b11": "msd_bulk_1024", "r10_odd_b20": "msd_bulk_1024",
         "r11_odd_b21": "msd_bulk_2048", "r12_odd_b22": "msd_bulk_4096", "r12_2^20_b21": "msd_bulk_4096",
         "r13_odd_b23": "msd_local", "r16_odd_b26": "msd_local", "r20_odd_b30": "msd_local",
         **_BULK_PLANTS, "plant4096_r13": "msd_local", "plant4097_r13": "msd_lsd_fallback",
         "many_big_r12": "msd_lsd_fallback",
-        "dev_lo_hi_unknown": "msd_local", "dev_lo_hi_b22": "msd_bulk_4096", "dev_lo_eq_hi": "lsd8",
+        "dev_lo_hi_unknown": "msd_local", "dev_lo_hi_b22": "msd_bulk_4096", "dev_lo_eq_hi": "lsd",
         "dev_lo_plant4097": "msd_big",
         "built_b22": "msd_bulk_4096", "built_ids_b24": "msd_local", "built_b22_hist24": "msd_bulk_4096",
         "built_b22_hist22": "msd_bulk_4096", "host_b22_hist22": "msd_bulk_4096", "in_order_2^20+1": "in_order",
         **_WIDE_ROUTES}),
-    "msd-off": ({"QCE_MSD": "0"}, {"r12_odd_b22": "lsd8", "r0_2^20_b9": "lsd8", "plant4097_r12": "lsd8",
-                                   "built_b22": "lsd8", "dev_lo_hi_b22": "lsd8"}),
-    # QCE_MSD_SHAPE also picks the count sort of 3072 < max_sub <= 4096
-    **{"partition-%s" % tag: (dict(QCE_MSD_BULK="0", QCE_MSD_SHAPE=s, QCE_MSD_VARIANT=v),
-                              dict(_PARTITION_CASES, plant3073_r12="msd_count_%s_4096" % ("256x16x3" if s == "0" else "512x8x3")))
-       for tag, s, v in (("256x16", "0", "0"), ("512x8", "2", "0"), ("512x8-32regs", "2", "1"),
-                         ("512x8-vec", "2", "2"), ("512x8-32regs-vec", "2", "3"))},
-    **{"count-plain-shape%d" % s: (dict(QCE_COUNT_SORT_BULK="0", QCE_MSD_SHAPE=str(s)), _count_bulk_off(s))
-       for s in range(4)},
-    "count-small-off": (dict(QCE_COUNT_SORT_BULK="0", QCE_COUNT_SORT_SMALL="0"), {
-        "plant2048_r10": "msd_count_256x8x4_4096", "plant2048_r11": "msd_count_256x8x4_4096",
-        "plant2049_r10": "msd_count_256x12x4_4096", "plant3072_r11": "msd_count_256x12x4_4096"}),
-    "count-mid-off": (dict(QCE_COUNT_SORT_BULK="0", QCE_COUNT_SORT_MID="0"), {
-        "plant2048_r10": "msd_count_256x8x4_1024", "plant2049_r10": "msd_count_512x8x3_4096",
-        "plant3072_r12": "msd_count_512x8x3_4096"}),
+    "msd-off": ({"QCE_MSD": "0"}, {"r12_odd_b22": "lsd", "r0_2^20_b9": "lsd", "plant4097_r12": "lsd",
+                                   "built_b22": "lsd", "dev_lo_hi_b22": "lsd"}),
     "big-off": ({"QCE_MSD_BIG": "0"}, {"plant4097_r12": "msd_lsd_fallback", "plant4097_r10": "msd_lsd_fallback",
-                                       "dev_lo_plant4097": "msd_lsd_fallback", "plant4096_r12": "msd_count_512x8x3_4096"}),
-    "digit-bits-9": ({"QCE_DIGIT_BITS": "9"}, {
-        "block_1000_b12": "block", "block_4096_b27": "block", "lsd_4097_b27": "lsd9", "lsd_2^20-1_b20": "lsd9",
-        "lsd_2^20+1_b8": "lsd9", "lsd_dense_b9": "lsd9", "plant4097_r13": "msd_lsd_fallback",
-        "dev_lo_eq_hi": "lsd9", "r12_odd_b22": "msd_bulk_4096", "wide_os_hi_12289": "wide_onesweep"}),
-    **{"onesweep-cfg%d" % c: ({"QCE_ONESWEEP_CFG": str(c)}, {
-        "lsd_4097_b27": "lsd8", **{t: "lsd8" for t in _LSD_TILES}, "plant4097_r13": "msd_lsd_fallback",
-        **{w: r for w, r in _WIDE_ROUTES.items() if r == "wide_onesweep"}}) for c in range(1, 6)},
+                                       "dev_lo_plant4097": "msd_lsd_fallback", "plant4096_r12": "msd_count_512x8x3"}),
     "build-hist-off": ({"QCE_FUSED_BUILD_HIST": "0"}, {"built_b22": "msd_bulk_4096", "built_ids_b24": "msd_local",
                                                         "built_b22_hist22": "msd_bulk_4096"}),
     "probe-off": ({"QCE_SORT_PROBE": "0"}, {"in_order_2^20+1": "msd_bulk_4096", "built_b22": "msd_bulk_4096"}),
@@ -423,10 +361,8 @@ def test_planner_restates_edges():
     assert partition_bits(2700 * 512, (1 << 20) - 1) == 9 and partition_bits(2700 * 512 + 512, (1 << 20) - 1) == 10
     assert partition_bits(26_000_000, (1 << 26) - 1) == 14
     assert partition_bits(P_AVG * (1 << 16) + (1 << 16), (1 << 32) - 1) is None
-    sw = switches({})
-    assert _count_shape(sw, 12, 3073, False) == "512x8x3_4096"
-    assert _count_shape(switches({"QCE_MSD_SHAPE": "0"}), 12, 3073, False) == "256x16x3_4096"
-    assert switches({"QCE_DIGIT_BITS": "7"})["digit_bits"] == 8
+    assert switches({}) == {"msd": 1, "big": 1, "fused_hist": 1, "probe": 1}
+    assert switches({"QCE_MSD_BIG": "off"})["big"] == 0        # atoi: a value that is not a number reads as 0
 
 
 # ---- GPU: every switch set in a fresh process (the switches are read once per process) --------------------------

@@ -3,8 +3,3 @@ for cfg in "QCE_CHECKSUM_PER_COL=0 QCE_CHECKSUM_WAVES=1" "QCE_CHECKSUM_PER_COL=0
   python -c "
 import json; d=json.load(open('gpurun_out/ck.json')); k=d['roofline']['kernels_ms_per_step']; print('$cfg', round(d['ms_per_step'],3), 'checksum', k.get('checksum'), d['parity']['full_vs_checker'])"
 done
-for cfg in "QCE_COUNT_SORT_SMALL=0 QCE_CHECKSUM_WAVES=3" "QCE_COUNT_SORT_SMALL=1 QCE_CHECKSUM_WAVES=3"; do
-  env $cfg python bench.py --config c2 --steps 6 --warmup 3 --no-cpu-baseline > gpurun_out/ck.json 2> gpurun_out/ck.err
-  python -c "
-import json; d=json.load(open('gpurun_out/ck.json')); k=d['roofline']['kernels_ms_per_step']; print('$cfg', round(d['ms_per_step'],3), 'count_sort', k.get('msd_count_sort'), d['parity']['full_vs_checker'])"
-done

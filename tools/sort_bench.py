@@ -1,38 +1,44 @@
-"""Sweep the one-sweep tile shapes (QCE_ONESWEEP_CFG) on one 100M-row sort.
-Each configuration runs in its own process (the choice is read once)."""
-import json, os, subprocess, sys
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CHILD = r'''
-import sys, os, json
-sys.path.insert(0, %r)
-import numpy as np, qce_b200
-n = int(float(sys.argv[1]))
+"""Time the LSD one-sweep pass (k_onesweep) and its digit histogram (k_radix_hist) on one packed sort.
+
+usage: python tools/sort_bench.py [rows, default 1e8]
+
+The run is built from a column of `rows` uniform keys below `rows` and sorted with the MSD route turned off
+(QCE_MSD=0), so every one of its digits takes a one-sweep pass.  Prints one JSON line: ms per pass, the pass's
+rate over its 16 B per tuple, and k_radix_hist's ms per sort, each from the launch profile of three sorts after two
+warm-up sorts.  `ok` also checks a 300001-tuple sort against numpy's stable argsort."""
+import json
+import os
+import sys
+
+os.environ["QCE_MSD"] = "0"  # read by the engine at its first sort
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import numpy as np  # noqa: E402
+import qce_b200  # noqa: E402
+
+n = int(float(sys.argv[1])) if len(sys.argv) > 1 else 100_000_000
 e = qce_b200.Engine()
 rng = np.random.default_rng(1)
 col = rng.integers(0, n, n, dtype=np.uint64)
 e.upload_column(0, 0, col)
 small = rng.integers(0, 1 << 27, 300001, dtype=np.uint64)
-t = e.tuples_from_host(small, np.arange(len(small), dtype=np.uint64)); e.sort_tuples(t)
-k, p = e.tuples_to_host(t); o = np.argsort(small, kind="stable")
-ok = bool((k == small[o]).all() and (p == o.astype(np.uint64)).all()); e.tuples_free(t)
+t = e.tuples_from_host(small, np.arange(len(small), dtype=np.uint64))
+e.sort_tuples(t)
+k, p = e.tuples_to_host(t)
+o = np.argsort(small, kind="stable")
+ok = bool((k == small[o]).all() and (p == o.astype(np.uint64)).all())
+e.tuples_free(t)
 for _ in range(2):
-    t = e.build_tuples(0, 0); e.sort_tuples(t); e.tuples_free(t)
+    t = e.build_tuples(0, 0)
+    e.sort_tuples(t)
+    e.tuples_free(t)
 e.profile(True)
 for _ in range(3):
-    t = e.build_tuples(0, 0); e.sort_tuples(t); srt = e.is_sorted(t); e.tuples_free(t)
+    t = e.build_tuples(0, 0)
+    e.sort_tuples(t)
+    ok = ok and e.is_sorted(t)
+    e.tuples_free(t)
 prof = e.profile_read()
+e.profile(False)
 ms = prof["onesweep_k"]["ms"] / prof["onesweep_k"]["launches"]
-print(json.dumps({"cfg": os.environ.get("QCE_ONESWEEP_CFG"), "ok": ok and srt, "ms_per_pass": ms,
+print(json.dumps({"rows": n, "ok": ok, "passes_per_sort": prof["onesweep_k"]["launches"] // 3, "ms_per_pass": ms,
                   "GBps": 16.0 * n / ms / 1e6, "hist_ms": prof["radix_hist"]["ms"] / 3}))
-''' % ROOT
-n = sys.argv[1] if len(sys.argv) > 1 else "1e8"
-cfgs = sys.argv[2].split(",") if len(sys.argv) > 2 else [str(i) for i in range(6)]
-out = []
-for c in cfgs:
-    env = dict(os.environ, QCE_ONESWEEP_CFG=c)
-    p = subprocess.run([sys.executable, "-c", CHILD, n], env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=300)
-    line = p.stdout.strip().splitlines()[-1] if p.stdout.strip() else "ERR " + p.stderr[-300:]
-    print(line, flush=True)
-    out.append(line)
-os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-open(os.path.join(ROOT, "gpurun_out", "sort_sweep.txt"), "w").write("\n".join(out) + "\n")

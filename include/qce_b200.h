@@ -180,7 +180,9 @@ int qce_build_tuples_rowids(uint32_t rel, uint32_t col, const qce_rowids *ids, q
  * build_reordered_array, src/utilities.c:20-70; random_quicksort,
  * src/quicksort.c:54-64): ascending by key.  The order among equal keys is
  * unspecified, as in the reference (its quicksort is rand()-driven): runs below
- * 2^20 tuples are sorted stably, larger ones may take the MSD partition path. */
+ * 2^20 tuples are sorted stably, larger ones may take the MSD partition path.
+ * A run may hold up to 2^31 - 1 tuples (the reference's int limit); a longer one
+ * is refused with an error. */
 int qce_sort_tuples(qce_tuples *t);
 /* qce_build_tuples_base followed by qce_sort_tuples, in one call: the same run, sorted, with the same
  * unspecified order among equal keys.  A large whole column whose run takes the MSD route is never

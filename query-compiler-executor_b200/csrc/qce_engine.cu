@@ -419,11 +419,12 @@ int compact_from_mask(int layout, int mode, const u32 *mask, const u32 *tile_cou
 
 // ---- radix sort driver -------------------------------------------------------
 // One digit pass of the LSD sort (k_onesweep).
-template <bool HAS_VALS, typename DigitOp>
+// BIG: the status-word decode for runs of 2^30 tuples or more (k_radix.cuh).
+template <bool HAS_VALS, bool BIG, typename DigitOp>
 int launch_onesweep(const u64 *kin, u64 *kout, const u32 *vin, u32 *vout, u32 n, DigitOp dop, const u32 *gbase,
                     u32 *status, u32 *counter)
 {
-    auto kern = k_onesweep<HAS_VALS, DigitOp>;
+    auto kern = k_onesweep<HAS_VALS, DigitOp, BIG>;
     const size_t smem = sizeof(OnesweepSmem) + (HAS_VALS ? QCE_OS_TILE * sizeof(u32) : 0);
     static bool attr_set = false; // per instantiation
     if (!attr_set) {
@@ -443,7 +444,9 @@ constexpr int BS_THREADS = 512, BS_ITEMS = 8, BS_TILE = BS_THREADS * BS_ITEMS; /
 int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs)
 {
     if (n <= 1 || rs.npass == 0) return 0;
-    if (n >= (1ull << 30)) return fail("sort of %llu tuples exceeds the 2^30 per-run limit", (unsigned long long)n);
+    // the reference's runs are indexed by int (src/utilities.c:20), and the one-sweep status word holds prefixes below 2^31
+    if (n >= (1ull << 31))
+        return fail("sort of %llu tuples exceeds the per-run limit of 2^31 - 1 tuples", (unsigned long long)n);
     if (n <= BS_TILE) {
         // small run: the whole sort in one CTA (k_block_sort), in place
         const size_t smem = BS_TILE * sizeof(u64) + (vals ? BS_TILE * sizeof(u32) : 0) +
@@ -488,11 +491,17 @@ int radix_sort(u64 **keys, u32 **vals, u64 n, const RadixShifts &rs)
         u32 *gb = gbase + p * bins, *st = status + (u64)p * ntiles * bins;
         const u32 m = (u32)n;
         int rc;
-        if (vals)
-            rc = launch_onesweep<true>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+        if (n >= (1ull << 30)) {
+            if (vals)
+                rc = launch_onesweep<true, true>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+            else
+                rc = rs.shift[p] >= 32 ? launch_onesweep<false, true>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
+                                       : launch_onesweep<false, true>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+        } else if (vals)
+            rc = launch_onesweep<true, false>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
         else
-            rc = rs.shift[p] >= 32 ? launch_onesweep<false>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
-                                   : launch_onesweep<false>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
+            rc = rs.shift[p] >= 32 ? launch_onesweep<false, false>(kin, kout, vin, vout, m, dhi, gb, st, counters + p)
+                                   : launch_onesweep<false, false>(kin, kout, vin, vout, m, dop, gb, st, counters + p);
         if (rc != 0) return -1;
         std::swap(kin, kout);
         std::swap(vin, vout);
@@ -557,13 +566,14 @@ int msd_plan(u64 n, u64 key_min, u64 key_max, MsdPlan *p)
         const char *e = getenv("QCE_MSD");
         enabled = e ? atoi(e) : 1;
     }
-    if (!enabled || n < (1ull << 20) || n >= (1ull << 30)) return 0;
+    if (!enabled || n < (1ull << 20)) return 0;
     // the kernels work on key - key_min, so a run that covers only a slice of the
     // key space (a rank's share after the exchange) still spreads over the buckets
     const u64 base = key_min << 32;
     key_max -= key_min;
     const int key_bits = bitlen(key_max);
     if (n / (key_max + 1) >= 16) tl_sort_skewed = true; // 16 or more tuples per possible key: every join tile is heavy
+    if (n >= (1ull << 30)) return 0; // the LSD passes sort runs this long
     if (key_bits < 9 || key_bits > 32) return 0;
     // Partition bits P: the smallest count for which a populated sub-bucket holds
     // at most ~2700 tuples on average (finish capacity 4096), assuming keys spread

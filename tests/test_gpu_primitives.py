@@ -194,50 +194,6 @@ def test_merge_join_heavy_key(engine):
     assert m >= 6_000_000
 
 
-_JOIN_CHILD = r"""
-import sys, numpy as np
-sys.path.insert(0, %r)
-import qce_b200
-from oracle import qce_oracle as orc
-e = qce_b200.Engine()
-rng = np.random.default_rng(11)
-U64 = np.uint64
-cases = [(rng.integers(0, 100000, 100000, dtype=U64), rng.integers(0, 100000, 100000, dtype=U64)),      # ~1 match per tuple
-         (rng.integers(0, 3000, 40000, dtype=U64), rng.integers(0, 3000, 60000, dtype=U64)),            # ~20 per tuple: the balanced expansion
-         (np.concatenate([np.full(3000, 77, dtype=U64), rng.integers(0, 1000, 5000, dtype=U64)]),
-          np.concatenate([np.full(2000, 77, dtype=U64), rng.integers(0, 1000, 5000, dtype=U64)])),      # one key: 6 M pairs, deferred chunks
-         (rng.integers(0, 50, 4097, dtype=U64), rng.integers(0, 50, 200000, dtype=U64)),                # windows beyond the staging buffer
-         (rng.integers(0, 1 << 34, 50000, dtype=U64), rng.integers(0, 1 << 34, 50000, dtype=U64)),      # wide keys, (almost) no match
-         (rng.integers(0, 1 << 20, 300000, dtype=U64), rng.integers(0, 1 << 20, 1000, dtype=U64))]
-for kR, kS in cases:
-    kR, pR = orc.sort_tuples(kR, np.arange(len(kR), dtype=U64))
-    kS, pS = orc.sort_tuples(kS, np.arange(len(kS), dtype=U64))
-    R, S = e.tuples_from_host(kR, pR), e.tuples_from_host(kS, pS)
-    res = e.merge_join(R, S)
-    gR, gS = e.rowids_to_host(res[0]), e.rowids_to_host(res[1])
-    wR, wS = orc.merge_join(kR, pR, kS, pS)
-    assert (gR == wR).all() and (gS == wS).all(), (len(gR), len(wR))
-    for h in res: e.rowids_free(h)
-    e.tuples_free(R); e.tuples_free(S)
-print("ok")
-"""
-
-
-@pytest.mark.parametrize("env", [{"QCE_JOIN_CAP": "1"}, {"QCE_JOIN_CAP": "70000"}, {"QCE_JOIN_TICKET": "0"},
-                                 {"QCE_JOIN_MINB": "4"}, {"QCE_JOIN_FUSED": "0"}],
-                         ids=["guess-1", "guess-70000", "block-order", "4-ctas", "two-phase"])
-def test_merge_join_routes(env):
-    """The single-pass join under its routing switches, each in a fresh process (they are read once): an output
-    guess of one pair (every later tile is deferred to the chunked writer and the outputs are re-sized), a guess
-    that only some joins overflow, tiles taken in blockIdx order instead of through the ticket, the 64-register build, and the two-phase
-    join it replaces -- all against the oracle's merge."""
-    import os, subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    p = subprocess.run([sys.executable, "-c", _JOIN_CHILD % root], env=dict(os.environ, **env), capture_output=True,
-                       text=True, timeout=300)
-    assert p.returncode == 0 and p.stdout.strip().endswith("ok"), p.stderr[-2000:]
-
-
 def test_merge_join_distinct_pairs(engine):
     """Row ids repeat on both sides (as after an earlier join): the distinct
     (rowid_R,rowid_S) pairs are what the reference's Hashmap dedup keeps."""

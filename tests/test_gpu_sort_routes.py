@@ -76,10 +76,15 @@ def partition_bits(n: int, span: int):
 
 
 def _msd(keys, n, kmin, kmax, hist_bits, sw, info):
-    """msd_sort: (route or None, tags launched).  None = the LSD passes sort the run."""
-    if not sw["msd"] or n < MSD_MIN_N or n >= RUN_LIMIT:
+    """msd_sort: (route or None, tags launched).  None = the LSD passes sort the run.  info["skewed"]: the flag
+    the sort leaves on the run (msd_plan: 16 or more tuples per possible key; msd_after_level_a: a sub-bucket over
+    BIG_CAP tuples), which sends its joins down the two-phase route."""
+    if not sw["msd"] or n < MSD_MIN_N:
         return None, {}
     span = kmax - kmin
+    info["skewed"] = n // (span + 1) >= 16
+    if n >= RUN_LIMIT:
+        return None, {}
     kb = _bitlen(span)
     info["msd_key_bits"] = kb
     if kb < MSD_MIN_BITS or kb > MSD_MAX_BITS:
@@ -93,6 +98,8 @@ def _msd(keys, n, kmin, kmax, hist_bits, sw, info):
     sub = np.bincount(((keys - U64(kmin)) >> U64(R)).astype(np.int64), minlength=1 << P)
     max_sub, nbig = int(sub.max()), int((sub > BIG_CAP).sum())
     info.update(R=R, cached_hist=cached, max_sub=max_sub, nbig=nbig)
+    if max_sub > BIG_CAP:
+        info["skewed"] = True
     tags = {"msd_hist": 1 if cached else 2, "msd_partition": 1}
     big_route = max_sub > MSD_LOCAL_CAP and bool(sw["big"]) and 0 < R <= COUNT_MAX_R and nbig <= BIG_MAX
     if not (max_sub <= MSD_LOCAL_CAP or R == 0 or big_route):
@@ -122,8 +129,9 @@ def plan(run, keys, env):
     (route, {tag: launches} for the tags in WATCH, the planner's inputs and intermediates)."""
     sw = switches(env)
     n, key_bits, kmin, kmax = run["n"], run["key_bits"], run["key_min"], run["key_max"]
-    info = {"n": n, "key_bits": key_bits, "key_min": kmin, "key_max": kmax, "kind": run["kind"]}
+    info = {"n": n, "key_bits": key_bits, "key_min": kmin, "key_max": kmax, "kind": run["kind"], "skewed": False}
     if run["in_order"] and sw["probe"]:
+        info["skewed"] = kmax < (1 << 64) - 1 and n // (kmax + 1) >= 16  # qce_sort_tuples: from the statistics
         return "in_order", {}, info
     if run["wide"]:
         npass = -(-key_bits // 8)

@@ -408,6 +408,45 @@ int qce_rowid_push_plan(const uint64_t *hists, uint32_t world, uint32_t rank, ui
                         uint32_t bins_per_rank, uint64_t *bin_u32_offset, uint64_t *view_u32_offset,
                         uint64_t *view_count, uint64_t *window_bytes, uint64_t *sent_ids);
 
+/* Exchange plan of a join whose two packed sides (side 0 = R, the outer side; side 1 = S) are
+ * both pushed, and whose rank boundaries may fall inside one heavy key K: R's tuples of K are
+ * divided by position (the first q of K's global group below the cut), S's tuples of K go to
+ * every rank of K's span.  Concatenating the ranks' merge outputs stays R-major and key-ordered.
+ *
+ * Called once per refinement level, identically on every rank.  hists[world][2][256] are the
+ * top-8-bit histograms (qce_exchange_plan's); sub_hists holds, level after level, the
+ * [world][2][nsel][256] histograms of the bins this entry asked for at that level: over the keys
+ * with key >> sel_shift == prefix, bin = the next min(sel_shift, 8) key bits below the prefix.  It returns 0 and either *next_nsel > 0 with the prefixes to
+ * histogram next (next_sel[], next_sel_shift), or *next_nsel = 0 and the final plan.  next_sel
+ * holds QCE_SPLIT_MAX (15) entries; at most world - 1 are used.
+ * When the bin cuts leave no rank more than 10 % over total / world the plan is qce_exchange_plan's
+ * (levels = 0, every cut_q 0) and nothing is refined. */
+#define QCE_PLAN_MAX_RANKS 16 /* the engine's rank limit */
+#define QCE_SPLIT_MAX 15
+#define QCE_PLAN_MAX_COLS 12
+typedef struct {
+    uint32_t refined;                     /* 0: the bin cuts kept every rank within 10 % (qce_exchange_plan's plan) */
+    uint32_t levels;                      /* refinement levels consumed */
+    uint32_t nsplit;                      /* keys cut by position */
+    uint64_t cut_key[QCE_PLAN_MAX_RANKS]; /* world-1 cuts: rank r+1 starts at key cut_key[r] ... */
+    uint64_t cut_q[QCE_PLAN_MAX_RANKS];   /* ... after its first cut_q[r] outer tuples (0: whole key) */
+    uint64_t split_key[QCE_SPLIT_MAX];
+    uint32_t split_first[QCE_SPLIT_MAX], split_last[QCE_SPLIT_MAX]; /* the key's span of ranks */
+    /* [key][source][d - first]: in source's own index space of its outer tuples of the key, where
+     * destination d starts (0 for d = first); the source's count follows in split_count */
+    uint64_t split_bound[QCE_SPLIT_MAX][QCE_PLAN_MAX_RANKS][QCE_PLAN_MAX_RANKS];
+    uint64_t split_count[QCE_SPLIT_MAX][QCE_PLAN_MAX_RANKS][2]; /* [key][source][side] tuples of the key */
+    uint64_t key_lo[QCE_PLAN_MAX_RANKS], key_hi[QCE_PLAN_MAX_RANKS]; /* inclusive; adjacent ranks may share a
+                                                                        split key; key_lo > key_hi: no key */
+    uint64_t count[2][QCE_PLAN_MAX_RANKS][QCE_PLAN_MAX_RANKS];      /* [side][source][destination], copies included */
+    uint64_t recv[2][QCE_PLAN_MAX_RANKS], before[2][QCE_PLAN_MAX_RANKS], run_off[2][QCE_PLAN_MAX_RANKS];
+    uint64_t col_off[QCE_PLAN_MAX_COLS][QCE_PLAN_MAX_RANKS];
+    uint64_t window_bytes, sent[2];
+} qce_split_plan_t;
+int qce_split_plan(const uint64_t *hists, uint32_t world, uint32_t rank, const uint32_t *ncols, uint32_t key_bits,
+                   uint32_t nlevels, const uint32_t *nsel, const uint64_t *sub_hists, uint32_t *next_nsel,
+                   uint64_t *next_sel, uint32_t *next_sel_shift, qce_split_plan_t *plan);
+
 #ifdef __cplusplus
 }
 #endif

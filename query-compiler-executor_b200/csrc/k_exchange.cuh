@@ -233,6 +233,141 @@ k_push(const KeyT *__restrict__ in, u32 n, PushDigit<KeyT> digit, PushPlan plan,
     }
 }
 
+// ---- exchange that cuts inside heavy keys (qce_split_plan) -------------------------------------
+// Destination of a packed tuple: the number of thresholds at or below its key, except for the split
+// keys: an outer (R) tuple of split key j goes by its index among this rank's tuples of the key
+// (bound[j][i] = where destination first[j] + i starts), an inner (S) tuple to every rank of
+// [first[j], last[j]].  W <= 16, <= 15 split keys.
+#define QCE_SPLIT_KEYS 15
+struct SplitRoute {
+    unsigned long long thr[QCE_MAX_RANKS - 1]; // key >= thr[c]: past cut c
+    u32 ncut, nsplit, inner;                    // inner: this side's split-key tuples are copied over the span
+    u32 key[QCE_SPLIT_KEYS], first[QCE_SPLIT_KEYS], last[QCE_SPLIT_KEYS];
+    u32 bound[QCE_SPLIT_KEYS][QCE_MAX_RANKS];
+};
+
+// every lane calls it; a lane with k < 0 takes nothing.  Lanes with the same k share one shared
+// atomic (a heavy key puts whole warps on one counter).  Returns the lane's rank under counter k.
+__device__ __forceinline__ u32 warp_agg_add(u32 *ctr, int k)
+{
+    const u32 peers = __match_any_sync(QCE_FULL_MASK, k);
+    const int leader = __ffs(peers) - 1;
+    u32 b = 0;
+    if (k >= 0 && (int)(threadIdx.x & 31) == leader) b = atomicAdd(&ctr[k], (u32)__popc(peers));
+    b = __shfl_sync(QCE_FULL_MASK, b, leader);
+    return b + (u32)__popc(peers & lanemask_lt());
+}
+
+// 256-bin histograms of the next min(shift, 8) key bits of the packed tuples whose key >> shift is one
+// of the nsel prefixes (out[j * 256 + bin], zeroed by the caller)
+struct SubBins {
+    u32 prefix[QCE_SPLIT_KEYS];
+    u32 nsel;
+    int shift, sub_shift;
+    u32 mask;
+};
+__global__ void __launch_bounds__(512)
+k_key_histogram_sub(const u64 *__restrict__ in, u64 n, const __grid_constant__ SubBins sb, u32 *__restrict__ out)
+{
+    __shared__ u32 sh[QCE_SPLIT_KEYS * 256];
+    for (u32 i = threadIdx.x; i < sb.nsel * 256; i += 512) sh[i] = 0;
+    __syncthreads();
+    const u64 stride = (u64)gridDim.x * 512;
+    for (u64 base = (u64)blockIdx.x * 512 + (threadIdx.x & ~31u); base < n; base += stride) {
+        const u64 i = base + (threadIdx.x & 31);
+        int k = -1;
+        if (i < n) {
+            const u64 key = ld_stream_u64(in + i) >> 32;
+            for (u32 j = 0; j < sb.nsel; j++)
+                if ((key >> sb.shift) == sb.prefix[j]) k = (int)(j * 256 + (((u32)key >> sb.sub_shift) & sb.mask));
+        }
+        warp_agg_add(sh, k);
+    }
+    __syncthreads();
+    for (u32 i = threadIdx.x; i < sb.nsel * 256; i += 512)
+        if (sh[i]) atomicAdd(&out[i], sh[i]);
+}
+
+// The push of one side under a split plan.  A 1024-tuple tile counts its tuples (and copies) per
+// destination in shared memory, reserves one run per destination with one atomicAdd on that
+// destination's LOCAL cursor, and stores every tuple into its run (REWRITE: the payload becomes the
+// copy's index in the receiver's run, and the attached columns go with every copy).  The outer index
+// of a split key comes from one atomicAdd per (tile, key) on split_seen.
+template <bool REWRITE>
+__global__ void __launch_bounds__(256, 4)
+k_push_split(const u64 *__restrict__ in, u32 n, const __grid_constant__ SplitRoute rt, PushPlan plan,
+             const __grid_constant__ PeerWindows peers, const __grid_constant__ PushCols cols,
+             unsigned long long *__restrict__ split_seen)
+{
+    constexpr int THREADS = 256, ITEMS = 4, TILE = THREADS * ITEMS;
+    __shared__ u32 kcnt[QCE_SPLIT_KEYS], dcnt[QCE_MAX_RANKS], dput[QCE_MAX_RANKS];
+    __shared__ unsigned long long kbase[QCE_SPLIT_KEYS], dbase[QCE_MAX_RANKS];
+    const u32 tid = threadIdx.x, begin = blockIdx.x * TILE;
+    if (begin >= n) return;
+    if (tid < QCE_SPLIT_KEYS) kcnt[tid] = 0;
+    if (tid < QCE_MAX_RANKS) { dcnt[tid] = 0; dput[tid] = 0; }
+    __syncthreads();
+    u64 w[ITEMS];
+    u32 dlo[ITEMS], dhi[ITEMS]; // destinations [dlo, dhi] of each tuple (dhi < dlo: none)
+    int sk[ITEMS];
+    u32 pos[ITEMS];
+#pragma unroll
+    for (int t = 0; t < ITEMS; t++) {
+        const u32 i = begin + tid + t * THREADS;
+        w[t] = 0; dlo[t] = 1; dhi[t] = 0; sk[t] = -1;
+        if (i < n) {
+            w[t] = ld_stream_u64(in + i);
+            const u32 key = (u32)(w[t] >> 32);
+            u32 d = 0;
+            for (u32 c = 0; c < rt.ncut; c++) d += (unsigned long long)key >= rt.thr[c];
+            dlo[t] = dhi[t] = d;
+            for (u32 j = 0; j < rt.nsplit; j++)
+                if (key == rt.key[j]) sk[t] = (int)j;
+            if (sk[t] >= 0 && rt.inner) { dlo[t] = rt.first[sk[t]]; dhi[t] = rt.last[sk[t]]; }
+        }
+        pos[t] = warp_agg_add(kcnt, rt.inner ? -1 : sk[t]);
+    }
+    __syncthreads();
+    if (tid < rt.nsplit && !rt.inner) kbase[tid] = kcnt[tid] ? atomicAdd(&split_seen[tid], (unsigned long long)kcnt[tid]) : 0ull;
+    __syncthreads();
+#pragma unroll
+    for (int t = 0; t < ITEMS; t++) {
+        if (sk[t] >= 0 && !rt.inner) {
+            const int j = sk[t];
+            const unsigned long long idx = kbase[j] + pos[t];
+            u32 d = rt.first[j];
+            for (u32 e = rt.first[j] + 1; e <= rt.last[j]; e++) d += idx >= rt.bound[j][e - rt.first[j]];
+            dlo[t] = dhi[t] = d;
+        }
+    }
+    // per destination: count, reserve, store (the same walk twice, so each copy finds its slot again)
+    for (int pass = 0; pass < 2; pass++) {
+#pragma unroll
+        for (int t = 0; t < ITEMS; t++) {
+            for (u32 c = 0; c < plan.ndigits; c++) { // copies: block-uniform trip count for the warp vote
+                const u32 e = dlo[t] + c;
+                const int k = (dlo[t] <= dhi[t] && e <= dhi[t]) ? (int)e : -1;
+                if (!__any_sync(QCE_FULL_MASK, k >= 0)) break;
+                const u32 s = warp_agg_add(pass == 0 ? dcnt : dput, k);
+                if (pass == 1 && k >= 0) {
+                    const unsigned long long at = dbase[e] + s;
+                    u64 v = w[t];
+                    if (REWRITE) v = (v & ~0xffffffffull) | (u64)(plan.run_base[e] + (u32)(at - plan.seg_start[e]));
+                    ((u64 *)peers.base[e])[at] = v;
+                    if (REWRITE) {
+                        const u32 i = begin + tid + t * THREADS;
+                        for (int cc = 0; cc < cols.n; cc++)
+                            ((u32 *)peers.base[e])[cols.region[cc][e] + (at - plan.seg_start[e])] = ld_stream_u32(cols.in[cc] + i);
+                    }
+                }
+            }
+        }
+        __syncthreads();
+        if (pass == 0 && tid < plan.ndigits) dbase[tid] = dcnt[tid] ? atomicAdd(&plan.cursor[tid], (unsigned long long)dcnt[tid]) : 0ull;
+        __syncthreads();
+    }
+}
+
 // Wide runs (keys >= 2^32: SoA u64 keys + u32 row ids).  Such keys usually sit at a high offset
 // (64-bit ids, timestamps), so the digit is the top byte of key - base over the exchange's width,
 // not of the key itself: the top bits of the key would put every tuple in one bin.
@@ -499,6 +634,18 @@ k_gather_u32(const u32 *__restrict__ src, const u32 *__restrict__ index, u64 n, 
 {
     const u64 stride = (u64)gridDim.x * 256;
     for (u64 i = (u64)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) out[i] = __ldg(src + ld_stream_u32(index + i));
+}
+
+// A packed run back to its two halves: hi[i] = in[i] >> 32, lo[i] = (u32)in[i]
+__global__ void __launch_bounds__(256)
+k_unpack_pairs(const u64 *__restrict__ in, u64 n, u32 *__restrict__ hi, u32 *__restrict__ lo)
+{
+    const u64 stride = (u64)gridDim.x * 256;
+    for (u64 i = (u64)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) {
+        const u64 w = ld_stream_u64(in + i);
+        hi[i] = (u32)(w >> 32);
+        lo[i] = (u32)w;
+    }
 }
 
 // Carried join-key column: the low 32 bits of rows [begin, begin + n) of a base column.

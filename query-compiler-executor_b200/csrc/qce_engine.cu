@@ -27,6 +27,7 @@
 #include "../../include/qce_b200.h"
 #include "k_filter.cuh"
 #include "k_join.cuh"
+#include <memory>
 #include "k_radix.cuh"
 #include "k_exchange.cuh"
 #include "qce_comm.cuh"
@@ -47,6 +48,7 @@ struct Dist {
     std::vector<uint64_t> split;  // KEYS: world-1 ascending splitters, rank r holds keys in [split[r-1], split[r])
     bool wide = false;       // KEYS of a wide exchange: the splitters and key_bits are those of key - base
     u64 base = 0;            // (a splitter of ~0 lies past every key: the cut 2^64 at width 64)
+    bool from_split = false; // output of a join whose exchange cut inside a key: one key's pairs on several ranks
 };
 struct qce_rowids {
     u32 *d;        // device row ids (this rank's share)
@@ -3137,6 +3139,12 @@ int qce_exchange_plan(const uint64_t *hists, uint32_t world, uint32_t rank, uint
     return exchange_plan_impl(hists, world, rank, nsides, ncols, key_bits, nullptr, splitters, recv, before, run_off, col_off,
                               window_bytes, sent_tuples);
 }
+int qce_split_plan(const uint64_t *hists, uint32_t world, uint32_t rank, const uint32_t *ncols, uint32_t key_bits,
+                   uint32_t nlevels, const uint32_t *nsel, const uint64_t *sub_hists, uint32_t *next_nsel,
+                   uint64_t *next_sel, uint32_t *next_sel_shift, qce_split_plan_t *plan)
+{
+    return split_plan_impl(hists, world, rank, ncols, key_bits, nlevels, nsel, sub_hists, next_nsel, next_sel, next_sel_shift, plan);
+}
 
 // Row ids routed to the ranks that own the rows: per binding, where this rank's ids of every
 // bin go in the owner's window (bin-major inside an owner, earlier ranks first inside a bin).
@@ -3243,6 +3251,205 @@ int exchange_plan_impl(const uint64_t *hists, uint32_t world, uint32_t rank, uin
             }
     }
     *window_bytes = *std::max_element(top.begin(), top.end());
+    return 0;
+}
+
+// ---- exchange plan with cuts inside heavy keys (qce_split_plan) ---------------------------
+// The key space as an ordered list of pieces -- histogram bins of some level, refined where a cut
+// falls -- each with its tuples per (source, side).  A cut is (key, q): the next rank starts at
+// `key`, after the first q outer tuples of that key's global group (q = 0: at the key's start).
+struct PlanPiece {
+    u64 lo;    // first key; the piece holds [lo, lo + 2^shift)
+    int shift;
+    std::vector<u64> c; // [source * 2 + side]
+};
+struct PlanCut {
+    u64 key = 0, q = 0;
+    bool operator<(const PlanCut &o) const { return key != o.key ? key < o.key : q < o.q; }
+};
+
+// Tuple positions are counted in one stream, key by key, a key's inner tuples before its outer
+// ones (a rank that takes part of a key's outer group also holds all of its inner group).  Cut k
+// aims at T * k / W and is good within share / 20, which keeps every rank within 10 % of its share
+// (plus the inner copies of split keys).  *refine gets the pieces that hold a cut that missed and
+// can still be refined.
+void plan_cuts(const std::vector<PlanPiece> &pieces, u32 W, std::vector<PlanCut> *cuts, std::vector<size_t> *refine)
+{
+    std::vector<u64> tot(pieces.size()), inner(pieces.size()), outer(pieces.size());
+    u64 T = 0;
+    for (size_t i = 0; i < pieces.size(); i++) {
+        u64 r = 0, s = 0;
+        for (u32 src = 0; src < W; src++) { r += pieces[i].c[src * 2]; s += pieces[i].c[src * 2 + 1]; }
+        outer[i] = r; inner[i] = s; tot[i] = r + s; T += r + s;
+    }
+    cuts->assign(W - 1, PlanCut());
+    refine->clear();
+    size_t i = 0;
+    u64 cum = 0; // tuples before piece i
+    for (u32 k = 1; k < W; k++) {
+        typedef unsigned __int128 u128;
+        const u128 goal = (u128)T * k; // the target, scaled by W
+        while (i + 1 < pieces.size() && (u128)(cum + tot[i]) * W < goal) { cum += tot[i]; i++; }
+        const PlanPiece &p = pieces[i];
+        const u128 eb = goal - (u128)cum * W, ea = (u128)(cum + tot[i]) * W - goal; // misses of the two boundaries
+        PlanCut c;
+        c.key = eb <= ea ? p.lo : p.lo + (1ull << p.shift);
+        if (std::min(eb, ea) * 20 > (u128)T) {
+            if (p.shift > 0) {
+                if (refine->empty() || refine->back() != i) refine->push_back(i);
+            } else {
+                const u64 t = (u64)(goal / W);
+                if (outer[i] >= 2 && t > cum + inner[i]) {
+                    const u64 q = t - cum - inner[i];
+                    if (q < outer[i]) { c.key = p.lo; c.q = q; }
+                }
+            }
+        }
+        if (k > 1 && c < (*cuts)[k - 2]) c = (*cuts)[k - 2];
+        (*cuts)[k - 1] = c;
+    }
+}
+
+int split_plan_impl(const uint64_t *hists, uint32_t W, uint32_t rank, const uint32_t *ncols, uint32_t key_bits,
+                    uint32_t nlevels, const uint32_t *nsel, const uint64_t *sub_hists, uint32_t *next_nsel,
+                    uint64_t *next_sel, uint32_t *next_sel_shift, qce_split_plan_t *P)
+{
+    if (!hists || !ncols || !next_nsel || !next_sel || !next_sel_shift || !P || (nlevels && (!nsel || !sub_hists)))
+        return fail("null argument");
+    if (W < 1 || W > QCE_PLAN_MAX_RANKS || rank >= W) return fail("bad exchange shape");
+    if (key_bits == 0 || key_bits > 32) return fail("packed runs carry keys of 1..32 bits");
+    if (ncols[0] + ncols[1] > QCE_PLAN_MAX_COLS) return fail("at most %d columns travel with the two runs", QCE_PLAN_MAX_COLS);
+    memset(P, 0, sizeof *P);
+    *next_nsel = 0;
+    *next_sel_shift = 0;
+    const int shift0 = key_bits > 8 ? (int)key_bits - 8 : 0;
+    std::vector<PlanPiece> pieces(256);
+    for (u32 b = 0; b < 256; b++) {
+        pieces[b].lo = (u64)b << shift0;
+        pieces[b].shift = shift0;
+        pieces[b].c.resize((size_t)W * 2);
+        for (u32 s = 0; s < W; s++)
+            for (u32 k = 0; k < 2; k++) pieces[b].c[s * 2 + k] = hists[((size_t)s * 2 + k) * 256 + b];
+    }
+    std::vector<PlanCut> cuts(W - 1);
+    // today's bin cuts first: refine only when they leave a rank more than 10 % over its share
+    {
+        uint64_t sp[QCE_PLAN_MAX_RANKS], recv[2 * QCE_PLAN_MAX_RANKS], bef[2 * QCE_PLAN_MAX_RANKS], ro[2 * QCE_PLAN_MAX_RANKS];
+        uint64_t co[QCE_PLAN_MAX_COLS * QCE_PLAN_MAX_RANKS], need, sent[2];
+        if (exchange_plan_impl(hists, W, rank, 2, ncols, key_bits, nullptr, sp, recv, bef, ro, co, &need, sent) != 0) return -1;
+        u64 T = 0, mx = 0;
+        for (u32 d = 0; d < W; d++) { T += recv[d] + recv[W + d]; mx = std::max<u64>(mx, recv[d] + recv[W + d]); }
+        for (u32 k = 0; k + 1 < W; k++) cuts[k].key = sp[k];
+        const bool bins_balanced = W == 1 || (unsigned __int128)mx * 10 * W <= (unsigned __int128)T * 11;
+        if (!bins_balanced) {
+            P->refined = 1;
+            const uint64_t *sub = sub_hists;
+            for (u32 lvl = 0;; lvl++) {
+                std::vector<size_t> refine;
+                plan_cuts(pieces, W, &cuts, &refine);
+                if (refine.empty()) { P->levels = lvl; break; }
+                const int sh = pieces[refine[0]].shift, sub_shift = sh > 8 ? sh - 8 : 0;
+                for (size_t i : refine)
+                    if (pieces[i].shift != sh) return fail("refinement across levels");
+                if (lvl == nlevels) { // ask for the next level's histograms
+                    *next_nsel = (u32)refine.size();
+                    *next_sel_shift = (u32)sh;
+                    for (size_t j = 0; j < refine.size(); j++) next_sel[j] = pieces[refine[j]].lo >> sh;
+                    P->levels = lvl;
+                    return 0;
+                }
+                if (nsel[lvl] != refine.size()) return fail("level %u: %u histograms given, %zu asked", lvl, nsel[lvl], refine.size());
+                const u32 ns = nsel[lvl], nsub = 1u << (sh - sub_shift);
+                std::vector<PlanPiece> next;
+                next.reserve(pieces.size() + refine.size() * nsub);
+                for (size_t i = 0, j = 0; i < pieces.size(); i++) {
+                    if (j < refine.size() && refine[j] == i) {
+                        for (u32 b = 0; b < nsub; b++) {
+                            PlanPiece q;
+                            q.lo = pieces[i].lo + ((u64)b << sub_shift);
+                            q.shift = sub_shift;
+                            q.c.resize((size_t)W * 2);
+                            for (u32 s = 0; s < W; s++)
+                                for (u32 k = 0; k < 2; k++) q.c[s * 2 + k] = sub[(((size_t)s * 2 + k) * ns + j) * 256 + b];
+                            next.push_back(std::move(q));
+                        }
+                        j++;
+                    } else {
+                        next.push_back(std::move(pieces[i]));
+                    }
+                }
+                pieces.swap(next);
+                sub += (size_t)W * 2 * ns * 256;
+            }
+        }
+    }
+    // the plan of these cuts: per piece its destination, a split key's groups divided by position
+    for (u32 k = 0; k + 1 < W; k++) { P->cut_key[k] = cuts[k].key; P->cut_q[k] = cuts[k].q; }
+    size_t ci = 0; // cuts at or before the current piece's first key
+    for (const PlanPiece &p : pieces) {
+        while (ci < cuts.size() && cuts[ci].q == 0 && cuts[ci].key <= p.lo) ci++;
+        size_t cj = ci;
+        while (cj < cuts.size() && cuts[cj].key == p.lo && cuts[cj].q > 0) cj++;
+        const u32 first = (u32)ci, m = (u32)(cj - ci);
+        if (m == 0) {
+            for (u32 s = 0; s < W; s++)
+                for (u32 k = 0; k < 2; k++) P->count[k][s][first] += p.c[s * 2 + k];
+            continue;
+        }
+        const u32 j = P->nsplit++;
+        P->split_key[j] = p.lo;
+        P->split_first[j] = first;
+        P->split_last[j] = first + m;
+        u64 r = 0;
+        for (u32 s = 0; s < W; s++) r += p.c[s * 2];
+        u64 pre = 0;
+        for (u32 s = 0; s < W; s++) {
+            const u64 rs = p.c[s * 2];
+            for (u32 i = 0; i <= m; i++) {
+                const u64 q0 = i == 0 ? 0 : cuts[ci + i - 1].q, q1 = i == m ? r : cuts[ci + i].q;
+                const u64 a = std::max(q0, pre), b = std::min(q1, pre + rs);
+                P->count[0][s][first + i] += b > a ? b - a : 0;
+                P->count[1][s][first + i] += p.c[s * 2 + 1];
+                P->split_bound[j][s][i] = std::min(rs, q0 > pre ? q0 - pre : 0);
+            }
+            P->split_count[j][s][0] = rs;
+            P->split_count[j][s][1] = p.c[s * 2 + 1];
+            pre += rs;
+        }
+        ci = cj;
+    }
+    const u64 key_top = (1ull << key_bits) - 1;
+    // exactly the keys the push delivers: a rank between two equal whole-key cuts, or past the last key,
+    // gets an empty range (key_lo > key_hi)
+    for (u32 d = 0; d < W; d++) {
+        const int64_t lo = d == 0 ? 0 : (int64_t)cuts[d - 1].key; // keys < 2^32, cuts <= 2^32
+        const int64_t hi = std::min<int64_t>((int64_t)key_top, d + 1 == W ? (int64_t)key_top
+                                                                : cuts[d].q ? (int64_t)cuts[d].key : (int64_t)cuts[d].key - 1);
+        if (hi < lo) { P->key_lo[d] = 1; P->key_hi[d] = 0; }
+        else { P->key_lo[d] = (u64)lo; P->key_hi[d] = (u64)hi; }
+    }
+    // the window layout, as exchange_plan_impl lays it out
+    std::vector<u64> top(W, 0);
+    size_t col_at = 0;
+    for (u32 k = 0; k < 2; k++) {
+        P->sent[k] = 0;
+        for (u32 d = 0; d < W; d++) {
+            for (u32 s = 0; s < W; s++) {
+                const u64 c = P->count[k][s][d];
+                if (s < rank) P->before[k][d] += c;
+                if (s == rank && d != rank) P->sent[k] += c;
+                P->recv[k][d] += c;
+            }
+            P->run_off[k][d] = top[d];
+            top[d] = (top[d] + 8 * P->recv[k][d] + 15) / 16 * 16;
+        }
+        for (u32 c = 0; c < ncols[k]; c++, col_at++)
+            for (u32 d = 0; d < W; d++) {
+                P->col_off[col_at][d] = top[d];
+                top[d] = (top[d] + 4 * P->recv[k][d] + 15) / 16 * 16;
+            }
+    }
+    P->window_bytes = *std::max_element(top.begin(), top.end());
     return 0;
 }
 

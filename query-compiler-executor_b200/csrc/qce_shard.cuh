@@ -190,6 +190,108 @@ int tuples_to_root(const qce_tuples *in, qce_tuples **out)
 int exchange_plan_impl(const uint64_t *hists, uint32_t world, uint32_t rank, uint32_t nsides, const uint32_t *ncols,
                        uint32_t key_bits, const uint64_t *fixed_splitters, uint64_t *splitters, uint64_t *recv,
                        uint64_t *before, uint64_t *run_off, uint64_t *col_off, uint64_t *window_bytes, uint64_t *sent_tuples);
+int split_plan_impl(const uint64_t *hists, uint32_t W, uint32_t rank, const uint32_t *ncols, uint32_t key_bits,
+                    uint32_t nlevels, const uint32_t *nsel, const uint64_t *sub_hists, uint32_t *next_nsel,
+                    uint64_t *next_sel, uint32_t *next_sel_shift, qce_split_plan_t *P);
+
+static_assert(QCE_PLAN_MAX_RANKS == QCE_MAX_RANKS && QCE_SPLIT_MAX == QCE_SPLIT_KEYS, "qce_split_plan_t mirrors the engine's limits");
+
+// qce_split_plan's histograms of one packed run: the next min(shift, 8) key bits under each prefix
+int key_histogram_sub(const qce_tuples *t, u32 nsel, const uint64_t *prefix, u32 shift, uint64_t *out)
+{
+    SubBins sb;
+    memset(&sb, 0, sizeof sb);
+    sb.nsel = nsel;
+    sb.shift = (int)shift;
+    sb.sub_shift = shift > 8 ? (int)shift - 8 : 0;
+    sb.mask = (1u << std::min<u32>(shift, 8)) - 1;
+    for (u32 j = 0; j < nsel; j++) sb.prefix[j] = (u32)prefix[j];
+    u32 *d = nullptr;
+    if (dalloc(&d, (u64)nsel * 256) != 0) return -1;
+    CK(cudaMemsetAsync(d, 0, (size_t)nsel * 256 * sizeof(u32), cx().stream));
+    if (t->n) LAUNCH("key_hist_sub", k_key_histogram_sub, grid_for(4096, t->n, 4), 512, 0, (const u64 *)t->a, t->n, sb, d);
+    std::vector<u32> h((size_t)nsel * 256);
+    CK(cudaMemcpyAsync(h.data(), d, h.size() * sizeof(u32), cudaMemcpyDeviceToHost, cx().stream));
+    CK(cudaStreamSynchronize(cx().stream));
+    dfree(d);
+    for (size_t i = 0; i < h.size(); i++) out[i] = h[i];
+    return 0;
+}
+
+// k_push_split of side k (0 = outer, 1 = inner) of this rank under plan P; the arguments are those of
+// qce_push_tuples_cols
+int push_tuples_split(const qce_tuples *t, const qce_split_plan_t &P, u32 k, const uint64_t *dst_word_offset,
+                      const uint32_t *run_index, u32 ncols, const qce_rowids *const *cols, const uint64_t *col_u32_offset)
+{
+    const u32 W = G.world, me = G.rank;
+    if (t->wide || t->n >= (1ull << 32) - 4096) return fail("split push takes packed runs below 2^32 tuples");
+    for (u32 d = 0; d < W; d++) // a wrong plan must not scribble over a peer's memory
+        if (P.count[k][me][d] && (dst_word_offset[d] + P.count[k][me][d]) * 8 > G.xwin_bytes)
+            return fail("split push would overrun rank %u's window", d);
+    SplitRoute rt;
+    memset(&rt, 0, sizeof rt);
+    rt.ncut = W - 1;
+    for (u32 c = 0; c + 1 < W; c++) rt.thr[c] = P.cut_q[c] ? P.cut_key[c] + 1 : P.cut_key[c];
+    rt.nsplit = P.nsplit;
+    rt.inner = k;
+    for (u32 j = 0; j < P.nsplit; j++) {
+        rt.key[j] = (u32)P.split_key[j];
+        rt.first[j] = P.split_first[j];
+        rt.last[j] = P.split_last[j];
+        for (u32 i = 0; i <= P.split_last[j] - P.split_first[j]; i++) rt.bound[j][i] = (u32)P.split_bound[j][me][i];
+    }
+    PushCols pc;
+    memset(&pc, 0, sizeof pc);
+    pc.n = (int)ncols;
+    for (u32 c = 0; c < ncols; c++) {
+        if (!cols[c] || cols[c]->n != t->n) return fail("column %u travels with a run of different length", c);
+        pc.in[c] = cols[c]->d;
+        for (u32 r = 0; r < W; r++) pc.region[c][r] = col_u32_offset[(size_t)c * W + r];
+    }
+    if (t->n == 0) return 0;
+    unsigned long long *d_seg = nullptr, *d_cur = nullptr, *d_seen = nullptr;
+    u32 *d_run = nullptr;
+    if (dalloc(&d_seg, QCE_MAX_RANKS) || dalloc(&d_cur, QCE_MAX_RANKS) || dalloc(&d_run, QCE_MAX_RANKS) || dalloc(&d_seen, QCE_SPLIT_KEYS))
+        return -1;
+    unsigned long long seg[QCE_MAX_RANKS] = {0};
+    u32 run[QCE_MAX_RANKS] = {0};
+    for (u32 d = 0; d < W; d++) { seg[d] = dst_word_offset[d]; run[d] = run_index ? run_index[d] : 0u; }
+    CK(cudaMemcpyAsync(d_seg, seg, sizeof seg, cudaMemcpyHostToDevice, cx().stream));
+    CK(cudaMemcpyAsync(d_cur, seg, sizeof seg, cudaMemcpyHostToDevice, cx().stream));
+    CK(cudaMemcpyAsync(d_run, run, sizeof run, cudaMemcpyHostToDevice, cx().stream));
+    CK(cudaMemsetAsync(d_seen, 0, QCE_SPLIT_KEYS * sizeof(unsigned long long), cx().stream));
+    PushPlan plan{d_seg, d_run, d_cur, W, 1u};
+    const u32 n = (u32)t->n, grid = (u32)ceil_div(n, 1024);
+    if (run_index)
+        LAUNCH("push_split", k_push_split<true>, grid, 256, 0, (const u64 *)t->a, n, rt, plan, G.peers, pc, d_seen);
+    else
+        LAUNCH("push_split", k_push_split<false>, grid, 256, 0, (const u64 *)t->a, n, rt, plan, G.peers, pc, d_seen);
+    dfree_after_push(d_seg); dfree_after_push(d_cur); dfree_after_push(d_run); dfree_after_push(d_seen);
+    return 0;
+}
+
+// Both packed sides of a join pushed (0 = R, 1 = S): the plan that may cut inside a heavy key, its
+// sub-histograms taken level by level (one all-gather each).  P->refined == 0: the bin cuts stand.
+int plan_split(const std::vector<const qce_tuples *> &sides, const std::vector<uint64_t> &all, const uint32_t *ncols,
+               int key_bits, qce_split_plan_t *P)
+{
+    const u32 W = G.world;
+    std::vector<uint32_t> nsel;
+    std::vector<uint64_t> subs;
+    for (;;) {
+        uint32_t next = 0, shift = 0;
+        uint64_t sel[QCE_SPLIT_MAX];
+        if (split_plan_impl(all.data(), W, G.rank, ncols, (u32)key_bits, (u32)nsel.size(), nsel.data(), subs.data(), &next,
+                            sel, &shift, P) != 0) { qcecomm::abort_all(); return -1; }
+        if (next == 0) return 0;
+        std::vector<uint64_t> mine((size_t)2 * next * 256), got((size_t)W * 2 * next * 256);
+        for (u32 k = 0; k < 2; k++)
+            if (key_histogram_sub(sides[k], next, sel, shift, mine.data() + (size_t)k * next * 256) != 0) { qcecomm::abort_all(); return -1; }
+        CQ(qcecomm::allgather(mine.data(), mine.size() * sizeof(uint64_t), got.data()));
+        nsel.push_back(next);
+        subs.insert(subs.end(), got.begin(), got.end());
+    }
+}
 
 struct XRecv {
     qce_tuples *run = nullptr; // a view of this rank's window: valid until the window is written again
@@ -199,8 +301,12 @@ struct XRecv {
 // soon as ITS tuples have landed everywhere -- while the second side's push still crosses NVLink.
 // wide_base != nullptr: every side is wide, binned by key - *wide_base over key_bits (1..64) bits; a
 // side's ids are laid out like one travelling column behind its keys.
+// allow_split: the two packed sides of a join (R, S), both pushed -- the plan may cut inside a heavy key
+// (qce_split_plan) when the bin cuts leave a rank more than 10 % over its share; trace_split gets the
+// split keys and refinement levels.
 int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u64 key_max, const Dist *fixed,
-                  std::vector<XRecv> *out, Dist *dist_out, bool sort_received = false, const u64 *wide_base = nullptr)
+                  std::vector<XRecv> *out, Dist *dist_out, bool sort_received = false, const u64 *wide_base = nullptr,
+                  bool allow_split = false, u32 *trace_split = nullptr)
 {
     static int overlap = -1; // QCE_OVERLAP_PUSH=0: one barrier after all pushes, sorts afterwards
     if (overlap < 0) { const char *e = getenv("QCE_OVERLAP_PUSH"); overlap = e ? atoi(e) : 1; }
@@ -220,8 +326,25 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
     std::vector<uint64_t> splitters(W), recv((size_t)ns * W), before((size_t)ns * W), run_off((size_t)ns * W),
         col_off((total_cols ? total_cols : 1) * W), sent(ns);
     uint64_t need = 0;
-    if (exchange_plan_impl(all.data(), W, me, ns, ncols.data(), (u32)key_bits, fixed ? fixed->split.data() : nullptr,
-                           splitters.data(), recv.data(), before.data(), run_off.data(), col_off.data(), &need, sent.data()) != 0) {
+    std::unique_ptr<qce_split_plan_t> sp;
+    if (allow_split && !wide && !fixed && ns == 2) {
+        sp.reset(new qce_split_plan_t);
+        if (plan_split(sides, all, ncols.data(), key_bits, sp.get()) != 0) return -1;
+        if (!sp->refined) sp.reset();
+    }
+    if (trace_split) { trace_split[0] = sp ? sp->nsplit : 0; trace_split[1] = sp ? sp->levels : 0; }
+    if (sp) {
+        for (u32 k = 0; k < ns; k++)
+            for (u32 d = 0; d < W; d++) {
+                recv[(size_t)k * W + d] = sp->recv[k][d];
+                before[(size_t)k * W + d] = sp->before[k][d];
+                run_off[(size_t)k * W + d] = sp->run_off[k][d];
+            }
+        for (size_t c = 0; c < total_cols; c++)
+            for (u32 d = 0; d < W; d++) col_off[c * W + d] = sp->col_off[c][d];
+        need = sp->window_bytes;
+    } else if (exchange_plan_impl(all.data(), W, me, ns, ncols.data(), (u32)key_bits, fixed ? fixed->split.data() : nullptr,
+                                  splitters.data(), recv.data(), before.data(), run_off.data(), col_off.data(), &need, sent.data()) != 0) {
         qcecomm::abort_all();
         return -1;
     }
@@ -237,7 +360,15 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
         std::vector<uint64_t> dst_words(W);
         for (u32 d = 0; d < W; d++) dst_words[d] = run_off[(size_t)k * W + d] / 8 + before[(size_t)k * W + d];
         int rc;
-        if (wide) {
+        if (sp) {
+            std::vector<uint32_t> run_index(W);
+            std::vector<uint64_t> regions((size_t)std::max<u32>(ncols[k], 1) * W);
+            for (u32 d = 0; d < W; d++) run_index[d] = (u32)before[(size_t)k * W + d];
+            for (u32 c = 0; c < ncols[k]; c++)
+                for (u32 d = 0; d < W; d++) regions[(size_t)c * W + d] = col_off[(col_at + c) * W + d] / 4 + before[(size_t)k * W + d];
+            rc = push_tuples_split(sides[k], *sp, k, dst_words.data(), ncols[k] ? run_index.data() : nullptr, ncols[k],
+                                   sides[k]->attached.data(), regions.data());
+        } else if (wide) {
             std::vector<uint64_t> dst_ids(W);
             for (u32 d = 0; d < W; d++) dst_ids[d] = col_off[col_at * W + d] / 4 + before[(size_t)k * W + d];
             rc = qce_push_tuples_wide(sides[k], base, (u32)key_bits, splitters.data(), W, dst_words.data(), dst_ids.data());
@@ -264,6 +395,10 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
     // the last rank's range ends at the largest key that exists, not at 2^key_bits - 1: the
     // local sort sizes its MSD buckets from this range
     u64 hi = me < W - 1 ? splitters[me] - 1 : key_max;
+    if (sp) { // adjacent ranks may share a split key
+        lo = sp->key_lo[me];
+        hi = me < W - 1 ? sp->key_hi[me] : key_max;
+    }
     if (wide) { // base + [cut, next cut), clipped to the largest key (base + a cut past it may overflow)
         const u64 span = key_max - base, c0 = me > 0 ? splitters[me - 1] : 0, c1 = me < W - 1 ? splitters[me] : ~0ull;
         lo = base + std::min(c0, span);
@@ -323,7 +458,8 @@ int exchange_runs(const std::vector<const qce_tuples *> &sides, int key_bits, u6
         (*out)[k].travelled = ncols[k] != 0;
         col_at += ncols[k];
     }
-    dist_out->kind = Dist::KEYS;
+    dist_out->kind = sp ? Dist::ANY : Dist::KEYS; // a split key's outputs sit on several ranks: never "in place"
+    dist_out->from_split = sp != nullptr;
     dist_out->key_bits = key_bits;
     dist_out->split.assign(splitters.begin(), splitters.begin() + (W - 1));
     dist_out->wide = wide;
@@ -408,6 +544,7 @@ int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_row
     qce_tuples *lr = nullptr, *ls = nullptr;  // the local inputs of the merge
     bool own_r = false, own_s = false, travelled_r = false, travelled_s = false;
     int trace_bits = std::max(R->key_bits, S->key_bits);
+    u32 trace_split[2] = {0, 0}; // split keys, refinement levels
     Dist dist;
     dist.kind = Dist::ANY;
     if (root_only && (!R->attached.empty() || !S->attached.empty())) {
@@ -467,7 +604,7 @@ int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_row
         std::vector<XRecv> got;
         int xrc = 0;
         if (sides.empty()) dist = R->dist;
-        else xrc = exchange_runs(sides, key_bits, key_max, fixed, &got, &dist, true, wide ? &base : nullptr);
+        else xrc = exchange_runs(sides, key_bits, key_max, fixed, &got, &dist, true, wide ? &base : nullptr, !wide, trace_split);
         qce_tuples_free(wr); // the received copies live in the window
         qce_tuples_free(ws);
         if (xrc != 0) return -1;
@@ -481,10 +618,10 @@ int sh_join_runs(qce_tuples *R, qce_tuples *S, bool want_r, bool want_s, qce_row
     }
     static const bool trace = getenv("QCE_TRACE") != nullptr;
     if (trace) // route "local": a side is empty everywhere, nothing moves
-        fprintf(stderr, "[qce] join rank %u/%u: route=%s keys=%s width=%d recv R=%llu/%llu S=%llu/%llu\n", G.rank, G.world,
+        fprintf(stderr, "[qce] join rank %u/%u: route=%s keys=%s width=%d recv R=%llu/%llu S=%llu/%llu split=%u levels=%u\n", G.rank, G.world,
                 !lr ? "local" : root_only ? "root" : "exchange", wide ? "wide" : "packed", trace_bits,
                 (unsigned long long)(lr ? lr->n : 0), (unsigned long long)(R->n + R->n_others), (unsigned long long)(ls ? ls->n : 0),
-                (unsigned long long)(S->n + S->n_others));
+                (unsigned long long)(S->n + S->n_others), trace_split[0], trace_split[1]);
     if (own_r) qce_tuples_free(lr);
     if (own_s) qce_tuples_free(ls);
     if (rc != 0) { qcecomm::abort_all(); return -1; }
@@ -606,11 +743,45 @@ int sh_is_sorted(const qce_tuples *t, int *sorted)
 }
 
 int distinct_pairs(const qce_rowids *pr, const qce_rowids *ps, qce_rowids **dr, qce_rowids **ds);
+// The pairs of a join whose exchange cut inside a key: the copies of one pair may sit on several ranks
+// (a row id repeated under a split key is sliced over its span).  After the local dedup the survivors
+// are exchanged by rowid_R range (key = rowid_R, payload = rowid_S) and deduplicated once more.
+int distinct_pairs_across(const qce_rowids *pr, const qce_rowids *ps, qce_rowids **dr, qce_rowids **ds)
+{
+    qce_rowids *lr = nullptr, *ls = nullptr;
+    if (distinct_pairs(pr, ps, &lr, &ls) != 0) { qcecomm::abort_all(); return -1; }
+    const int bits = pr->id_bound ? std::max(1, bitlen(pr->id_bound - 1)) : 32;
+    qce_tuples T;
+    T.n = lr->n; T.n_others = 0; T.wide = false; T.ids = nullptr; T.key_bits = bits; T.key_min = 0;
+    T.key_max = pr->id_bound ? pr->id_bound - 1 : 0xffffffffull; T.id_bound = ps->id_bound; T.sorted = false;
+    T.a = nullptr; T.sort_pending = true;
+    int rc = dalloc(&T.a, T.n);
+    if (rc == 0 && T.n) LAUNCH("pack_pairs", k_pack_pairs, grid_for(256, T.n), 256, 0, lr->d, ls->d, T.n, T.a);
+    qce_rowids_free(lr);
+    qce_rowids_free(ls);
+    std::vector<XRecv> got;
+    Dist dist;
+    if (rc == 0) rc = exchange_runs({&T}, bits, T.key_max, nullptr, &got, &dist, false);
+    dfree(T.a);
+    dfree(T.hist256);
+    if (rc != 0) return -1;
+    const qce_tuples *g = got[0].run;
+    rc = new_rowids(g->n, pr->id_bound, &lr) || new_rowids(g->n, ps->id_bound, &ls) ? -1 : 0;
+    if (rc == 0 && g->n) LAUNCH("unpack_pairs", k_unpack_pairs, grid_for(2048, g->n), 256, 0, (const u64 *)g->a, g->n, lr->d, ls->d);
+    qce_tuples_free(got[0].run);
+    if (rc == 0) rc = distinct_pairs(lr, ls, dr, ds);
+    qce_rowids_free(lr);
+    qce_rowids_free(ls);
+    if (rc != 0) qcecomm::abort_all();
+    return rc;
+}
 int sh_distinct_pairs(const qce_rowids *pr, const qce_rowids *ps, qce_rowids **dr, qce_rowids **ds)
 {
     // a duplicate (rowid_R, rowid_S) pair carries one key, so both copies live on the rank that
-    // owns the key: the distinct pairs of the whole output are the ranks' distinct pairs
-    if (distinct_pairs(pr, ps, dr, ds) != 0) { qcecomm::abort_all(); return -1; }
+    // owns the key: the distinct pairs of the whole output are the ranks' distinct pairs -- unless
+    // the exchange cut inside a key
+    const int rc = pr->dist.from_split ? distinct_pairs_across(pr, ps, dr, ds) : distinct_pairs(pr, ps, dr, ds);
+    if (rc != 0) { qcecomm::abort_all(); return -1; }
     (*dr)->dist.kind = Dist::ANY;
     (*ds)->dist.kind = Dist::ANY;
     if (others_of((*dr)->n, &(*dr)->n_others) != 0) return -1;

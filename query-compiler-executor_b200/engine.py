@@ -39,7 +39,7 @@ SYMBOLS = [
     "qce_set_replicate_bytes", "qce_column_would_be_whole", "qce_column_is_whole", "qce_rowids_count_local", "qce_xwin_unmap_peers", "qce_build_tuples_positions", "qce_merge_join_stats",
     "qce_elision_supported", "qce_tuples_attach", "qce_placement_cap",
     "qce_key_histogram_wide", "qce_push_tuples_wide", "qce_tuples_from_window_wide",
-    "qce_build_sorted_tuples_base", "qce_column_histogram",
+    "qce_build_sorted_tuples_base", "qce_column_histogram", "qce_split_plan",
 ]
 
 
@@ -115,6 +115,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
         "qce_key_histogram_wide": (i32, [vp, u64, u32, P(u64)]),
         "qce_push_tuples_wide": (i32, [vp, u64, u32, vp, u32, vp, vp]),
         "qce_tuples_from_window_wide": (i32, [u64, u64, u64, u32, u64, u64, P(vp)]),
+        "qce_split_plan": (i32, [vp, u32, u32, vp, u32, u32, vp, vp, P(u32), vp, P(u32), vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -142,6 +143,62 @@ def exchange_plan(lib, hists: np.ndarray, world: int, rank: int, ncols: Sequence
                              C.byref(need), sent.ctypes.data) != 0:
         raise EngineError(lib.qce_last_error().decode())
     return [int(x) for x in splitters[:world - 1]], recv, before, run_off, col_off, need.value, sent
+
+
+_R, _K, _COLS = 16, 15, 12  # QCE_PLAN_MAX_RANKS, QCE_SPLIT_MAX, QCE_PLAN_MAX_COLS
+
+
+class SplitPlan(C.Structure):
+    """qce_split_plan_t"""
+    _fields_ = [("refined", C.c_uint32), ("levels", C.c_uint32), ("nsplit", C.c_uint32),
+                ("cut_key", C.c_uint64 * _R), ("cut_q", C.c_uint64 * _R), ("split_key", C.c_uint64 * _K),
+                ("split_first", C.c_uint32 * _K), ("split_last", C.c_uint32 * _K),
+                ("split_bound", C.c_uint64 * (_K * _R * _R)), ("split_count", C.c_uint64 * (_K * _R * 2)),
+                ("key_lo", C.c_uint64 * _R), ("key_hi", C.c_uint64 * _R), ("count", C.c_uint64 * (2 * _R * _R)),
+                ("recv", C.c_uint64 * (2 * _R)), ("before", C.c_uint64 * (2 * _R)), ("run_off", C.c_uint64 * (2 * _R)),
+                ("col_off", C.c_uint64 * (_COLS * _R)), ("window_bytes", C.c_uint64), ("sent", C.c_uint64 * 2)]
+
+
+def split_plan(lib, hists: np.ndarray, world: int, rank: int, ncols: Sequence[int], key_bits: int, sub_histograms):
+    """qce_split_plan driven to its end (host arithmetic only).  sub_histograms(prefixes, shift) returns the
+    [world][2][len(prefixes)][256] histograms of the next min(shift, 8) key bits over the keys
+    with key >> shift == prefix -- what the ranks take and all-gather on the device.  Returns the plan as a dict of arrays
+    trimmed to `world` ranks."""
+    h = np.ascontiguousarray(hists, dtype=np.uint64)
+    nc = np.ascontiguousarray(ncols, dtype=np.uint32)
+    nsel, subs = [], []
+    while True:
+        plan = SplitPlan()
+        nxt, shift = C.c_uint32(), C.c_uint32()
+        sel = np.zeros(_K, dtype=np.uint64)
+        ns = np.ascontiguousarray(nsel if nsel else [0], dtype=np.uint32)
+        sub = np.ascontiguousarray(np.concatenate(subs) if subs else np.zeros(1, dtype=np.uint64), dtype=np.uint64)
+        if lib.qce_split_plan(h.ctypes.data, world, rank, nc.ctypes.data, key_bits, len(nsel), ns.ctypes.data,
+                              sub.ctypes.data, C.byref(nxt), sel.ctypes.data, C.byref(shift), C.byref(plan)) != 0:
+            raise EngineError(lib.qce_last_error().decode())
+        if nxt.value == 0:
+            break
+        prefixes = [int(x) for x in sel[:nxt.value]]
+        subs.append(np.ascontiguousarray(sub_histograms(prefixes, shift.value), dtype=np.uint64).ravel())
+        nsel.append(nxt.value)
+    W, k = world, plan.nsplit
+
+    def arr(name, shape):
+        return np.frombuffer(getattr(plan, name), dtype=np.uint64).reshape(shape)
+    return {
+        "refined": plan.refined, "levels": plan.levels, "nsplit": k, "requests": list(zip(nsel, [len(x) for x in subs])),
+        "cut_key": arr("cut_key", _R)[:W - 1].copy(), "cut_q": arr("cut_q", _R)[:W - 1].copy(),
+        "split_key": arr("split_key", _K)[:k].copy(),
+        "split_first": np.frombuffer(plan.split_first, dtype=np.uint32)[:k].copy(),
+        "split_last": np.frombuffer(plan.split_last, dtype=np.uint32)[:k].copy(),
+        "split_bound": arr("split_bound", (_K, _R, _R))[:k, :W, :W].copy(),
+        "split_count": arr("split_count", (_K, _R, 2))[:k, :W].copy(),
+        "key_lo": arr("key_lo", _R)[:W].copy(), "key_hi": arr("key_hi", _R)[:W].copy(),
+        "count": arr("count", (2, _R, _R))[:, :W, :W].copy(), "recv": arr("recv", (2, _R))[:, :W].copy(),
+        "before": arr("before", (2, _R))[:, :W].copy(), "run_off": arr("run_off", (2, _R))[:, :W].copy(),
+        "col_off": arr("col_off", (_COLS, _R))[:int(nc.sum()), :W].copy(), "window_bytes": plan.window_bytes,
+        "sent": arr("sent", 2).copy(),
+    }
 
 
 def rowid_push_plan(lib, hists: np.ndarray, world: int, rank: int, nbind: int, bins_per_rank: int):
